@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA path through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU implementation on the host cores
+  python bench.py ... --dump-outputs DIR                    also save a seeded sample of the last timed step's outputs
 
 Workload (BASELINE.json configs[2], SURVEY.md §8d cfg 3 — the headline config): LibriSpeech-shape DELTA+SAT,
 16 kHz synthetic int16 audio, 13 MFCC -> per-speaker CMVN -> delta+delta-delta (39) -> per-speaker fMLLR ->
@@ -257,7 +258,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warm = 1 if args.warmup > 0 else 0
     r = cpu_reference_run(steps, warm, target_s=8.0)
     line = {
@@ -268,8 +269,8 @@ def run_reference_arm(args):
                          "sample": r["sample"]},
         "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0, "steps_requested": args.steps, "warmup_requested": args.warmup,
-        "note": "the reference's CPU path uses the host cores only: the same number is reported for every --gpus; steps / "
-                "warmup are CAPPED at 5 / 1 (each step is ~8 s of CPU work on a bounded sample of the workload)",
+        "note": "the reference's CPU path uses the host cores only: the same number is reported for every --gpus; warmup "
+                "is CAPPED at 1 (each step is ~8 s of CPU work on a bounded sample of the workload)",
     }
     print(json.dumps(line), flush=True)
 
@@ -436,6 +437,8 @@ def run_ours(args):
     rescored = int(sum_over_ranks(am.rescored_frames()))   # frames of the last step the FP32 kernel had to re-score
     total_audio = sum_over_ranks(audio_s)
     value = total_audio / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_ll, d_feats, col_of_pdf, T)
 
     # ---- parity on the timed batch itself (outside the timed region): 256 frames, all pdfs, vs the reference's CPU code ----
     parity = None
@@ -736,6 +739,24 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 2048  # 2048 frames x 4000 pdfs x 4 bytes = 33 MB: the dump stays under 64 MB
+
+
+def dump_outputs(out_dir, d_ll, d_feats, col_of_pdf, T):
+    """What the timed step hands its caller, on a fixed seeded sample of DUMP_ROWS frames of rank 0's batch, so that two
+    builds run with the same arguments can be compared output for output:
+      loglikes.npy    [rows x P_PDFS] float32, in the model's pdf order (the device column order mapped back)
+      feats.npy       [rows x DIM]    float32, the fMLLR-transformed features the loglikes were scored on
+      frame_rows.npy  [rows]          float64, the frame index of each sampled row"""
+    import torch
+    rows = np.sort(np.random.default_rng(SEED + 31).choice(T, min(DUMP_ROWS, T), replace=False))
+    idx = torch.from_numpy(rows).to(d_ll.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loglikes.npy"), np.ascontiguousarray(d_ll[idx].cpu().numpy()[:, col_of_pdf]))
+    np.save(os.path.join(out_dir, "feats.npy"), np.ascontiguousarray(d_feats[idx][:, :DIM].cpu().numpy()))
+    np.save(os.path.join(out_dir, "frame_rows.npy"), rows.astype(np.float64))
+
+
 def am_is_tc(am):
     """True when the tensor-core scorer serves this model (set_kernel(2) is accepted only then)."""
     from voicebridge_b200 import capi
@@ -756,7 +777,14 @@ def main():
     ap.add_argument("--kernel", type=int, default=0, help="0 auto, 1 fp32 simt, 2 tcgen05")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-others", action="store_true", help="skip the other_configs leg (cfg 2 / cfg 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of rank 0's loglikes and features of the last step "
+                         "as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the CUDA path's outputs: it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -741,7 +741,9 @@ def test_scoring_long_run_of_sunk_frames_is_rescored_in_parallel(orc):
                                         (16000, 8000, 7), (11025, 8000, 3000), (16000, 8000, 0)])
 def test_downsample_waveform_vs_oracle_and_reference(orc, orig, new, n):
     """DownsampleWaveForm (feat/resample.cc:368-376) on the device: length and samples.  The oracle port is pinned against the
-    compiled reference in tests/test_oracle_vs_ref.py; 2e-6 of the largest sample (FP32 dot products in a different order)."""
+    compiled reference in tests/test_oracle_vs_ref.py; 2e-6 of the largest sample (FP32 dot products in a different order).
+    The comparison with the compiled reference itself runs only where oracle/_ref is built; in every checkout the same rate
+    pairs are checked against stored reference outputs by test_downsample_golden_dumps_of_the_reference."""
     w = (np.random.default_rng(n + orig).standard_normal(n) * 3000).astype(np.float32)
     want = orc.downsample_waveform(orig, new, w)
     d = host.Downsampler(orig, new)
