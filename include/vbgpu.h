@@ -24,6 +24,9 @@
  *                               file-based reduce of VB/src/gmmbin/gmm-sum-accs.cpp:44-50 (vbgpu_acc_add / all-reduce)
  *   vbgpu_fmllr_*     replaces  FmllrDiagGmmAccs::AccumulateForGmm (fMLLR statistics beta, K, G per speaker)
  *                               transform/fmllr-diag-gmm.cc:30-45,110-121,562-583 (caller VB/src/gmmbin/gmm-est-fmllr.cpp:40-55)
+ *   vbgpu_lda_*       replaces  LdaEstimate::Init / ZeroAccumulators / Accumulate (LDA class statistics of acc-lda)
+ *                               transform/lda-estimate.{h,cc} (caller VB/scr/steps/train_lda_mllt.cpp) and the summing of
+ *                               the per-job lda.*.acc files by est-lda (vbgpu_lda_allreduce)
  *   vbgpu_io_*        reads / writes  Matrix / CompressedMatrix / Vector / int32-vector objects, archive entries, model
  *                               files (-> tid2pdf + flattened AmDiagGmm) and gmm-acc-stats-ali statistics files
  *                               matrix/kaldi-matrix.cc:1375-1460, matrix/compressed-matrix.cc:531-670, gmm/diag-gmm.cc:705-756
@@ -111,6 +114,7 @@ typedef struct vbgpu_acc_s *vbgpu_acc_t;
 typedef struct vbgpu_fmllr_s *vbgpu_fmllr_t;
 typedef struct vbgpu_pipeline_s *vbgpu_pipeline_t;
 typedef struct vbgpu_pitch_s *vbgpu_pitch_t;
+typedef struct vbgpu_lda_s *vbgpu_lda_t;
 
 /* ---- library ------------------------------------------------------------------------------------------------ */
 int vbgpu_version(void);
@@ -191,6 +195,15 @@ int vbgpu_cmvn_stats(vbgpu_feat_t h, const float *feats, int32_t stride, const i
 int vbgpu_feat_run(vbgpu_feat_t h, const float *feats, int32_t in_stride, const int64_t *frame_offsets, int32_t n_utts,
                    const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats, const float *fmllr,
                    int32_t fmllr_cols, float *out, int32_t out_stride);
+/* Device form of vbgpu_feat_run: d_feats, d_out and d_fmllr are device pointers; frame_offsets, utt2spk and cmvn_stats stay
+ * host arrays.  Speakers with a CMVN count below 1 (or non-finite statistics) are rejected on the host before any work.
+ * Splice-only output (what acc-lda reads): lda mode with the K x K identity as transform (K = in_dim * (left + right + 1))
+ * gives the spliced CMVN'd rows bit for bit, since the kernel's products with 1 and 0 are exact.  The transform has to fit
+ * the kernel's shared memory (K = 91 and 117 do; larger K fails cleanly at launch) and costs K^2 FP32 multiply-adds per
+ * frame. */
+int vbgpu_feat_run_dev(vbgpu_feat_t h, const float *d_feats, int32_t in_stride, const int64_t *frame_offsets,
+                       int32_t n_utts, const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats,
+                       const float *d_fmllr, int32_t fmllr_cols, float *d_out, int32_t out_stride, void *stream);
 
 /* ---- acoustic model + scoring ------------------------------------------------------------------------------------------ */
 /* Flattened AmDiagGmm: pdf p owns Gaussians [pdf_offsets[p], pdf_offsets[p+1]); arrays are what
@@ -332,6 +345,33 @@ int vbgpu_fmllr_download(vbgpu_fmllr_t h, int32_t spk, double *beta, double *K, 
  * Runs the fMLLR G contraction over one pseudo-frame per (frame, Gaussian of its pdf). */
 int vbgpu_mllt_accumulate(vbgpu_gmm_t model, const float *feats, int64_t T, int32_t stride, const int32_t *pdf_ids,
                           const float *weights, double *beta, double *G, double *tot_like);
+
+/* ---- LDA class statistics (acc-lda) ----------------------------------------------------------------------------------
+ * LdaEstimate::Accumulate (transform/lda-estimate.cc) for every frame of a batch, one (class, weight) per frame: what
+ * ali-to-post | weight-silence-post 0.0 hands acc-lda.  For each frame with weight w != 0 and class c:
+ *   zero[c] += w,  first[c][:] += w x,  second += w x x^T (lower triangle, SpMatrix packing: (i, j), i >= j, at i(i+1)/2 + j)
+ * all in FP64 with x widened from float first.  Frames of weight exactly 0 are skipped (non-finite features there do no
+ * harm); any other weight, negative included, is used as given.  A class id outside [0, C) adds nothing for its frame and
+ * is counted.  rand_prune is not emulated: every frame is accumulated exactly.  dim 1 ... 256, num_classes >= 1.
+ * The solver (LdaEstimate::Estimate, est-lda) stays on the host and takes these statistics unchanged. */
+int vbgpu_lda_create(int32_t num_classes, int32_t dim, int device, vbgpu_lda_t *out); /* LdaEstimate::Init */
+int vbgpu_lda_destroy(vbgpu_lda_t h);
+int vbgpu_lda_zero(vbgpu_lda_t h); /* ZeroAccumulators */
+/* Host form, synchronous: feats [T x stride], class_ids[T], weights[T] or NULL (= 1.0).  Returns VBGPU_ERR_NUMERIC after
+ * adding every valid frame when some class id was out of range. */
+int vbgpu_lda_accumulate(vbgpu_lda_t h, const float *feats, int64_t T, int32_t stride, const int32_t *class_ids,
+                         const float *weights);
+int vbgpu_lda_accumulate_dev(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_class_ids,
+                             const float *d_weights, void *stream);
+/* Invalid class ids seen by _dev calls since the last query; resets the count (synchronises the handle's work). */
+int vbgpu_lda_bad_count(vbgpu_lda_t h, int64_t *count);
+/* zero[C], first[C x D] row-major, second[D(D+1)/2]; any output may be NULL. */
+int vbgpu_lda_download(vbgpu_lda_t h, double *zero, double *first, double *second);
+/* The statistics are ONE device buffer [ zero (C) | first (C x D) | second (D(D+1)/2) ], so that merging GPUs is a single
+ * in-place sum all-reduce (replaces est-lda summing the per-job accumulator files). */
+int vbgpu_lda_buffer(vbgpu_lda_t h, double **d_ptr, int64_t *n_doubles);
+/* In-place ncclAllReduce(ncclDouble, ncclSum) of that buffer, resolved at run time as for vbgpu_acc_allreduce. */
+int vbgpu_lda_allreduce(vbgpu_lda_t h, void *nccl_comm, void *stream);
 
 /* ---- Kaldi wire / disk formats on memory buffers (SURVEY.md §8f n2) ----------------------------------------------------
  * Binary forms only (what the recipes' temp files and archives hold).  Every object may carry the "\0B" marker of

@@ -112,6 +112,7 @@ _SIGS = {
     "vbgpu_feat_out_dim": (C.c_int, [_vp]),
     "vbgpu_cmvn_stats": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _vp]),
     "vbgpu_feat_run": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _vp, _i32]),
+    "vbgpu_feat_run_dev": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _vp, _i32, _vp]),
     "vbgpu_gmm_create": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _i32, C.c_int, C.POINTER(_vp)]),
     "vbgpu_gmm_destroy": (C.c_int, [_vp]),
     "vbgpu_gmm_num_pdfs": (C.c_int, [_vp]),
@@ -154,6 +155,15 @@ _SIGS = {
     "vbgpu_fmllr_accumulate_dev": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _i32, _vp, _vp]),
     "vbgpu_fmllr_download": (C.c_int, [_vp, _i32, C.POINTER(_d), _vp, _vp]),
     "vbgpu_mllt_accumulate": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, C.POINTER(_d), _vp, C.POINTER(_d)]),
+    "vbgpu_lda_create": (C.c_int, [_i32, _i32, C.c_int, C.POINTER(_vp)]),
+    "vbgpu_lda_destroy": (C.c_int, [_vp]),
+    "vbgpu_lda_zero": (C.c_int, [_vp]),
+    "vbgpu_lda_accumulate": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
+    "vbgpu_lda_accumulate_dev": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
+    "vbgpu_lda_bad_count": (C.c_int, [_vp, C.POINTER(_i64)]),
+    "vbgpu_lda_download": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "vbgpu_lda_buffer": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_i64)]),
+    "vbgpu_lda_allreduce": (C.c_int, [_vp, _vp, _vp]),
     "vbgpu_io_object_info": (C.c_int, [_vp, _i64, C.POINTER(IoInfo)]),
     "vbgpu_io_read_matrix": (C.c_int, [_vp, _i64, _vp, _i32]),
     "vbgpu_io_read_vector": (C.c_int, [_vp, _i64, _vp]),

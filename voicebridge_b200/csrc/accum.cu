@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(kWarps * 32) acc_kernel(const float *__restric
 }
 
 // ---- bucketed path ----------------------------------------------------------------------------------------------------
-constexpr int kChunk = 128;   // frames of one pdf per work unit
+constexpr int kChunk = vb::kSortChunk;  // frames of one pdf per work unit
 constexpr int kMaxM = 64;     // Gaussians per pdf served by the bucketed kernel
 // workspace (int32): count[P+1] | start[P+2] | cursor[P+1] | unit_off[P+2] | order[T]      (bin P = invalid pdf ids)
 
@@ -163,7 +163,8 @@ __global__ void acc_hist_kernel(const int32_t *__restrict__ pdf_ids, int64_t T, 
   }
 }
 
-// One block: exclusive scans of the counts (-> start, cursor) and of the units per pdf (-> unit_off).
+// One block: exclusive scans of the counts (-> start, cursor) and of the units per pdf (-> unit_off).  pdf_offsets == NULL
+// (the LDA statistics): every bin gets units.
 __global__ void acc_scan_kernel(const int32_t *__restrict__ count, const int32_t *__restrict__ pdf_offsets, int32_t P,
                                 int32_t *__restrict__ start, int32_t *__restrict__ cursor, int32_t *__restrict__ unit_off,
                                 unsigned long long *bad) {
@@ -176,7 +177,7 @@ __global__ void acc_scan_kernel(const int32_t *__restrict__ count, const int32_t
     int c = 0, u = 0;
     if (p <= P) {
       c = count[p];
-      if (p < P && pdf_offsets[p + 1] - pdf_offsets[p] <= kMaxM) u = (c + kChunk - 1) / kChunk;
+      if (p < P && (!pdf_offsets || pdf_offsets[p + 1] - pdf_offsets[p] <= kMaxM)) u = (c + kChunk - 1) / kChunk;
     }
     s_a[threadIdx.x] = c;
     s_b[threadIdx.x] = u;
@@ -446,6 +447,22 @@ __global__ void axpy_kernel(double *__restrict__ dst, const double *__restrict__
 
 namespace vb {
 
+int bin_sort_launch(const int32_t *d_ids, int64_t T, int32_t P, const int32_t *d_pdf_offsets, int device, DevBuf *work,
+                    unsigned long long *bad, cudaStream_t s, BinSort *out) {
+  const size_t n_int = (size_t)(P + 1) + (P + 2) + (P + 1) + (P + 2) + (size_t)T;
+  VB_TRY(work->reserve(n_int * 4));
+  int32_t *count = work->as<int32_t>(), *start = count + (P + 1), *cursor = start + (P + 2), *unit_off = cursor + (P + 1),
+          *order = unit_off + (P + 2);
+  VB_CUDA(cudaMemsetAsync(count, 0, (size_t)(P + 1) * 4, s));
+  const int g1 = (int)std::min<int64_t>((T + 255) / 256, (int64_t)num_sms(device) * 16);
+  acc_hist_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, count);
+  acc_scan_kernel<<<1, 1024, 0, s>>>(count, d_pdf_offsets, P, start, cursor, unit_off, bad);
+  acc_scatter_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, cursor, order);
+  VB_CUDA(cudaGetLastError());
+  *out = BinSort{start, unit_off, order};
+  return 0;
+}
+
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
                const int32_t *d_ids, const float *d_w, cudaStream_t s) {
   if (T == 0) return 0;
@@ -460,16 +477,9 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
   const bool bucket = getenv("VBGPU_ACC_FRAMEWISE") == nullptr && smem <= 200 * 1024;
   if (bucket) {
     // counting sort of the frames by pdf, then (pdf, chunk) work units
-    const size_t n_int = (size_t)(P + 1) + (P + 2) + (P + 1) + (P + 2) + (size_t)T;
-    VB_TRY(h->d_work.reserve(n_int * 4));
-    int32_t *count = h->d_work.as<int32_t>(), *start = count + (P + 1), *cursor = start + (P + 2),
-            *unit_off = cursor + (P + 1), *order = unit_off + (P + 2);
-    VB_CUDA(cudaMemsetAsync(count, 0, (size_t)(P + 1) * 4, s));
-    const int g1 = (int)std::min<int64_t>((T + 255) / 256, (int64_t)sms * 16);
-    acc_hist_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, count);
-    acc_scan_kernel<<<1, 1024, 0, s>>>(count, g->d_pdf_offsets.as<int32_t>(), P, start, cursor, unit_off,
-                                      g->d_bad.as<unsigned long long>());
-    acc_scatter_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, cursor, order);
+    BinSort bs;
+    VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), h->device, &h->d_work,
+                           g->d_bad.as<unsigned long long>(), s, &bs));
     if (!h->bucket_attr_set) {
       VB_CUDA(cudaFuncSetAttribute(acc_bucket_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       h->bucket_attr_set = true;
@@ -477,8 +487,8 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
     const int64_t max_units = (int64_t)P + T / kChunk + 1;
     const int g2 = (int)std::min<int64_t>(max_units, (int64_t)sms * 3);
     acc_bucket_kernel<<<g2, kWarps * 32, smem, s>>>(d_feats, d_feats2, stride, g->D, g->DP, DY, d_w, g->d_rows.as<float>(),
-                                                    g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, start,
-                                                    unit_off, order, h->d_acc.as<double>(),
+                                                    g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, bs.start,
+                                                    bs.unit_off, bs.order, h->d_acc.as<double>(),
                                                     g->d_bad.as<unsigned long long>(), nullptr, 0, nullptr, nullptr);
     VB_CUDA(cudaGetLastError());
     if (g->max_pdf_size <= kMaxM) return 0;
@@ -499,16 +509,9 @@ int acc_posterior_ab_launch(vbgpu_gmm_t g, DevBuf *work, const float *d_feats, i
                             const int32_t *d_ids, const float *d_w, float *d_ab, int32_t ab_pitch, float *d_cnt,
                             double *d_like, int32_t *max_gauss_served, cudaStream_t s) {
   const int P = g->P, sms = num_sms(g->device);
-  const size_t n_int = (size_t)(P + 1) + (P + 2) + (P + 1) + (P + 2) + (size_t)T;
-  VB_TRY(work->reserve(n_int * 4));
-  int32_t *count = work->as<int32_t>(), *start = count + (P + 1), *cursor = start + (P + 2), *unit_off = cursor + (P + 1),
-          *order = unit_off + (P + 2);
-  VB_CUDA(cudaMemsetAsync(count, 0, (size_t)(P + 1) * 4, s));
-  const int g1 = (int)std::min<int64_t>((T + 255) / 256, (int64_t)sms * 16);
-  acc_hist_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, count);
-  acc_scan_kernel<<<1, 1024, 0, s>>>(count, g->d_pdf_offsets.as<int32_t>(), P, start, cursor, unit_off,
-                                    g->d_bad.as<unsigned long long>());
-  acc_scatter_kernel<<<g1, 256, 0, s>>>(d_ids, T, P, cursor, order);
+  BinSort bs;
+  VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), g->device, work, g->d_bad.as<unsigned long long>(),
+                         s, &bs));
   const int DY = (g->D + 3) / 4 * 4;
   const size_t smem = ((size_t)kChunk * DY + (size_t)2 * g->D * kMP + (size_t)kChunk * kMP) * 4;
   // (per device: set on every call — a process may drive several GPUs, and the call costs microseconds)
@@ -516,8 +519,8 @@ int acc_posterior_ab_launch(vbgpu_gmm_t g, DevBuf *work, const float *d_feats, i
   const int64_t max_units = (int64_t)P + T / kChunk + 1;
   const int g2 = (int)std::min<int64_t>(max_units, (int64_t)sms * 3);
   acc_bucket_kernel<<<g2, kWarps * 32, smem, s>>>(d_feats, nullptr, stride, g->D, g->DP, DY, d_w, g->d_rows.as<float>(),
-                                                  g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, start,
-                                                  unit_off, order, nullptr, g->d_bad.as<unsigned long long>(), d_ab, ab_pitch,
+                                                  g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, bs.start,
+                                                  bs.unit_off, bs.order, nullptr, g->d_bad.as<unsigned long long>(), d_ab, ab_pitch,
                                                   d_cnt, d_like);
   VB_CUDA(cudaGetLastError());
   *max_gauss_served = kMaxM;

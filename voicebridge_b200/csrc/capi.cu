@@ -547,18 +547,38 @@ static int check_fmllr(vbgpu_feat_t h, const float *fmllr, int32_t fmllr_cols) {
   return 0;
 }
 
-int vbgpu_feat_run(vbgpu_feat_t h, const float *feats, int32_t in_stride, const int64_t *frame_offsets, int32_t n_utts,
-                   const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats, const float *fmllr,
-                   int32_t fmllr_cols, float *out, int32_t out_stride) {
+static int check_feat_run(vbgpu_feat_t h, int32_t in_stride, const int64_t *frame_offsets, int32_t n_utts,
+                          const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats, const float *fmllr,
+                          int32_t fmllr_cols, int32_t out_stride) {
   VB_CHECK(h && frame_offsets && n_utts >= 0 && n_spk >= 0, "bad argument");
   VB_CHECK(in_stride >= h->in_dim, "in_stride %d < dim %d", in_stride, h->in_dim);
   VB_CHECK(out_stride >= h->out_dim, "out_stride %d < out dim %d", out_stride, h->out_dim);
-  const bool need_stats = h->opts.norm_means || h->opts.norm_vars;
-  VB_CHECK(!need_stats || cmvn_stats, "cmvn_stats is null but normalisation is requested");
+  VB_CHECK(!(h->opts.norm_means || h->opts.norm_vars) || cmvn_stats, "cmvn_stats is null but normalisation is requested");
   VB_TRY(check_spk(utt2spk, n_utts, n_spk));
   VB_TRY(check_fmllr(h, fmllr, fmllr_cols));
+  if (n_utts > 0) VB_CHECK(frame_offsets[0] == 0, "frame_offsets[0] must be 0");
+  return 0;
+}
+
+// Shared by vbgpu_feat_run and vbgpu_feat_run_dev once the layout is on the device: host CMVN statistics -> norm table,
+// then the feature kernel from d_in to d_out, on stream s.
+static int feat_run_device(vbgpu_feat_t h, const float *d_in, int32_t in_stride, int32_t n_spk, const double *cmvn_stats,
+                           bool check_stats, const float *d_fmllr, int32_t fmllr_cols, float *d_out, int32_t out_stride,
+                           cudaStream_t s) {
+  if (h->opts.norm_means || h->opts.norm_vars) {
+    const size_t nst = (size_t)n_spk * 2 * (h->in_dim + 1);
+    VB_TRY(h->d_stats.reserve(nst * 8));
+    VB_TRY(h2d(h->d_stats.p, cmvn_stats, nst * 8, s));
+    VB_TRY(feat_norm_from_stats(h, h->d_stats.as<double>(), n_spk, check_stats, s));
+  }
+  return feat_launch(h, d_in, in_stride, d_fmllr, fmllr_cols, d_out, out_stride, s);
+}
+
+int vbgpu_feat_run(vbgpu_feat_t h, const float *feats, int32_t in_stride, const int64_t *frame_offsets, int32_t n_utts,
+                   const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats, const float *fmllr,
+                   int32_t fmllr_cols, float *out, int32_t out_stride) {
+  VB_TRY(check_feat_run(h, in_stride, frame_offsets, n_utts, utt2spk, n_spk, cmvn_stats, fmllr, fmllr_cols, out_stride));
   if (n_utts == 0) return 0;
-  VB_CHECK(frame_offsets[0] == 0, "frame_offsets[0] must be 0");
   DeviceGuard g(h->device);
   cudaStream_t s = h->stream;
   VB_TRY(h->layout.update(nullptr, frame_offsets, n_utts, utt2spk, nullptr, s));
@@ -568,12 +588,6 @@ int vbgpu_feat_run(vbgpu_feat_t h, const float *feats, int32_t in_stride, const 
   VB_TRY(h->d_in.reserve((size_t)T * in_stride * 4));
   VB_TRY(h->d_out.reserve((size_t)T * out_stride * 4));
   VB_TRY(h2d(h->d_in.p, feats, (size_t)T * in_stride * 4, s));
-  if (need_stats) {
-    const size_t nst = (size_t)n_spk * 2 * (h->in_dim + 1);
-    VB_TRY(h->d_stats.reserve(nst * 8));
-    VB_TRY(h2d(h->d_stats.p, cmvn_stats, nst * 8, s));
-    VB_TRY(feat_norm_from_stats(h, h->d_stats.as<double>(), n_spk, true, s));
-  }
   const float *d_fm = nullptr;
   if (fmllr) {
     const size_t nb = (size_t)n_spk * h->out_dim * fmllr_cols * 4;
@@ -581,10 +595,37 @@ int vbgpu_feat_run(vbgpu_feat_t h, const float *feats, int32_t in_stride, const 
     VB_TRY(h2d(h->d_fmllr.p, fmllr, nb, s));
     d_fm = h->d_fmllr.as<float>();
   }
-  VB_TRY(feat_launch(h, h->d_in.as<float>(), in_stride, d_fm, fmllr_cols, h->d_out.as<float>(), out_stride, s));
+  VB_TRY(feat_run_device(h, h->d_in.as<float>(), in_stride, n_spk, cmvn_stats, true, d_fm, fmllr_cols,
+                         h->d_out.as<float>(), out_stride, s));
   VB_TRY(d2h(out, h->d_out.p, (size_t)T * out_stride * 4, s));
   VB_CUDA(cudaStreamSynchronize(s));
   return 0;
+}
+
+int vbgpu_feat_run_dev(vbgpu_feat_t h, const float *d_feats, int32_t in_stride, const int64_t *frame_offsets,
+                       int32_t n_utts, const int32_t *utt2spk, int32_t n_spk, const double *cmvn_stats,
+                       const float *d_fmllr, int32_t fmllr_cols, float *d_out, int32_t out_stride, void *stream) {
+  VB_TRY(check_feat_run(h, in_stride, frame_offsets, n_utts, utt2spk, n_spk, cmvn_stats, d_fmllr, fmllr_cols,
+                        out_stride));
+  if (n_utts == 0 || frame_offsets[n_utts] == 0) return 0;
+  VB_CHECK(d_feats && d_out, "null buffer");
+  if (h->opts.norm_means || h->opts.norm_vars) {
+    // the statistics are on the host: reject what cmvn_norm_kernel would flag (count < 1, cmvn.cc:80-82) without a
+    // round trip, so that the call stays asynchronous
+    const int32_t w = 2 * (h->in_dim + 1);
+    for (int32_t k = 0; k < n_spk; k++) {
+      const double *st = cmvn_stats + (size_t)k * w;
+      bool ok = st[h->in_dim] >= 1.0;
+      for (int32_t i = 0; i < w && ok; i++) ok = std::isfinite(st[i]);
+      if (!ok) return fail(VBGPU_ERR_NUMERIC, "insufficient or degenerate CMVN stats for speaker %d (count < 1 or NaN)", k);
+    }
+  }
+  DeviceGuard g(h->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  VB_TRY(h->order.enter(s));  // batch layout, statistics and norm table of the handle
+  VB_TRY(h->layout.update(nullptr, frame_offsets, n_utts, utt2spk, nullptr, s));
+  VB_TRY(feat_run_device(h, d_feats, in_stride, n_spk, cmvn_stats, false, d_fmllr, fmllr_cols, d_out, out_stride, s));
+  return h->order.leave(s);
 }
 
 // ================================================================================================================
@@ -1160,8 +1201,9 @@ int vbgpu_acc_buffer(vbgpu_acc_t h, double **d_ptr, int64_t *n_doubles) {
   return 0;
 }
 
-int vbgpu_acc_allreduce(vbgpu_acc_t h, void *nccl_comm, void *stream) {
-  VB_CHECK(h && nccl_comm, "null argument");
+// In-place ncclAllReduce(ncclDouble, ncclSum) of n doubles on `device`.  libnccl is looked up at run time (already loaded
+// by the caller, else dlopen), so the library has no link-time NCCL dependency.
+static int nccl_allreduce_sum_f64(double *buf, int64_t n, int device, void *nccl_comm, void *stream) {
   typedef int (*allreduce_fn)(const void *, void *, size_t, int, int, void *, cudaStream_t);
   static allreduce_fn fn = nullptr;
   if (!fn) {
@@ -1172,12 +1214,16 @@ int vbgpu_acc_allreduce(vbgpu_acc_t h, void *nccl_comm, void *stream) {
     }
     if (!fn) return fail(VBGPU_ERR_INVALID, "ncclAllReduce not found: load libnccl.so.2 before calling");
   }
-  DeviceGuard g(h->device);
+  DeviceGuard g(device);
   const int ncclDouble = 8, ncclSum = 0;
-  int rc = fn(h->d_acc.p, h->d_acc.p, (size_t)h->n_doubles, ncclDouble, ncclSum, nccl_comm,
-              static_cast<cudaStream_t>(stream));
+  int rc = fn(buf, buf, (size_t)n, ncclDouble, ncclSum, nccl_comm, static_cast<cudaStream_t>(stream));
   if (rc != 0) return fail(VBGPU_ERR_CUDA, "ncclAllReduce returned %d", rc);
   return 0;
+}
+
+int vbgpu_acc_allreduce(vbgpu_acc_t h, void *nccl_comm, void *stream) {
+  VB_CHECK(h && nccl_comm, "null argument");
+  return nccl_allreduce_sum_f64(h->d_acc.as<double>(), h->n_doubles, h->device, nccl_comm, stream);
 }
 
 int vbgpu_acc_add(vbgpu_acc_t h, double scale, vbgpu_acc_t other) {
@@ -1205,6 +1251,140 @@ int vbgpu_acc_download(vbgpu_acc_t h, double *occ, double *mean_acc, double *var
   if (tot_like) *tot_like = tail[0];
   if (tot_frames) *tot_frames = tail[1];
   return 0;
+}
+
+// ================================================================================================================
+// LDA class statistics
+// ================================================================================================================
+int vbgpu_lda_create(int32_t num_classes, int32_t dim, int device, vbgpu_lda_t *out) {
+  VB_CHECK(out, "null argument");
+  *out = nullptr;
+  VB_CHECK(num_classes >= 1, "num_classes %d < 1", num_classes);
+  VB_CHECK(dim >= 1 && dim <= 256, "dim %d outside 1 ... 256", dim);
+  VB_TRY(check_device(device));
+  DeviceGuard g(device);
+  vbgpu_lda_s *h = new vbgpu_lda_s;
+  h->device = device;
+  h->C = num_classes;
+  h->D = dim;
+  h->n_doubles = (int64_t)num_classes * (dim + 1) + (int64_t)dim * (dim + 1) / 2;
+  int rc = 0;
+  cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+  if (e != cudaSuccess) rc = fail(VBGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+  if (rc == 0) rc = h->d_acc.reserve((size_t)h->n_doubles * 8);
+  if (rc == 0) rc = h->d_bad.reserve(8);
+  if (rc == 0 && (cudaMemset(h->d_acc.p, 0, (size_t)h->n_doubles * 8) != cudaSuccess ||
+                  cudaMemset(h->d_bad.p, 0, 8) != cudaSuccess))
+    rc = fail(VBGPU_ERR_CUDA, "cudaMemset failed");
+  if (rc < 0) {
+    vbgpu_lda_destroy(h);
+    return rc;
+  }
+  *out = h;
+  return 0;
+}
+
+int vbgpu_lda_destroy(vbgpu_lda_t h) {
+  if (!h) return 0;
+  h->order.release();
+  DeviceGuard g(h->device);
+  if (h->stream) cudaStreamSynchronize(h->stream);
+  for (DevBuf *b : {&h->d_acc, &h->d_bad, &h->d_work, &h->d_feats, &h->d_ids, &h->d_w}) b->release();
+  if (h->stream) cudaStreamDestroy(h->stream);
+  delete h;
+  return 0;
+}
+
+int vbgpu_lda_zero(vbgpu_lda_t h) {
+  VB_CHECK(h, "null handle");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  VB_CUDA(cudaMemset(h->d_acc.p, 0, (size_t)h->n_doubles * 8));
+  return 0;
+}
+
+static int check_lda_args(vbgpu_lda_t h, const float *feats, int64_t T, int32_t stride, const int32_t *ids) {
+  VB_CHECK(h && T >= 0, "bad argument");
+  VB_CHECK(stride >= h->D, "stride %d < dim %d", stride, h->D);
+  VB_CHECK(T == 0 || (feats && ids), "null buffer");
+  return 0;
+}
+
+int vbgpu_lda_accumulate_dev(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_class_ids,
+                             const float *d_weights, void *stream) {
+  VB_TRY(check_lda_args(h, d_feats, T, stride, d_class_ids));
+  if (T == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  VB_TRY(h->order.enter(s));  // the counting-sort work space
+  VB_TRY(lda_launch(h, d_feats, T, stride, d_class_ids, d_weights, s));
+  return h->order.leave(s);
+}
+
+int vbgpu_lda_accumulate(vbgpu_lda_t h, const float *feats, int64_t T, int32_t stride, const int32_t *class_ids,
+                         const float *weights) {
+  VB_TRY(check_lda_args(h, feats, T, stride, class_ids));
+  if (T == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->stream;
+  VB_TRY(h->order.enter(s));
+  const size_t fb = (size_t)T * stride * 4;
+  VB_TRY(h->d_feats.reserve(fb));
+  VB_TRY(h->d_ids.reserve((size_t)T * 4));
+  VB_TRY(h2d(h->d_feats.p, feats, fb, s));
+  VB_TRY(h2d(h->d_ids.p, class_ids, (size_t)T * 4, s));
+  const float *d_w = nullptr;
+  if (weights) {
+    VB_TRY(h->d_w.reserve((size_t)T * 4));
+    VB_TRY(h2d(h->d_w.p, weights, (size_t)T * 4, s));
+    d_w = h->d_w.as<float>();
+  }
+  // this call's invalid ids only: the count of earlier _dev calls is kept for vbgpu_lda_bad_count
+  unsigned long long before = 0, after = 0;
+  VB_CUDA(cudaMemcpyAsync(&before, h->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
+  VB_TRY(lda_launch(h, h->d_feats.as<float>(), T, stride, h->d_ids.as<int32_t>(), d_w, s));
+  VB_CUDA(cudaMemcpyAsync(&after, h->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
+  VB_CUDA(cudaStreamSynchronize(s));
+  VB_CUDA(cudaMemcpy(h->d_bad.p, &before, 8, cudaMemcpyHostToDevice));
+  VB_TRY(h->order.leave(s));
+  if (after != before)
+    return fail(VBGPU_ERR_NUMERIC, "%llu frames had a class id outside [0, %d)", after - before, h->C);
+  return 0;
+}
+
+int vbgpu_lda_bad_count(vbgpu_lda_t h, int64_t *count) {
+  VB_CHECK(h && count, "null argument");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  unsigned long long v = 0;
+  VB_CUDA(cudaMemcpy(&v, h->d_bad.p, 8, cudaMemcpyDeviceToHost));
+  VB_CUDA(cudaMemset(h->d_bad.p, 0, 8));
+  *count = (int64_t)v;
+  return 0;
+}
+
+int vbgpu_lda_download(vbgpu_lda_t h, double *zero, double *first, double *second) {
+  VB_CHECK(h, "null handle");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  const size_t C = h->C, D = h->D;
+  const double *a = h->d_acc.as<double>();
+  if (zero) VB_CUDA(cudaMemcpy(zero, a, C * 8, cudaMemcpyDeviceToHost));
+  if (first) VB_CUDA(cudaMemcpy(first, a + C, C * D * 8, cudaMemcpyDeviceToHost));
+  if (second) VB_CUDA(cudaMemcpy(second, a + C + C * D, D * (D + 1) / 2 * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int vbgpu_lda_buffer(vbgpu_lda_t h, double **d_ptr, int64_t *n_doubles) {
+  VB_CHECK(h && d_ptr && n_doubles, "null argument");
+  *d_ptr = h->d_acc.as<double>();
+  *n_doubles = h->n_doubles;
+  return 0;
+}
+
+int vbgpu_lda_allreduce(vbgpu_lda_t h, void *nccl_comm, void *stream) {
+  VB_CHECK(h && nccl_comm, "null argument");
+  return nccl_allreduce_sum_f64(h->d_acc.as<double>(), h->n_doubles, h->device, nccl_comm, stream);
 }
 
 // ================================================================================================================

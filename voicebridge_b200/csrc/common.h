@@ -215,6 +215,18 @@ struct vbgpu_acc_s {
   bool bucket_attr_set = false;
 };
 
+struct vbgpu_lda_s {
+  vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
+  int device = 0;
+  cudaStream_t stream = nullptr;
+  int32_t C = 0, D = 0;
+  int64_t n_doubles = 0;  // C + C*D + D(D+1)/2
+  vb::DevBuf d_acc;       // [zero C | first C*D | second D(D+1)/2, SpMatrix packing]
+  vb::DevBuf d_bad;       // uint64 count of invalid class ids since the last query
+  vb::DevBuf d_work;      // counting-sort workspace
+  vb::DevBuf d_feats, d_ids, d_w;  // staging of the host entry point
+};
+
 struct vbgpu_pipeline_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_t mfcc = nullptr;
@@ -265,6 +277,20 @@ int sparse_subset_launch(const float *d_slab, int32_t slab_stride, int64_t t0, i
                          const int64_t *d_out_offsets, float *d_out, cudaStream_t s);
 int sparse_gather_launch(const float *d_slab, int32_t slab_stride, int64_t t0, int64_t t1, const int32_t *d_frames,
                          const int32_t *d_cols, int64_t n, float *d_out, cudaStream_t s);
+
+// Counting sort of T frames by bin id (pdf or class) in [0, P): ids outside go to bin P, which gets no work units, and
+// are added to *bad.  Bin p then owns order[start[p] .. start[p+1]) and work units [unit_off[p], unit_off[p+1]) of up to
+// kSortChunk frames each; unit_off[P+1] is the total.  With d_pdf_offsets, only pdfs of at most 64 Gaussians get units
+// (the bucketed EM kernel's limit); NULL gives every bin its units.  work is the caller's (grown as needed).
+constexpr int kSortChunk = 128;
+struct BinSort {
+  const int32_t *start, *unit_off, *order;
+};
+int bin_sort_launch(const int32_t *d_ids, int64_t T, int32_t P, const int32_t *d_pdf_offsets, int device, DevBuf *work,
+                    unsigned long long *bad, cudaStream_t s, BinSort *out);
+
+int lda_launch(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_ids, const float *d_w,
+               cudaStream_t s);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
                const int32_t *d_ids, const float *d_w, cudaStream_t s);

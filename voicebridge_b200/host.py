@@ -8,6 +8,7 @@ Class / method names and argument meaning follow the Kaldi types VoiceBridge lin
   AmDiagGmmGpu             AmDiagGmm                                 gmm/am-diag-gmm.h:36-105
   DecodableAmDiagGmmGpu    DecodableAmDiagGmmScaled                  gmm/decodable-am-diag-gmm.h:121-160
   AccumAmDiagGmmGpu        AccumAmDiagGmm                            gmm/mle-am-diag-gmm.h:34-108
+  LdaEstimateGpu           LdaEstimate (accumulation)                transform/lda-estimate.h
   ScoringPipeline          the fused PCM -> loglikes job (compute-mfcc-feats ... gmm-latgen-faster's decodable)
 
 Errors surface as capi.VbgpuError (the reference throws std::runtime_error from KALDI_ERR).
@@ -336,6 +337,20 @@ class FeaturePipeline(_Handle):
                                         n_spk, _ptr(st), _ptr(fm), fcols, out.ctypes.data, ost))
         return out[:T, :OD]
 
+    def run_dev(self, d_feats, in_stride, frame_offsets, d_out, out_stride, utt2spk=None, n_spk=None, cmvn_stats=None,
+                d_fmllr=None, fmllr_cols=0, stream=None):
+        """vbgpu_feat_run_dev: device features in and out (d_out [T x out_stride]); frame_offsets, utt2spk and cmvn_stats
+        are host arrays.  Enqueued on `stream` (default: torch's current stream)."""
+        fo = _np(frame_offsets, np.int64)
+        n_utts = len(fo) - 1
+        u2s = _np(utt2spk, np.int32) if utt2spk is not None else None
+        if n_spk is None:
+            n_spk = n_utts if u2s is None else int(u2s.max()) + 1 if len(u2s) else 0
+        st = _np(cmvn_stats, np.float64) if cmvn_stats is not None else None
+        check(capi.lib().vbgpu_feat_run_dev(self.h, _ptr(d_feats), in_stride, fo.ctypes.data, n_utts, _ptr(u2s), n_spk,
+                                            _ptr(st), _ptr(d_fmllr), fmllr_cols, _ptr(d_out), out_stride,
+                                            _stream_ptr(stream)))
+
 
 class AmDiagGmmGpu(_Handle):
     """Device-resident AmDiagGmm, flattened: pdf p owns Gaussians [pdf_offsets[p], pdf_offsets[p+1])."""
@@ -627,6 +642,68 @@ class MlltAccsGpu:
                                                _ptr(w), C.byref(beta), self.G.ctypes.data, C.byref(tl)))
         self.beta = beta.value
         return tl.value
+
+
+class LdaEstimateGpu(_Handle):
+    """The accumulation half of LdaEstimate (transform/lda-estimate.h): zero-, first- and second-order class statistics in
+    one FP64 device buffer [zero C | first C*D | second D(D+1)/2].  Every frame is accumulated (no rand_prune); the solver
+    (LdaEstimate::Estimate) stays on the host: hand it stats()."""
+    _destroy = "vbgpu_lda_destroy"
+
+    def __init__(self, num_classes, dim, device=0):
+        super().__init__()
+        self.C, self.D, self.device = int(num_classes), int(dim), int(device)
+        check(capi.lib().vbgpu_lda_create(self.C, self.D, self.device, C.byref(self.h)))
+
+    def NumClasses(self):
+        return self.C
+
+    def Dim(self):
+        return self.D
+
+    def ZeroAccumulators(self):
+        check(capi.lib().vbgpu_lda_zero(self.h))
+
+    def Accumulate(self, feats, class_ids, weights=None):
+        """Accumulate(row t, class_ids[t], weights[t] or 1.0) for every row; a weight of 0 skips the frame.  Raises
+        VbgpuError (ERR_NUMERIC) after adding every valid frame when a class id is outside [0, NumClasses())."""
+        feats = _np(feats, np.float32)
+        ids = _np(class_ids, np.int32)
+        w = _np(weights, np.float32) if weights is not None else None
+        check(capi.lib().vbgpu_lda_accumulate(self.h, feats.ctypes.data, feats.shape[0], feats.shape[1], ids.ctypes.data,
+                                              _ptr(w)))
+
+    def accumulate_dev(self, d_feats, T, stride, d_class_ids, d_weights=None, stream=None):
+        check(capi.lib().vbgpu_lda_accumulate_dev(self.h, _ptr(d_feats), T, stride, _ptr(d_class_ids), _ptr(d_weights),
+                                                  _stream_ptr(stream)))
+
+    def bad_count(self):
+        """Invalid class ids seen by accumulate_dev since the last query (the count is reset)."""
+        n = C.c_int64(0)
+        check(capi.lib().vbgpu_lda_bad_count(self.h, C.byref(n)))
+        return n.value
+
+    def stats(self):
+        """(zero[C], first[C, D], second packed [D(D+1)/2], SpMatrix order)."""
+        zero, first, second = np.zeros(self.C), np.zeros((self.C, self.D)), np.zeros(self.D * (self.D + 1) // 2)
+        check(capi.lib().vbgpu_lda_download(self.h, zero.ctypes.data, first.ctypes.data, second.ctypes.data))
+        return zero, first, second
+
+    def TotCount(self):
+        zero = np.zeros(self.C)
+        check(capi.lib().vbgpu_lda_download(self.h, zero.ctypes.data, None, None))
+        return float(zero.sum())
+
+    def buffer(self):
+        """(device pointer, n_doubles) of [zero | first | second]."""
+        p, n = C.c_void_p(), C.c_int64(0)
+        check(capi.lib().vbgpu_lda_buffer(self.h, C.byref(p), C.byref(n)))
+        return p.value, n.value
+
+    def allreduce(self, comm, stream=None):
+        """In-place sum all-reduce of the statistics over a raw ncclComm_t (replaces est-lda summing the job files)."""
+        c = comm.value if isinstance(comm, C.c_void_p) else comm
+        check(capi.lib().vbgpu_lda_allreduce(self.h, c, _stream_ptr(stream)))
 
 
 class ScoringPipeline(_Handle):
