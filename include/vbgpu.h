@@ -27,6 +27,9 @@
  *   vbgpu_lda_*       replaces  LdaEstimate::Init / ZeroAccumulators / Accumulate (LDA class statistics of acc-lda)
  *                               transform/lda-estimate.{h,cc} (caller VB/scr/steps/train_lda_mllt.cpp) and the summing of
  *                               the per-job lda.*.acc files by est-lda (vbgpu_lda_allreduce)
+ *   vbgpu_tree_*      replaces  AccumulateTreeStats (tree statistics of acc-tree-stats, with SplitToPhones / IsReordered)
+ *                               hmm/tree-accu.cc, hmm/hmm-utils.cc, tree/clusterable-classes.cc (callers train_deltas,
+ *                               train_lda_mllt, train_sat) and the summing of the per-job treeacc files (sum-tree-stats)
  *   vbgpu_io_*        reads / writes  Matrix / CompressedMatrix / Vector / int32-vector objects, archive entries, model
  *                               files (-> tid2pdf + flattened AmDiagGmm) and gmm-acc-stats-ali statistics files
  *                               matrix/kaldi-matrix.cc:1375-1460, matrix/compressed-matrix.cc:531-670, gmm/diag-gmm.cc:705-756
@@ -115,6 +118,7 @@ typedef struct vbgpu_fmllr_s *vbgpu_fmllr_t;
 typedef struct vbgpu_pipeline_s *vbgpu_pipeline_t;
 typedef struct vbgpu_pitch_s *vbgpu_pitch_t;
 typedef struct vbgpu_lda_s *vbgpu_lda_t;
+typedef struct vbgpu_tree_s *vbgpu_tree_t;
 
 /* ---- library ------------------------------------------------------------------------------------------------ */
 int vbgpu_version(void);
@@ -373,6 +377,60 @@ int vbgpu_lda_buffer(vbgpu_lda_t h, double **d_ptr, int64_t *n_doubles);
 /* In-place ncclAllReduce(ncclDouble, ncclSum) of that buffer, resolved at run time as for vbgpu_acc_allreduce. */
 int vbgpu_lda_allreduce(vbgpu_lda_t h, void *nccl_comm, void *stream);
 
+/* ---- tree statistics (acc-tree-stats) -----------------------------------------------------------------------------------
+ * AccumulateTreeStats (hmm/tree-accu.cc) for a packed batch of whole utterances: transition-ids tids[T] (one per feature
+ * row) and rows [frame_offsets[u], frame_offsets[u+1]) of utterance u.  Each alignment is split into phones as
+ * SplitToPhones does (hmm/hmm-utils.cc; reordered or not as IsReordered finds); an alignment it calls bad (or one holding a
+ * transition-id outside [1, num_tids]) adds nothing, its rows are never read, and it is counted.  Every frame of a good
+ * utterance adds GaussClusterable::AddStats(row, 1.0) to its key: count += 1, sum_x += x, sum_x2 += x * x, all FP64.
+ * The key (EventType) of a frame in phone segment s: (kPdfClass = -1, pdf-class of its transition-id) and (j, phone of
+ * segment s - P + j, 0 outside the utterance) for j = 0 ... N-1, or only (P, central phone) when the central phone is
+ * one of ci_phones.  No --phone-map, no frame weights.
+ * Limits, checked at create: N <= 4, P < N, phones 1 ... 4095, pdf-classes 0 ... 255, dim 1 ... 256.
+ * Keys live in a device hash table of max_keys entries; frames whose key finds no room add nothing and are counted.
+ * Every accumulate call sorts frames over the whole id range, at a cost that grows with max_keys: size it to the expected
+ * key count (vbgpu_tree_num_keys after a first job tells it). */
+#define VBGPU_TID_SELF_LOOP 1       /* IsSelfLoop: the transition's destination is its own hmm-state */
+#define VBGPU_TID_FINAL 2           /* IsFinal: destination + 1 == the number of states of the phone's topology entry */
+#define VBGPU_TID_STATE0_EMITTING 4 /* state 0 of the phone's topology entry has forward_pdf_class != kNoPdf */
+/* Per transition-id tables (vbgpu_io_mdl_transitions fills them from a model file): arrays of num_tids + 1, entry 0
+ * unused (transition-ids are 1-based).  pdf_class is the state's self_loop_pdf_class for a self-loop, else its
+ * forward_pdf_class; trans_state is the 1-based transition state (tuple index). */
+typedef struct vbgpu_tid_tables {
+  int32_t num_tids;
+  const int32_t *phone, *hmm_state, *pdf_class, *trans_state, *flags;
+} vbgpu_tid_tables;
+typedef struct vbgpu_tree_opts {
+  int32_t context_width;     /* N (acc-tree-stats --context-width, default 3) */
+  int32_t central_position;  /* P (--central-position, default 1) */
+  const int32_t *ci_phones;  /* --ci-phones, sorted ascending; may be NULL when num_ci_phones == 0 */
+  int32_t num_ci_phones;
+} vbgpu_tree_opts;
+int vbgpu_tree_create(const vbgpu_tree_opts *opts, const vbgpu_tid_tables *tables, int32_t dim, int32_t max_keys,
+                      int device, vbgpu_tree_t *out);
+int vbgpu_tree_destroy(vbgpu_tree_t h);
+int vbgpu_tree_zero(vbgpu_tree_t h); /* empties the statistics and the key table */
+/* Host form, synchronous: feats [T x stride], tids[T], T = frame_offsets[n_utts].  Returns VBGPU_ERR_NUMERIC after adding
+ * everything else when some frame of this call found no room in the key table. */
+int vbgpu_tree_accumulate(vbgpu_tree_t h, const float *feats, int32_t stride, const int32_t *tids,
+                          const int64_t *frame_offsets, int32_t n_utts);
+/* Device form: d_feats and d_tids on the device, frame_offsets on the host (the batch layout is cached). */
+int vbgpu_tree_accumulate_dev(vbgpu_tree_t h, const float *d_feats, int32_t stride, const int32_t *d_tids,
+                              const int64_t *frame_offsets, int32_t n_utts, void *stream);
+/* Bad utterances (dropped as "alignment appears to be bad") and frames without room in the key table, over every
+ * accumulate call since the last query; resets both (synchronises the handle's work).  Either output may be NULL. */
+int vbgpu_tree_bad_count(vbgpu_tree_t h, int64_t *bad_utterances, int64_t *dropped_frames);
+int vbgpu_tree_num_keys(vbgpu_tree_t h, int32_t *num_keys);
+/* The K = num_keys statistics in the order std::map<EventType, GaussClusterable*> iterates them (what acc-tree-stats
+ * writes): pdf_class[K], phones[K x N] (-1 where the EventType has no such position), count[K], sum_x[K x D],
+ * sum_x2[K x D].  Any output may be NULL. */
+int vbgpu_tree_download(vbgpu_tree_t h, int32_t *pdf_class, int32_t *phones, double *count, double *sum_x,
+                        double *sum_x2);
+/* Adds n entries in the layout of vbgpu_tree_download, key by key (sum-tree-stats; merging the handles of several GPUs,
+ * whose keys differ).  Returns VBGPU_ERR_NUMERIC when some entry found no room in the key table. */
+int vbgpu_tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t *phones, const double *count,
+                   const double *sum_x, const double *sum_x2);
+
 /* ---- Kaldi wire / disk formats on memory buffers (SURVEY.md §8f n2) ----------------------------------------------------
  * Binary forms only (what the recipes' temp files and archives hold).  Every object may carry the "\0B" marker of
  * WriteKaldiObject / the table holders in front. */
@@ -403,6 +461,11 @@ int vbgpu_io_ark_next(const void *buf, int64_t n, int64_t pos, char *key, int32_
 int vbgpu_io_mdl_info(const void *buf, int64_t n, int32_t *dim, int32_t *num_pdfs, int32_t *num_gauss, int32_t *num_tids);
 int vbgpu_io_mdl_read(const void *buf, int64_t n, int32_t *pdf_offsets, float *gconsts, float *weights,
                       float *means_invvars, float *inv_vars, int32_t *tid2pdf, float *trans_log_probs);
+/* The per transition-id tables of the model file's TransitionModel (the arrays of vbgpu_tid_tables, num_tids + 1 each,
+ * entry 0 unused), from its topology (forward / self-loop pdf classes, transitions) and <Triples> or <Tuples>.  Returns
+ * num_tids; any output may be NULL. */
+int vbgpu_io_mdl_transitions(const void *buf, int64_t n, int32_t *phone, int32_t *hmm_state, int32_t *pdf_class,
+                             int32_t *trans_state, int32_t *flags);
 /* A statistics file as gmm-acc-stats-ali writes it (gmm-acc-stats-ali.cpp:124-128): transition accs (n_trans may be 0)
  * + AccumAmDiagGmm::Write with flags kGmmAll, doubles narrowed to float (mle-diag-gmm.cc:86-101). */
 int64_t vbgpu_io_write_acc(int32_t num_pdfs, int32_t dim, const int32_t *pdf_offsets, const double *trans_accs,

@@ -74,6 +74,20 @@ class IoInfo(C.Structure):
                 ("range", C.c_float), ("header_bytes", C.c_int64), ("total_bytes", C.c_int64)]
 
 
+class TidTables(C.Structure):
+    """vbgpu_tid_tables: per transition-id arrays of num_tids + 1 (entry 0 unused)."""
+    _fields_ = [("num_tids", C.c_int32), ("phone", _vp), ("hmm_state", _vp), ("pdf_class", _vp), ("trans_state", _vp),
+                ("flags", _vp)]
+
+
+class TreeOpts(C.Structure):
+    """vbgpu_tree_opts (acc-tree-stats --context-width / --central-position / --ci-phones)."""
+    _fields_ = [("context_width", C.c_int32), ("central_position", C.c_int32), ("ci_phones", _vp),
+                ("num_ci_phones", C.c_int32)]
+
+
+TID_SELF_LOOP, TID_FINAL, TID_STATE0_EMITTING = 1, 2, 4
+
 # name -> (restype, argtypes).  Pointers to data are passed as void* (integers / numpy .ctypes.data / torch .data_ptr()).
 _SIGS = {
     "vbgpu_version": (C.c_int, []),
@@ -164,6 +178,15 @@ _SIGS = {
     "vbgpu_lda_download": (C.c_int, [_vp, _vp, _vp, _vp]),
     "vbgpu_lda_buffer": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_i64)]),
     "vbgpu_lda_allreduce": (C.c_int, [_vp, _vp, _vp]),
+    "vbgpu_tree_create": (C.c_int, [C.POINTER(TreeOpts), C.POINTER(TidTables), _i32, _i32, C.c_int, C.POINTER(_vp)]),
+    "vbgpu_tree_destroy": (C.c_int, [_vp]),
+    "vbgpu_tree_zero": (C.c_int, [_vp]),
+    "vbgpu_tree_accumulate": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i32]),
+    "vbgpu_tree_accumulate_dev": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i32, _vp]),
+    "vbgpu_tree_bad_count": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
+    "vbgpu_tree_num_keys": (C.c_int, [_vp, C.POINTER(_i32)]),
+    "vbgpu_tree_download": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "vbgpu_tree_add": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "vbgpu_io_object_info": (C.c_int, [_vp, _i64, C.POINTER(IoInfo)]),
     "vbgpu_io_read_matrix": (C.c_int, [_vp, _i64, _vp, _i32]),
     "vbgpu_io_read_vector": (C.c_int, [_vp, _i64, _vp]),
@@ -173,6 +196,7 @@ _SIGS = {
     "vbgpu_io_ark_next": (C.c_int, [_vp, _i64, _i64, _vp, _i32, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(IoInfo)]),
     "vbgpu_io_mdl_info": (C.c_int, [_vp, _i64, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32)]),
     "vbgpu_io_mdl_read": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "vbgpu_io_mdl_transitions": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "vbgpu_io_write_acc": (_i64, [_i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _d, _d, _vp, _i64]),
     "vbgpu_io_matrix_to_device": (C.c_int, [_vp, _i64, _vp, _i32, _vp, _i64, _vp]),
     "vbgpu_pipeline_create": (C.c_int, [_vp, _vp, _vp, C.POINTER(_vp)]),

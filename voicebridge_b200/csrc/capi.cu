@@ -1388,6 +1388,145 @@ int vbgpu_lda_allreduce(vbgpu_lda_t h, void *nccl_comm, void *stream) {
 }
 
 // ================================================================================================================
+// Tree statistics (kernels and the key layout in tree.cu)
+// ================================================================================================================
+int vbgpu_tree_create(const vbgpu_tree_opts *opts, const vbgpu_tid_tables *tables, int32_t dim, int32_t max_keys,
+                      int device, vbgpu_tree_t *out) {
+  VB_CHECK(out, "null argument");
+  *out = nullptr;
+  VB_TRY(tree_check(opts, tables, dim, max_keys));
+  VB_TRY(check_device(device));
+  DeviceGuard g(device);
+  vbgpu_tree_s *h = new vbgpu_tree_s;
+  h->device = device;
+  h->D = dim;
+  h->max_keys = max_keys;
+  int rc = 0;
+  cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+  if (e != cudaSuccess) rc = fail(VBGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+  if (rc == 0) rc = tree_init(h, opts, tables);
+  if (rc < 0) {
+    vbgpu_tree_destroy(h);
+    return rc;
+  }
+  *out = h;
+  return 0;
+}
+
+int vbgpu_tree_destroy(vbgpu_tree_t h) {
+  if (!h) return 0;
+  h->order.release();
+  DeviceGuard g(h->device);
+  if (h->stream) cudaStreamSynchronize(h->stream);
+  for (DevBuf *b : {&h->d_info, &h->d_ts, &h->d_acc, &h->d_hkeys, &h->d_hvals, &h->d_keys_by_id, &h->d_ctr, &h->d_seg,
+                    &h->d_seg_phone, &h->d_ids, &h->d_work, &h->d_feats, &h->d_tids, &h->d_stage})
+    b->release();
+  h->layout.release();
+  if (h->stream) cudaStreamDestroy(h->stream);
+  delete h;
+  return 0;
+}
+
+int vbgpu_tree_zero(vbgpu_tree_t h) {
+  VB_CHECK(h, "null handle");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  return tree_zero(h, h->stream);
+}
+
+static int check_tree_args(vbgpu_tree_t h, const float *feats, int32_t stride, const int32_t *tids,
+                           const int64_t *frame_offsets, int32_t n_utts) {
+  VB_CHECK(h && n_utts >= 0, "bad argument");
+  VB_CHECK(stride >= h->D, "stride %d < dim %d", stride, h->D);
+  VB_CHECK(n_utts == 0 || frame_offsets, "null frame_offsets");
+  if (n_utts == 0) return 0;
+  VB_CHECK(frame_offsets[0] == 0, "frame_offsets[0] = %lld, not 0", (long long)frame_offsets[0]);
+  for (int32_t u = 0; u < n_utts; u++)
+    VB_CHECK(frame_offsets[u + 1] >= frame_offsets[u], "frame_offsets not monotone at utterance %d", u);
+  VB_CHECK(frame_offsets[n_utts] == 0 || (feats && tids), "null buffer");
+  return 0;
+}
+
+int vbgpu_tree_accumulate_dev(vbgpu_tree_t h, const float *d_feats, int32_t stride, const int32_t *d_tids,
+                              const int64_t *frame_offsets, int32_t n_utts, void *stream) {
+  VB_TRY(check_tree_args(h, d_feats, stride, d_tids, frame_offsets, n_utts));
+  if (n_utts == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  VB_TRY(h->order.enter(s));
+  VB_TRY(h->layout.update(nullptr, frame_offsets, n_utts, nullptr, nullptr, s));
+  VB_TRY(tree_launch(h, d_feats, stride, d_tids, h->layout.d_frame_offsets.as<int64_t>(), n_utts, h->layout.total_frames,
+                     s));
+  return h->order.leave(s);
+}
+
+int vbgpu_tree_accumulate(vbgpu_tree_t h, const float *feats, int32_t stride, const int32_t *tids,
+                          const int64_t *frame_offsets, int32_t n_utts) {
+  VB_TRY(check_tree_args(h, feats, stride, tids, frame_offsets, n_utts));
+  if (n_utts == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->stream;
+  VB_TRY(h->order.enter(s));
+  const int64_t T = frame_offsets[n_utts];
+  VB_TRY(h->d_feats.reserve((size_t)std::max<int64_t>(T, 1) * stride * 4));
+  VB_TRY(h->d_tids.reserve((size_t)std::max<int64_t>(T, 1) * 4));
+  VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
+  VB_TRY(h2d(h->d_tids.p, tids, (size_t)T * 4, s));
+  int64_t before = 0, after = 0;
+  VB_CUDA(cudaStreamSynchronize(s));
+  VB_TRY(tree_counters(h, nullptr, &before, nullptr, false));
+  VB_TRY(h->layout.update(nullptr, frame_offsets, n_utts, nullptr, nullptr, s));
+  VB_TRY(tree_launch(h, h->d_feats.as<float>(), stride, h->d_tids.as<int32_t>(), h->layout.d_frame_offsets.as<int64_t>(),
+                     n_utts, T, s));
+  VB_CUDA(cudaStreamSynchronize(s));
+  VB_TRY(tree_counters(h, nullptr, &after, nullptr, false));
+  VB_TRY(h->order.leave(s));
+  if (after != before)
+    return fail(VBGPU_ERR_NUMERIC, "%lld frames found no room in the key table (max_keys %d)", (long long)(after - before),
+                h->max_keys);
+  return 0;
+}
+
+int vbgpu_tree_bad_count(vbgpu_tree_t h, int64_t *bad_utterances, int64_t *dropped_frames) {
+  VB_CHECK(h, "null handle");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  return tree_counters(h, bad_utterances, dropped_frames, nullptr, true);
+}
+
+int vbgpu_tree_num_keys(vbgpu_tree_t h, int32_t *num_keys) {
+  VB_CHECK(h && num_keys, "null argument");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  int64_t k = 0;
+  VB_TRY(tree_counters(h, nullptr, nullptr, &k, false));
+  *num_keys = (int32_t)k;
+  return 0;
+}
+
+int vbgpu_tree_download(vbgpu_tree_t h, int32_t *pdf_class, int32_t *phones, double *count, double *sum_x,
+                        double *sum_x2) {
+  VB_CHECK(h, "null handle");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  return tree_download(h, pdf_class, phones, count, sum_x, sum_x2);
+}
+
+int vbgpu_tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t *phones, const double *count,
+                   const double *sum_x, const double *sum_x2) {
+  VB_CHECK(h && n >= 0, "bad argument");
+  VB_CHECK(n == 0 || (pdf_class && phones && count && sum_x && sum_x2), "null buffer");
+  DeviceGuard g(h->device);
+  VB_CUDA(cudaDeviceSynchronize());
+  int64_t dropped = 0;
+  VB_TRY(tree_add(h, n, pdf_class, phones, count, sum_x, sum_x2, &dropped));
+  if (dropped)
+    return fail(VBGPU_ERR_NUMERIC, "%lld entries found no room in the key table (max_keys %d)", (long long)dropped,
+                h->max_keys);
+  return 0;
+}
+
+// ================================================================================================================
 // Fused pipelines
 // ================================================================================================================
 int vbgpu_pipeline_create(vbgpu_mfcc_t mfcc, vbgpu_feat_t feat, vbgpu_gmm_t gmm, vbgpu_pipeline_t *out) {

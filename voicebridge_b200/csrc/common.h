@@ -227,6 +227,21 @@ struct vbgpu_lda_s {
   vb::DevBuf d_feats, d_ids, d_w;  // staging of the host entry point
 };
 
+struct vbgpu_tree_s {
+  vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
+  int device = 0;
+  cudaStream_t stream = nullptr;
+  int32_t N = 3, P = 1, D = 0, max_keys = 0, num_tids = 0;
+  uint32_t mask = 0;                 // hash table slots - 1 (a power of two >= 2 max_keys)
+  vb::DevBuf d_info, d_ts;           // per transition-id: packed phone / pdf-class / flags, transition state
+  vb::DevBuf d_acc;                  // [count K | sum_x K*D | sum_x2 K*D], K = max_keys, by dense id
+  vb::DevBuf d_hkeys, d_hvals, d_keys_by_id;  // hash table (open addressing on the 64-bit key) and key of each dense id
+  vb::DevBuf d_ctr;                  // uint64 counters (tree.cu)
+  vb::DevBuf d_seg, d_seg_phone, d_ids, d_work;  // per-frame scratch and the counting-sort workspace
+  vb::DevBuf d_feats, d_tids, d_stage;           // staging of the host entry points
+  vb::BatchLayout layout;
+};
+
 struct vbgpu_pipeline_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_t mfcc = nullptr;
@@ -291,6 +306,16 @@ int bin_sort_launch(const int32_t *d_ids, int64_t T, int32_t P, const int32_t *d
 
 int lda_launch(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_ids, const float *d_w,
                cudaStream_t s);
+
+int tree_check(const vbgpu_tree_opts *o, const vbgpu_tid_tables *t, int32_t dim, int32_t max_keys);
+int tree_init(vbgpu_tree_t h, const vbgpu_tree_opts *o, const vbgpu_tid_tables *t);  // h->D, max_keys, stream set
+int tree_zero(vbgpu_tree_t h, cudaStream_t s);
+int tree_launch(vbgpu_tree_t h, const float *d_feats, int32_t stride, const int32_t *d_tids, const int64_t *d_fo,
+                int32_t n_utts, int64_t T, cudaStream_t s);
+int tree_counters(vbgpu_tree_t h, int64_t *bad_utts, int64_t *dropped, int64_t *num_keys, bool reset);
+int tree_download(vbgpu_tree_t h, int32_t *pdf_class, int32_t *phones, double *count, double *sum_x, double *sum_x2);
+int tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t *phones, const double *count,
+             const double *sum_x, const double *sum_x2, int64_t *dropped);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
                const int32_t *d_ids, const float *d_w, cudaStream_t s);

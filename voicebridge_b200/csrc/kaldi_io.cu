@@ -270,6 +270,7 @@ __global__ void narrow_kernel(const double *__restrict__ v, int32_t R, int32_t C
 struct Topo {
   std::vector<int32_t> phone2idx;
   std::vector<std::vector<std::vector<int32_t>>> entries;  // [entry][state] -> destination states of its transitions
+  std::vector<std::vector<std::pair<int32_t, int32_t>>> pdf_classes;  // [entry][state] -> (forward, self-loop) pdf class
 };
 bool read_int_vector(Reader &r, std::vector<int32_t> *v) {
   if (!r.need(5) || r.p[r.pos] != 4) return r.ok = false;
@@ -291,13 +292,15 @@ bool read_topology(Reader &r, Topo *t) {  // binary branch of HmmTopology::Read
   if (sz == -1) is_hmm = false, sz = r.basic<int32_t>();
   if (!r.ok || sz < 0 || sz > 100000) return r.ok = false;
   t->entries.resize(sz);
+  t->pdf_classes.resize(sz);
   for (int32_t i = 0; i < sz && r.ok; i++) {
     const int32_t ns = r.basic<int32_t>();
     if (!r.ok || ns < 0 || ns > 100000) return r.ok = false;
     t->entries[i].resize(ns);
+    t->pdf_classes[i].resize(ns);
     for (int32_t j = 0; j < ns && r.ok; j++) {
-      r.basic<int32_t>();                 // forward pdf class
-      if (!is_hmm) r.basic<int32_t>();    // self-loop pdf class
+      const int32_t fwd = r.basic<int32_t>();
+      t->pdf_classes[i][j] = {fwd, is_hmm ? fwd : r.basic<int32_t>()};
       const int32_t nt = r.basic<int32_t>();
       if (!r.ok || nt < 0 || nt > 100000) return r.ok = false;
       for (int32_t k = 0; k < nt && r.ok; k++) {
@@ -308,9 +311,10 @@ bool read_topology(Reader &r, Topo *t) {  // binary branch of HmmTopology::Read
   }
   return r.expect("</Topology>");
 }
-// TransitionModel::Read + ComputeDerived: tid2pdf[0] = -1 (transition-ids are 1-based), log_probs as stored.
-bool read_transition_model(Reader &r, std::vector<int32_t> *tid2pdf, std::vector<float> *log_probs) {
-  Topo topo;
+// TransitionModel::Read + ComputeDerived: tid2pdf[0] = -1 (transition-ids are 1-based), log_probs as stored; the topology
+// and the (phone, hmm-state) of every transition state (tuples[ts - 1]) for callers that want them.
+bool read_transition_model(Reader &r, std::vector<int32_t> *tid2pdf, std::vector<float> *log_probs, Topo &topo,
+                           std::vector<std::pair<int32_t, int32_t>> *tuples) {
   if (!r.expect("<TransitionModel>") || !read_topology(r, &topo)) return false;
   const std::string tok = r.token();
   if (!r.ok || (tok != "<Triples>" && tok != "<Tuples>")) return r.ok = false;
@@ -325,6 +329,7 @@ bool read_transition_model(Reader &r, std::vector<int32_t> *tid2pdf, std::vector
     if (e < 0 || e >= (int32_t)topo.entries.size() || state < 0 || state >= (int32_t)topo.entries[e].size())
       return r.ok = false;
     for (int32_t dst : topo.entries[e][state]) tid2pdf->push_back(dst == state ? self : fwd);  // IsSelfLoop
+    tuples->emplace_back(phone, state);
   }
   const std::string end = r.token();
   if (!r.ok || (end != "</Triples>" && end != "</Tuples>")) return r.ok = false;
@@ -377,7 +382,9 @@ bool read_mdl(Reader &r, Mdl *m) {
     const int64_t at = r.pos;
     const std::string t = r.token();
     r.pos = at;
-    if (t == "<TransitionModel>" && !read_transition_model(r, &m->tid2pdf, &m->log_probs)) return false;
+    Topo topo;
+    std::vector<std::pair<int32_t, int32_t>> tuples;
+    if (t == "<TransitionModel>" && !read_transition_model(r, &m->tid2pdf, &m->log_probs, topo, &tuples)) return false;
   }
   if (!r.expect("<DIMENSION>")) return false;
   m->D = r.basic<int32_t>();
@@ -526,6 +533,46 @@ int vbgpu_io_mdl_info(const void *buf, int64_t n, int32_t *dim, int32_t *num_pdf
   if (num_gauss) *num_gauss = m.pdf_offsets.back();
   if (num_tids) *num_tids = m.tid2pdf.empty() ? 0 : (int32_t)m.tid2pdf.size() - 1;
   return 0;
+}
+
+int vbgpu_io_mdl_transitions(const void *buf, int64_t n, int32_t *phone, int32_t *hmm_state, int32_t *pdf_class,
+                             int32_t *trans_state, int32_t *flags) {
+  VB_CHECK(buf && n >= 0, "bad argument");
+  Reader r(buf, n);
+  Topo topo;
+  std::vector<std::pair<int32_t, int32_t>> tuples;
+  std::vector<int32_t> tid2pdf;
+  std::vector<float> log_probs;
+  try {
+    r.skip_binary_marker();
+    if (!read_transition_model(r, &tid2pdf, &log_probs, topo, &tuples))
+      return fail(VBGPU_ERR_INVALID, "not a binary Kaldi model file starting with a TransitionModel");
+  } catch (const std::bad_alloc &) {
+    return fail(VBGPU_ERR_NOMEM, "out of memory while parsing the model");
+  } catch (const std::exception &e) {
+    return fail(VBGPU_ERR_INVALID, "model parse failed: %s", e.what());
+  }
+  // TransitionModel::TransitionIdToPdfClass / IsSelfLoop / IsFinal, and the check SplitToPhones makes on a phone's first
+  // frame (state 0 of its topology entry emitting)
+  int32_t tid = 0;
+  auto put = [](int32_t *a, int32_t i, int32_t v) {
+    if (a) a[i] = v;
+  };
+  put(phone, 0, 0), put(hmm_state, 0, 0), put(pdf_class, 0, 0), put(trans_state, 0, 0), put(flags, 0, 0);
+  for (size_t ts = 0; ts < tuples.size(); ts++) {
+    const int32_t ph = tuples[ts].first, st = tuples[ts].second, e = topo.phone2idx[ph];
+    const auto &entry = topo.entries[e];
+    const auto &pc = topo.pdf_classes[e][st];
+    const int32_t emit0 = topo.pdf_classes[e][0].first != -1 ? VBGPU_TID_STATE0_EMITTING : 0;
+    for (int32_t dst : entry[st]) {
+      tid++;
+      const bool self = dst == st;
+      put(phone, tid, ph), put(hmm_state, tid, st), put(pdf_class, tid, self ? pc.second : pc.first);
+      put(trans_state, tid, (int32_t)ts + 1);
+      put(flags, tid, (self ? VBGPU_TID_SELF_LOOP : 0) | (dst + 1 == (int32_t)entry.size() ? VBGPU_TID_FINAL : 0) | emit0);
+    }
+  }
+  return tid;
 }
 
 int vbgpu_io_mdl_read(const void *buf, int64_t n, int32_t *pdf_offsets, float *gconsts, float *weights, float *means_invvars,

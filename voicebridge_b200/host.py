@@ -9,6 +9,7 @@ Class / method names and argument meaning follow the Kaldi types VoiceBridge lin
   DecodableAmDiagGmmGpu    DecodableAmDiagGmmScaled                  gmm/decodable-am-diag-gmm.h:121-160
   AccumAmDiagGmmGpu        AccumAmDiagGmm                            gmm/mle-am-diag-gmm.h:34-108
   LdaEstimateGpu           LdaEstimate (accumulation)                transform/lda-estimate.h
+  TreeStatsGpu             AccumulateTreeStats (acc-tree-stats)      hmm/tree-accu.cc
   ScoringPipeline          the fused PCM -> loglikes job (compute-mfcc-feats ... gmm-latgen-faster's decodable)
 
 Errors surface as capi.VbgpuError (the reference throws std::runtime_error from KALDI_ERR).
@@ -704,6 +705,85 @@ class LdaEstimateGpu(_Handle):
         """In-place sum all-reduce of the statistics over a raw ncclComm_t (replaces est-lda summing the job files)."""
         c = comm.value if isinstance(comm, C.c_void_p) else comm
         check(capi.lib().vbgpu_lda_allreduce(self.h, c, _stream_ptr(stream)))
+
+
+class TreeStatsGpu(_Handle):
+    """The statistics of acc-tree-stats (AccumulateTreeStats, hmm/tree-accu.cc) on the device: one GaussClusterable
+    (count, sum x, sum x^2 in FP64) per EventType, in a device hash table of at most max_keys keys.  `tables` is the dict
+    of kaldi_io.read_transitions (or synth.make_phone_alignment); EventTypes are tuples of sorted (key, value) pairs,
+    (-1, pdf-class) first, as the reference's std::map holds them."""
+    _destroy = "vbgpu_tree_destroy"
+
+    def __init__(self, tables, dim, max_keys, context_width=3, central_position=1, ci_phones=(), device=0):
+        super().__init__()
+        self.N, self.P, self.D, self.device = int(context_width), int(central_position), int(dim), int(device)
+        self._tables = {k: _np(tables[k], np.int32) for k in ("phone", "hmm_state", "pdf_class", "trans_state", "flags")}
+        self._ci = _np(sorted(ci_phones), np.int32)
+        t = capi.TidTables(len(self._tables["phone"]) - 1, *(self._tables[k].ctypes.data for k in
+                                                              ("phone", "hmm_state", "pdf_class", "trans_state", "flags")))
+        o = capi.TreeOpts(self.N, self.P, self._ci.ctypes.data if len(self._ci) else None, len(self._ci))
+        check(capi.lib().vbgpu_tree_create(C.byref(o), C.byref(t), self.D, int(max_keys), self.device, C.byref(self.h)))
+
+    def ZeroAccumulators(self):
+        check(capi.lib().vbgpu_tree_zero(self.h))
+
+    def AccumulateTreeStats(self, feats, tids, frame_offsets):
+        """Host form over a packed batch: feats [T, >= dim] rows, tids[T], utterance u = rows frame_offsets[u] ... [u+1].
+        Raises VbgpuError (ERR_NUMERIC) after adding everything else when a frame found no room in the key table."""
+        feats = _np(feats, np.float32)
+        tids, fo = _np(tids, np.int32), _np(frame_offsets, np.int64)
+        check(capi.lib().vbgpu_tree_accumulate(self.h, feats.ctypes.data, feats.shape[1], tids.ctypes.data,
+                                               fo.ctypes.data, len(fo) - 1))
+
+    def accumulate_dev(self, d_feats, stride, d_tids, frame_offsets, stream=None):
+        fo = _np(frame_offsets, np.int64)
+        check(capi.lib().vbgpu_tree_accumulate_dev(self.h, _ptr(d_feats), stride, _ptr(d_tids), fo.ctypes.data,
+                                                   len(fo) - 1, _stream_ptr(stream)))
+
+    def bad_count(self):
+        """(bad utterances, frames without room in the key table) since the last query; resets both."""
+        b, d = C.c_int64(0), C.c_int64(0)
+        check(capi.lib().vbgpu_tree_bad_count(self.h, C.byref(b), C.byref(d)))
+        return b.value, d.value
+
+    def NumKeys(self):
+        n = C.c_int32(0)
+        check(capi.lib().vbgpu_tree_num_keys(self.h, C.byref(n)))
+        return n.value
+
+    def download(self):
+        """(pdf_class[K], phones[K, N] with -1 for absent positions, count[K], sum_x[K, D], sum_x2[K, D]) in EventType order."""
+        K = self.NumKeys()
+        pc, ph = np.zeros(K, np.int32), np.zeros((K, self.N), np.int32)
+        cnt, sx, sx2 = np.zeros(K), np.zeros((K, self.D)), np.zeros((K, self.D))
+        check(capi.lib().vbgpu_tree_download(self.h, pc.ctypes.data, ph.ctypes.data, cnt.ctypes.data, sx.ctypes.data,
+                                             sx2.ctypes.data))
+        return pc, ph, cnt, sx, sx2
+
+    def stats(self):
+        """dict EventType -> (count, sum_x[D], sum_x2[D]), inserted in the reference's std::map order."""
+        pc, ph, cnt, sx, sx2 = self.download()
+        out = {}
+        for k in range(len(pc)):
+            ev = ((-1, int(pc[k])),) + tuple((j, int(p)) for j, p in enumerate(ph[k]) if p >= 0)
+            out[ev] = (float(cnt[k]), sx[k], sx2[k])
+        return out
+
+    def Add(self, other_stats):
+        """Adds a dict of the form stats() returns, key by key (sum-tree-stats; merging handles of several GPUs)."""
+        evs = list(other_stats)
+        n = len(evs)
+        pc, ph = np.zeros(n, np.int32), np.full((n, self.N), -1, np.int32)
+        cnt, sx, sx2 = np.zeros(n), np.zeros((n, self.D)), np.zeros((n, self.D))
+        for k, ev in enumerate(evs):
+            for key, val in ev:
+                if key == -1:
+                    pc[k] = val
+                else:
+                    ph[k, key] = val
+            cnt[k], sx[k], sx2[k] = other_stats[ev]
+        check(capi.lib().vbgpu_tree_add(self.h, n, pc.ctypes.data, ph.ctypes.data, cnt.ctypes.data, sx.ctypes.data,
+                                        sx2.ctypes.data))
 
 
 class ScoringPipeline(_Handle):

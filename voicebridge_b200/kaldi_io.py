@@ -102,6 +102,17 @@ def read_mdl(b):
     return out
 
 
+def read_transitions(b):
+    """The per transition-id tables of a model file's TransitionModel: dict of int32 arrays phone, hmm_state, pdf_class,
+    trans_state and flags (capi.TID_*), num_tids + 1 each with entry 0 unused, as vbgpu_tree_create takes them."""
+    a, p, n = _buf(b)
+    nt = check(capi.lib().vbgpu_io_mdl_transitions(p, n, None, None, None, None, None))
+    out = {k: np.zeros(nt + 1, np.int32) for k in ("phone", "hmm_state", "pdf_class", "trans_state", "flags")}
+    check(capi.lib().vbgpu_io_mdl_transitions(p, n, *(out[k].ctypes.data for k in
+                                                      ("phone", "hmm_state", "pdf_class", "trans_state", "flags"))))
+    return out
+
+
 def write_acc(pdf_offsets, occ, mean_acc, var_acc, tot_like, tot_frames, trans_accs=None):
     """The bytes of a gmm-acc-stats-ali output file (x.JOBID.acc) from downloaded statistics."""
     po = np.ascontiguousarray(pdf_offsets, np.int32)

@@ -197,3 +197,79 @@ def make_pitch_wave(n_samples, seed, samp_freq=16000.0):
         gate = np.convolve(gate, np.ones(k) / k, mode="same")
     x = 4000.0 * x * gate + rng.standard_normal(n_samples) * 250.0 + rng.uniform(-100, 100)
     return np.clip(np.round(x), -32768, 32767).astype(np.int16)
+
+
+def phone_topology(n_phones):
+    """A Kaldi-style HMM topology and its per transition-id tables: phone 1 is a 1-state phone, phones 2 ... n_phones are
+    3-state left-to-right phones (pdf classes 0, 1, 2; each emitting state has a self-loop, then a forward transition;
+    the last state is final, non-emitting).  Every (phone, state) has its own pdf, so <Triples> and <Tuples> agree.
+    Returns a dict: the tables of vbgpu_tid_tables (phone, hmm_state, pdf_class, trans_state, flags, [num_tids + 1]),
+    entries (per topology entry: [(forward_pdf_class, self_loop_pdf_class, [destination, ...]), ...]), phone2entry,
+    tuples [(phone, hmm_state, forward_pdf, self_loop_pdf)] and tid {(phone, state, is_self_loop): transition-id}."""
+    one = [(0, 0, [0, 1]), (-1, -1, [])]
+    three = [(0, 0, [0, 1]), (1, 1, [1, 2]), (2, 2, [2, 3]), (-1, -1, [])]
+    entries = [one, three]
+    phone2entry = {p: (0 if p == 1 else 1) for p in range(1, n_phones + 1)}
+    tuples, cols, tid = [], {k: [0] for k in ("phone", "hmm_state", "pdf_class", "trans_state", "flags")}, {}
+    for p in range(1, n_phones + 1):
+        e = entries[phone2entry[p]]
+        for s, (fwd, slf, dsts) in enumerate(e):
+            if fwd < 0:
+                continue
+            tuples.append((p, s, len(tuples), len(tuples)))
+            for d in dsts:
+                is_self = d == s
+                tid[(p, s, is_self)] = len(cols["phone"])
+                cols["phone"].append(p)
+                cols["hmm_state"].append(s)
+                cols["pdf_class"].append(slf if is_self else fwd)
+                cols["trans_state"].append(len(tuples))
+                cols["flags"].append((1 if is_self else 0) | (2 if d + 1 == len(e) else 0) | (4 if e[0][0] >= 0 else 0))
+    out = {k: np.asarray(v, np.int32) for k, v in cols.items()}
+    out.update(entries=entries, phone2entry=phone2entry, tuples=tuples, tid=tid)
+    return out
+
+
+def phone_alignment(topo, phones, durations, reordered=False):
+    """Transition-ids of a phone sequence: durations[i] holds the frames of each emitting state of phones[i] (>= 1 each).
+    Plain: a state's self-loops, then its forward transition; reordered: the forward transition first."""
+    out = []
+    for p, durs in zip(phones, durations):
+        for s, d in enumerate(durs):
+            run = [topo["tid"][(p, s, True)]] * (d - 1)
+            fwd = topo["tid"][(p, s, False)]
+            out += ([fwd] + run) if reordered else (run + [fwd])
+    return np.asarray(out, np.int32)
+
+
+def make_phone_alignment(n_phones, frame_offsets, seed, reordered=False, zipf=1.0, mean_state_frames=3.0):
+    """Alignments that fill every utterance of a packed batch exactly: phones drawn with Zipf-like frequencies
+    (p(rank r) ~ 1 / r^zipf, so that triphone keys repeat as in speech), state durations 1 + Poisson(mean - 1); the
+    last phone of an utterance is shortened to fit, or is the 1-state phone.  Returns (topology, tids[T], phone
+    sequence per utterance)."""
+    rng = np.random.default_rng(seed)
+    topo = phone_topology(n_phones)
+    freq = 1.0 / np.arange(1, n_phones + 1) ** zipf
+    freq /= freq.sum()
+    rank2phone = rng.permutation(np.arange(1, n_phones + 1))
+    fo = np.asarray(frame_offsets, np.int64)
+    tids, seqs = [], []
+    for u in range(len(fo) - 1):
+        rem = int(fo[u + 1] - fo[u])
+        phones, durs = [], []
+        while rem > 0:
+            p = int(rank2phone[rng.choice(n_phones, p=freq)])
+            ns = len(topo["entries"][topo["phone2entry"][p]]) - 1
+            d = list(1 + rng.poisson(mean_state_frames - 1.0, ns))
+            if sum(d) > rem:
+                if rem >= ns:
+                    d = [1] * ns
+                    d[-1] += rem - ns
+                else:
+                    p, d = 1, [rem]
+            phones.append(p)
+            durs.append(d)
+            rem -= sum(d)
+        seqs.append(phones)
+        tids.append(phone_alignment(topo, phones, durs, reordered))
+    return topo, (np.concatenate(tids) if tids else np.zeros(0, np.int32)).astype(np.int32), seqs
