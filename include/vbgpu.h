@@ -252,6 +252,10 @@ int vbgpu_debug_tc_layout(int32_t num_pdfs, int32_t dim, const int32_t *pdf_offs
                           const float *means_invvars, const float *inv_vars, int32_t stride, int32_t pair, int32_t *info,
                           uint8_t *image, int64_t image_cap, int32_t *hdr, int32_t hdr_cap, int32_t *grp, int32_t grp_cap,
                           int32_t *col_of_pdf, int32_t *merge, int32_t merge_cap, float *centre, float *s1, float *s2, int32_t *bounds);
+/* Bytes of device memory and of pinned host memory the library holds right now, over all handles and devices of the
+ * process (scratch included).  Creating and destroying a handle leaves both where they were; tests use this to check
+ * that nothing leaks.  Needs no GPU. */
+int vbgpu_debug_live_bytes(int64_t *device_bytes, int64_t *pinned_bytes);
 /* SPARSE CONSUMERS (SURVEY.md §8f n3).  The dense matrix is 4 P bytes per frame; its consumers read far less, and shipping
  * only that is what takes the host path off the PCIe line.  Both forms score on the device in slabs of frames (bounded
  * footprint) and extract what was asked for; *_dev forms take device feature / output pointers (descriptors on the host).

@@ -62,6 +62,11 @@ def test_version_and_argument_errors_need_no_gpu():
     assert lib.vbgpu_pitch_create(C.byref(po_), 0, C.byref(h)) == capi.ERR_INVALID
     po_ = capi.default_pitch_opts(min_f0=400.0, max_f0=50.0)
     assert lib.vbgpu_pitch_create(C.byref(po_), 0, C.byref(h)) == capi.ERR_INVALID
+    # destroying a NULL handle is a no-op that succeeds
+    destroys = [n for n in capi.EXPORTS if n.endswith("_destroy") and capi._SIGS[n][0] is C.c_int]
+    assert len(destroys) >= 8
+    for n in destroys:
+        assert getattr(lib, n)(None) == 0, n
 
 
 def test_no_cpu_fallback():
@@ -77,6 +82,8 @@ def test_no_cpu_fallback():
     assert b"no CPU fallback" in lib.vbgpu_last_error()
     po_ = capi.default_pitch_opts()
     assert lib.vbgpu_pitch_create(C.byref(po_), 0, C.byref(h)) == capi.ERR_CUDA
+    assert b"no CPU fallback" in lib.vbgpu_last_error()
+    assert lib.vbgpu_downsample_create(16000.0, 8000.0, 0, C.byref(h)) == capi.ERR_CUDA
     assert b"no CPU fallback" in lib.vbgpu_last_error()
     from voicebridge_b200 import host
     with pytest.raises(capi.VbgpuError):

@@ -142,6 +142,7 @@ _SIGS = {
     "vbgpu_gmm_score_cols_dev": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _vp]),
     "vbgpu_debug_tc_layout": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _i64, _vp, _i32, _vp, _i32,
                                         _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "vbgpu_debug_live_bytes": (C.c_int, [C.POINTER(_i64), C.POINTER(_i64)]),
     "vbgpu_gmm_score_subset": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "vbgpu_gmm_score_subset_dev": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "vbgpu_gmm_score_gather": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _i64, _vp]),

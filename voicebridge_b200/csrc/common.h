@@ -2,10 +2,12 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <atomic>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -34,51 +36,133 @@ int fail(int code, const char *fmt, ...);
     if (rc_ < 0) return rc_; \
   } while (0)
 
-// ---- grow-only device / pinned buffers ---------------------------------------------------------------------
+// Fails with VBGPU_ERR_CUDA ("no CPU fallback") without a CUDA device, VBGPU_ERR_INVALID for a device out of range.
+int check_device(int device);
+
+// ---- owning handles of device memory, pinned memory, streams and events -----------------------------------------
+// Bytes of device and pinned memory the library holds right now (vbgpu_debug_live_bytes): every cudaMalloc and
+// cudaMallocHost goes through DevBuf / PinBuf.
+inline std::atomic<int64_t> live_device_bytes{0}, live_pinned_bytes{0};
+
+// Grow-only buffers, freed by their destructor.  A DevBuf is freed on the device that is current when its owner is
+// destroyed, so a function declares its DeviceGuard before any local DevBuf, and a handle is deleted while a
+// DeviceGuard for its device is alive.
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  ~DevBuf() { release(); }
   int reserve(size_t bytes) {
     if (bytes <= cap) return 0;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
+    release();
     size_t want = bytes + bytes / 8 + 256;
     cudaError_t e = cudaMalloc(&p, want);
-    if (e != cudaSuccess) return fail(VBGPU_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+    if (e != cudaSuccess) {
+      p = nullptr;
+      cudaGetLastError();  // reported here: the next launch check must not see this error again
+      return fail(VBGPU_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+    }
     cap = want;
+    live_device_bytes += (int64_t)want;
     return 0;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
+  // reserve(bytes), then a synchronous copy of bytes from the host
+  int upload(const void *src, size_t bytes) {
+    int rc = reserve(bytes);
+    if (rc < 0 || bytes == 0) return rc;
+    cudaError_t e = cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) return fail(VBGPU_ERR_CUDA, "upload of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+    return 0;
   }
   template <typename T>
   T *as() const { return static_cast<T *>(p); }
+
+ private:
+  void release() {
+    if (p) {
+      cudaFree(p);
+      live_device_bytes -= (int64_t)cap;
+    }
+    p = nullptr;
+    cap = 0;
+  }
 };
 
 struct PinBuf {
   void *p = nullptr;
   size_t cap = 0;
+  PinBuf() = default;
+  PinBuf(const PinBuf &) = delete;
+  PinBuf &operator=(const PinBuf &) = delete;
+  ~PinBuf() { release(); }
   int reserve(size_t bytes) {
     if (bytes <= cap) return 0;
-    if (p) cudaFreeHost(p);
-    p = nullptr;
-    cap = 0;
+    release();
     size_t want = bytes + bytes / 8 + 256;
     cudaError_t e = cudaMallocHost(&p, want);
-    if (e != cudaSuccess) return fail(VBGPU_ERR_NOMEM, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
+    if (e != cudaSuccess) {
+      p = nullptr;
+      cudaGetLastError();
+      return fail(VBGPU_ERR_NOMEM, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
+    }
     cap = want;
+    live_pinned_bytes += (int64_t)want;
     return 0;
-  }
-  void release() {
-    if (p) cudaFreeHost(p);
-    p = nullptr;
-    cap = 0;
   }
   template <typename T>
   T *as() const { return static_cast<T *>(p); }
+
+ private:
+  void release() {
+    if (p) {
+      cudaFreeHost(p);
+      live_pinned_bytes -= (int64_t)cap;
+    }
+    p = nullptr;
+    cap = 0;
+  }
+};
+
+// A non-blocking stream, destroyed with its owner.  Converts to the raw handle (null until create()).
+struct Stream {
+  cudaStream_t s = nullptr;
+  Stream() = default;
+  Stream(const Stream &) = delete;
+  Stream &operator=(const Stream &) = delete;
+  ~Stream() {
+    if (s) cudaStreamDestroy(s);
+  }
+  int create() {
+    cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+    if (e != cudaSuccess) {
+      s = nullptr;
+      return fail(VBGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+    }
+    return 0;
+  }
+  operator cudaStream_t() const { return s; }
+};
+
+// An event without timing, destroyed with its owner.  Converts to the raw handle (null until create()).
+struct Event {
+  cudaEvent_t ev = nullptr;
+  Event() = default;
+  Event(const Event &) = delete;
+  Event &operator=(const Event &) = delete;
+  ~Event() {
+    if (ev) cudaEventDestroy(ev);
+  }
+  int create() {
+    cudaError_t e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e != cudaSuccess) {
+      ev = nullptr;
+      return fail(VBGPU_ERR_CUDA, "cudaEventCreate failed: %s", cudaGetErrorString(e));
+    }
+    return 0;
+  }
+  operator cudaEvent_t() const { return ev; }
 };
 
 struct DeviceGuard {
@@ -100,7 +184,7 @@ int num_sms(int device);
 // the scratch.  enter() makes the new stream wait on the event leave() recorded at the end of the previous call.
 struct StreamOrder {
   cudaStream_t last = nullptr;
-  cudaEvent_t ev = nullptr;
+  Event ev;
   bool used = false;
   int enter(cudaStream_t s) {
     if (used && last != s) {
@@ -110,20 +194,12 @@ struct StreamOrder {
     return 0;
   }
   int leave(cudaStream_t s) {
-    if (!ev) {
-      cudaError_t e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-      if (e != cudaSuccess) return fail(VBGPU_ERR_CUDA, "cudaEventCreate failed: %s", cudaGetErrorString(e));
-    }
+    if (!ev) VB_TRY(ev.create());
     cudaError_t e = cudaEventRecord(ev, s);
     if (e != cudaSuccess) return fail(VBGPU_ERR_CUDA, "cudaEventRecord failed: %s", cudaGetErrorString(e));
     last = s;
     used = true;
     return 0;
-  }
-  void release() {
-    if (ev) cudaEventDestroy(ev);
-    ev = nullptr;
-    used = false;
   }
 };
 
@@ -139,7 +215,6 @@ struct BatchLayout {
   // Upload (if changed) sample offsets + frame offsets and rebuild frame2utt.  utt2spk / utt_aux may be null.
   int update(const int64_t *sample_offsets, const int64_t *frame_offsets, int32_t n, const int32_t *utt2spk,
              const int32_t *utt_aux, cudaStream_t s);
-  void release();
 };
 
 void launch_fill_frame2utt(const int64_t *d_frame_offsets, int32_t n_utts, int64_t total_frames, int32_t *d_frame2utt,
@@ -156,7 +231,7 @@ struct vbgpu_mfcc_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_opts opts;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t L = 0, shift = 0, npad = 0, mel_pitch = 0;
   int32_t fbank = 0, use_log_fbank = 1, use_power = 1;  // fbank != 0: the handle is a FbankComputer (vbgpu_fbank_create)
   int32_t plp = 0, lpc_order = 12;                      // plp != 0: the handle is a PlpComputer (vbgpu_plp_create)
@@ -175,7 +250,7 @@ struct vbgpu_feat_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_feat_opts opts;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t in_dim = 0, mid_dim = 0, out_dim = 0, halo = 0;
   int32_t t_rows = 0, t_cols = 0;  // global transform (lda mode)
   std::vector<float> h_delta_scales;
@@ -187,7 +262,7 @@ struct vbgpu_feat_s {
 struct vbgpu_gmm_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t P = 0, N = 0, D = 0, DP = 0;  // DP: padded row length of the SIMT layout (multiple of 4)
   int32_t kernel = 0;
   int32_t max_pdf_size = 0;
@@ -196,8 +271,8 @@ struct vbgpu_gmm_s {
   vb::DevBuf d_bad;                             // int64 counter of NaN/Inf outputs
   vb::DevBuf d_feats, d_ll;
   vb::DevBuf d_sp_slab, d_sp_i64, d_sp_i32, d_sp_f2u, d_sp_out;  // sparse consumers (score_sparse.cu): slab + descriptors
-  cudaStream_t copy_stream = nullptr;        // host-facing subset calls: results of slab k leave while slab k+1 is scored
-  cudaEvent_t sp_done[2] = {nullptr, nullptr};
+  vb::Stream copy_stream;  // host-facing subset calls: results of slab k leave while slab k+1 is scored
+  vb::Event sp_done[2];
   void *tc = nullptr;  // tensor-core scoring state (score_tc.cu)
   std::string tc_note;  // why the model is NOT on the tensor-core plan ("" when it is)
 };
@@ -206,7 +281,7 @@ struct vbgpu_acc_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_gmm_t model = nullptr;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int64_t n_doubles = 0;
   int32_t n_trans = 0;  // transition accumulators behind tot_frames (num_tids + 1 entries, 0 = none)
   vb::DevBuf d_acc;  // [occ N | mean N*D | var N*D | tot_like | tot_frames | transition accs]
@@ -218,7 +293,7 @@ struct vbgpu_acc_s {
 struct vbgpu_lda_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t C = 0, D = 0;
   int64_t n_doubles = 0;  // C + C*D + D(D+1)/2
   vb::DevBuf d_acc;       // [zero C | first C*D | second D(D+1)/2, SpMatrix packing]
@@ -230,7 +305,7 @@ struct vbgpu_lda_s {
 struct vbgpu_tree_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t N = 3, P = 1, D = 0, max_keys = 0, num_tids = 0;
   uint32_t mask = 0;                 // hash table slots - 1 (a power of two >= 2 max_keys)
   vb::DevBuf d_info, d_ts;           // per transition-id: packed phone / pdf-class / flags, transition state
@@ -248,10 +323,10 @@ struct vbgpu_pipeline_s {
   vbgpu_feat_t feat = nullptr;
   vbgpu_gmm_t gmm = nullptr;
   int device = 0;
-  cudaStream_t stream = nullptr, copy_stream = nullptr;
+  vb::Stream stream, copy_stream;
   vb::DevBuf d_mfcc, d_feats, d_pcm, d_ll[2], d_fmllr, d_stats;
   vb::PinBuf pin_pcm, pin_ll[2], pin_feats;
-  cudaEvent_t ev_ll[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
+  vb::Event ev_ll[2], ev_copied[2];
 };
 
 // ---- kernel launchers (defined in the .cu files) ----------------------------------------------------------------

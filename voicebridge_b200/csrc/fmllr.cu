@@ -29,7 +29,7 @@ struct vbgpu_fmllr_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch
   vbgpu_gmm_t model = nullptr;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
   int32_t n_spk = 0, D = 0, np = 0;
   int64_t per_spk = 0;  // doubles per speaker: beta | K[D][D+1] | G[D][np]
   vb::DevBuf d_stats, d_ab, d_cnt, d_units, d_pairs, d_like, d_work;
@@ -471,7 +471,7 @@ int vbgpu_fmllr_create(vbgpu_gmm_t model, int32_t n_spk, vbgpu_fmllr_t *out) {
   *out = nullptr;
   VB_CHECK(model->D <= kMaxD, "fMLLR statistics serve feature dims up to %d (got %d)", kMaxD, model->D);
   DeviceGuard g(model->device);
-  vbgpu_fmllr_s *h = new vbgpu_fmllr_s;
+  std::unique_ptr<vbgpu_fmllr_s, decltype(&vbgpu_fmllr_destroy)> h(new vbgpu_fmllr_s, vbgpu_fmllr_destroy);
   h->model = model;
   h->device = model->device;
   h->n_spk = n_spk;
@@ -481,33 +481,21 @@ int vbgpu_fmllr_create(vbgpu_gmm_t model, int32_t n_spk, vbgpu_fmllr_t *out) {
   std::vector<uint8_t> pairs((size_t)2 * h->np);
   for (int j = 0; j <= h->D; j++)  // SpMatrix packing: (j, k), k <= j, at j(j+1)/2 + k
     for (int k = 0; k <= j; k++) pairs[2 * (j * (j + 1) / 2 + k)] = (uint8_t)j, pairs[2 * (j * (j + 1) / 2 + k) + 1] = (uint8_t)k;
-  int rc = 0;
-  cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-  if (e != cudaSuccess) rc = fail(VBGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+  VB_TRY(h->stream.create());
   const size_t bytes = (size_t)n_spk * h->per_spk * 8;
-  if (rc == 0) rc = h->d_stats.reserve(bytes);
-  if (rc == 0) rc = h->d_pairs.reserve(pairs.size());
-  if (rc == 0) rc = h->d_like.reserve(8);
-  if (rc == 0 && (cudaMemset(h->d_stats.p, 0, bytes) != cudaSuccess || cudaMemset(h->d_like.p, 0, 8) != cudaSuccess ||
-                  cudaMemcpy(h->d_pairs.p, pairs.data(), pairs.size(), cudaMemcpyHostToDevice) != cudaSuccess))
-    rc = fail(VBGPU_ERR_CUDA, "initialising the fMLLR statistics failed");
-  if (rc < 0) {
-    vbgpu_fmllr_destroy(h);
-    return rc;
-  }
-  *out = h;
+  VB_TRY(h->d_stats.reserve(bytes));
+  VB_TRY(h->d_pairs.upload(pairs.data(), pairs.size()));
+  VB_TRY(h->d_like.reserve(8));
+  VB_CUDA(cudaMemset(h->d_stats.p, 0, bytes));
+  VB_CUDA(cudaMemset(h->d_like.p, 0, 8));
+  *out = h.release();
   return 0;
 }
 
 int vbgpu_fmllr_destroy(vbgpu_fmllr_t h) {
   if (!h) return 0;
-  h->order.release();
   DeviceGuard g(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
-  for (vb::DevBuf *b : {&h->d_stats, &h->d_ab, &h->d_cnt, &h->d_units, &h->d_pairs, &h->d_like, &h->d_work, &h->d_feats, &h->d_ids,
-                        &h->d_w})
-    b->release();
-  if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
   return 0;
 }
@@ -587,92 +575,85 @@ int vbgpu_mllt_accumulate(vbgpu_gmm_t model, const float *feats, int64_t T, int3
   VB_CHECK(stride >= model->D, "stride %d < D %d", stride, model->D);
   if (T == 0) return 0;
   VB_CHECK(feats && pdf_ids, "null buffer");
-  vbgpu_fmllr_t h = nullptr;
-  VB_TRY(vbgpu_fmllr_create(model, 1, &h));  // one "speaker": beta | (unused K) | G of the pseudo-frames
-  DeviceGuard guard(h->device);
+  DeviceGuard guard(model->device);
+  vbgpu_fmllr_t raw = nullptr;
+  VB_TRY(vbgpu_fmllr_create(model, 1, &raw));  // one "speaker": beta | (unused K) | G of the pseudo-frames
+  std::unique_ptr<vbgpu_fmllr_s, decltype(&vbgpu_fmllr_destroy)> h(raw, vbgpu_fmllr_destroy);
   cudaStream_t s = h->stream;
   const int D = model->D, P = model->P, sms = vb::num_sms(h->device);
   const std::vector<int32_t> &po = model->h_pdf_offsets;
-  int rc = 0;
   vb::DevBuf d_xi, d_off;
   std::vector<int32_t> off;
-  auto run = [&]() -> int {
-    VB_CUDA(cudaMemsetAsync(model->d_bad.p, 0, 8, s));
-    const int64_t kMaxFrames = 262144, kMaxRows = 1500000;
-    for (int64_t t0 = 0; t0 < T;) {
-      // a slab of frames whose (frame, Gaussian) rows fit the row buffers
-      off.assign(1, 0);
-      int64_t t1 = t0;
-      while (t1 < T && t1 - t0 < kMaxFrames) {
-        const int32_t p = pdf_ids[t1];
-        const int32_t M = (p >= 0 && p < P) ? po[p + 1] - po[p] : 0;
-        if (off.back() + M > kMaxRows && t1 > t0) break;
-        off.push_back(off.back() + M);
-        t1++;
-      }
-      const int64_t n = t1 - t0, R = off.back();
-      VB_TRY(h->d_feats.reserve((size_t)n * stride * 4));
-      VB_TRY(h->d_ids.reserve((size_t)n * 4));
-      VB_TRY(d_off.reserve((size_t)(n + 1) * 4));
-      VB_CUDA(cudaMemcpyAsync(h->d_feats.p, feats + t0 * stride, (size_t)n * stride * 4, cudaMemcpyHostToDevice, s));
-      VB_CUDA(cudaMemcpyAsync(h->d_ids.p, pdf_ids + t0, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-      VB_CUDA(cudaMemcpyAsync(d_off.p, off.data(), (size_t)(n + 1) * 4, cudaMemcpyHostToDevice, s));
-      const float *d_w = nullptr;
-      if (weights) {
-        VB_TRY(h->d_w.reserve((size_t)n * 4));
-        VB_CUDA(cudaMemcpyAsync(h->d_w.p, weights + t0, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-        d_w = h->d_w.as<float>();
-      }
-      if (R > 0) {
-        VB_TRY(d_xi.reserve((size_t)R * kMaxD * 4));
-        VB_TRY(h->d_ab.reserve((size_t)R * 2 * kMaxD * 4));
-        VB_TRY(h->d_cnt.reserve((size_t)R * 4));
-        VB_CUDA(cudaMemsetAsync(d_xi.p, 0, (size_t)R * kMaxD * 4, s));
-        VB_CUDA(cudaMemsetAsync(h->d_ab.p, 0, (size_t)R * 2 * kMaxD * 4, s));
-        VB_CUDA(cudaMemsetAsync(h->d_cnt.p, 0, (size_t)R * 4, s));
-      }
-      const int grid = (int)std::min<int64_t>((n + kWarps - 1) / kWarps, (int64_t)sms * 8);
-      mllt_rows_kernel<true><<<grid, kWarps * 32, 0, s>>>(
-          h->d_feats.as<float>(), n, stride, D, model->DP, h->d_ids.as<int32_t>(), d_w, model->d_rows.as<float>(),
-          model->d_gconsts.as<float>(), model->d_pdf_offsets.as<int32_t>(), P, d_off.as<int32_t>(), d_xi.as<float>(),
-          h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(), model->d_bad.as<unsigned long long>(), nullptr);
-      VB_CUDA(cudaGetLastError());
-      if (R > 0) {
-        std::vector<int32_t> &u = h->h_units;
-        u.clear();
-        for (int64_t r0 = 0; r0 < R; r0 += kFChunk) {
-          u.push_back(0);
-          u.push_back((int32_t)r0);
-          u.push_back((int32_t)std::min<int64_t>(kFChunk, R - r0));
-        }
-        VB_TRY(h->d_units.reserve(u.size() * 4));
-        VB_CUDA(cudaMemcpyAsync(h->d_units.p, u.data(), u.size() * 4, cudaMemcpyHostToDevice, s));
-        VB_TRY(launch_gk(h, d_xi.as<float>(), kMaxD, (int)(u.size() / 3), s));
-      }
-      VB_CUDA(cudaStreamSynchronize(s));  // the host staging vectors are rebuilt for the next slab
-      t0 = t1;
+  VB_CUDA(cudaMemsetAsync(model->d_bad.p, 0, 8, s));
+  const int64_t kMaxFrames = 262144, kMaxRows = 1500000;
+  for (int64_t t0 = 0; t0 < T;) {
+    // a slab of frames whose (frame, Gaussian) rows fit the row buffers
+    off.assign(1, 0);
+    int64_t t1 = t0;
+    while (t1 < T && t1 - t0 < kMaxFrames) {
+      const int32_t p = pdf_ids[t1];
+      const int32_t M = (p >= 0 && p < P) ? po[p + 1] - po[p] : 0;
+      if (off.back() + M > kMaxRows && t1 > t0) break;
+      off.push_back(off.back() + M);
+      t1++;
     }
-    // beta | K (ignored) | G[i] packed over (D+1): its first D(D+1)/2 entries are the D x D block MlltAccs keeps
-    const int np1 = (D + 1) * (D + 2) / 2, np = D * (D + 1) / 2;
-    std::vector<double> st((size_t)h->per_spk);
-    double like = 0.0;
-    unsigned long long bad = 0;
-    VB_CUDA(cudaMemcpy(st.data(), h->d_stats.p, st.size() * 8, cudaMemcpyDeviceToHost));
-    VB_CUDA(cudaMemcpy(&like, h->d_like.p, 8, cudaMemcpyDeviceToHost));
-    VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
-    *beta += st[0];
-    const double *g = st.data() + 1 + (size_t)D * (D + 1);
-    for (int i = 0; i < D; i++)
-      for (int k = 0; k < np; k++) G[(size_t)i * np + k] += g[(size_t)i * np1 + k];
-    if (tot_like) *tot_like += like;
-    if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
-    return 0;
-  };
-  rc = run();
-  d_xi.release();
-  d_off.release();
-  vbgpu_fmllr_destroy(h);
-  return rc;
+    const int64_t n = t1 - t0, R = off.back();
+    VB_TRY(h->d_feats.reserve((size_t)n * stride * 4));
+    VB_TRY(h->d_ids.reserve((size_t)n * 4));
+    VB_TRY(d_off.reserve((size_t)(n + 1) * 4));
+    VB_CUDA(cudaMemcpyAsync(h->d_feats.p, feats + t0 * stride, (size_t)n * stride * 4, cudaMemcpyHostToDevice, s));
+    VB_CUDA(cudaMemcpyAsync(h->d_ids.p, pdf_ids + t0, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    VB_CUDA(cudaMemcpyAsync(d_off.p, off.data(), (size_t)(n + 1) * 4, cudaMemcpyHostToDevice, s));
+    const float *d_w = nullptr;
+    if (weights) {
+      VB_TRY(h->d_w.reserve((size_t)n * 4));
+      VB_CUDA(cudaMemcpyAsync(h->d_w.p, weights + t0, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+      d_w = h->d_w.as<float>();
+    }
+    if (R > 0) {
+      VB_TRY(d_xi.reserve((size_t)R * kMaxD * 4));
+      VB_TRY(h->d_ab.reserve((size_t)R * 2 * kMaxD * 4));
+      VB_TRY(h->d_cnt.reserve((size_t)R * 4));
+      VB_CUDA(cudaMemsetAsync(d_xi.p, 0, (size_t)R * kMaxD * 4, s));
+      VB_CUDA(cudaMemsetAsync(h->d_ab.p, 0, (size_t)R * 2 * kMaxD * 4, s));
+      VB_CUDA(cudaMemsetAsync(h->d_cnt.p, 0, (size_t)R * 4, s));
+    }
+    const int grid = (int)std::min<int64_t>((n + kWarps - 1) / kWarps, (int64_t)sms * 8);
+    mllt_rows_kernel<true><<<grid, kWarps * 32, 0, s>>>(
+        h->d_feats.as<float>(), n, stride, D, model->DP, h->d_ids.as<int32_t>(), d_w, model->d_rows.as<float>(),
+        model->d_gconsts.as<float>(), model->d_pdf_offsets.as<int32_t>(), P, d_off.as<int32_t>(), d_xi.as<float>(),
+        h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(), model->d_bad.as<unsigned long long>(), nullptr);
+    VB_CUDA(cudaGetLastError());
+    if (R > 0) {
+      std::vector<int32_t> &u = h->h_units;
+      u.clear();
+      for (int64_t r0 = 0; r0 < R; r0 += kFChunk) {
+        u.push_back(0);
+        u.push_back((int32_t)r0);
+        u.push_back((int32_t)std::min<int64_t>(kFChunk, R - r0));
+      }
+      VB_TRY(h->d_units.reserve(u.size() * 4));
+      VB_CUDA(cudaMemcpyAsync(h->d_units.p, u.data(), u.size() * 4, cudaMemcpyHostToDevice, s));
+      VB_TRY(launch_gk(h.get(), d_xi.as<float>(), kMaxD, (int)(u.size() / 3), s));
+    }
+    VB_CUDA(cudaStreamSynchronize(s));  // the host staging vectors are rebuilt for the next slab
+    t0 = t1;
+  }
+  // beta | K (ignored) | G[i] packed over (D+1): its first D(D+1)/2 entries are the D x D block MlltAccs keeps
+  const int np1 = (D + 1) * (D + 2) / 2, np = D * (D + 1) / 2;
+  std::vector<double> st((size_t)h->per_spk);
+  double like = 0.0;
+  unsigned long long bad = 0;
+  VB_CUDA(cudaMemcpy(st.data(), h->d_stats.p, st.size() * 8, cudaMemcpyDeviceToHost));
+  VB_CUDA(cudaMemcpy(&like, h->d_like.p, 8, cudaMemcpyDeviceToHost));
+  VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
+  *beta += st[0];
+  const double *g = st.data() + 1 + (size_t)D * (D + 1);
+  for (int i = 0; i < D; i++)
+    for (int k = 0; k < np; k++) G[(size_t)i * np + k] += g[(size_t)i * np1 + k];
+  if (tot_like) *tot_like += like;
+  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  return 0;
 }
 
 int vbgpu_gmm_component_posteriors(vbgpu_gmm_t model, const float *feats, int64_t T, int32_t stride, const int32_t *pdf_ids,
@@ -695,43 +676,37 @@ int vbgpu_gmm_component_posteriors(vbgpu_gmm_t model, const float *feats, int64_
   }
   const int64_t R = off.back();
   vb::DevBuf d_f, d_i, d_w, d_o, d_p, d_l, d_like;
-  int rc = 0;
-  auto run = [&]() -> int {
-    VB_TRY(d_f.reserve((size_t)T * stride * 4));
-    VB_TRY(d_i.reserve((size_t)T * 4));
-    VB_TRY(d_o.reserve((size_t)(T + 1) * 4));
-    VB_TRY(d_p.reserve((size_t)std::max<int64_t>(R, 1) * 4));
-    VB_TRY(d_l.reserve((size_t)T * 4));
-    VB_TRY(d_like.reserve(8));
-    VB_CUDA(cudaMemcpy(d_f.p, feats, (size_t)T * stride * 4, cudaMemcpyHostToDevice));
-    VB_CUDA(cudaMemcpy(d_i.p, pdf_ids, (size_t)T * 4, cudaMemcpyHostToDevice));
-    VB_CUDA(cudaMemcpy(d_o.p, off.data(), (size_t)(T + 1) * 4, cudaMemcpyHostToDevice));
-    VB_CUDA(cudaMemset(d_p.p, 0, (size_t)std::max<int64_t>(R, 1) * 4));
-    VB_CUDA(cudaMemset(d_like.p, 0, 8));
-    VB_CUDA(cudaMemset(model->d_bad.p, 0, 8));
-    const float *dw = nullptr;
-    if (weights) {
-      VB_TRY(d_w.reserve((size_t)T * 4));
-      VB_CUDA(cudaMemcpy(d_w.p, weights, (size_t)T * 4, cudaMemcpyHostToDevice));
-      dw = d_w.as<float>();
-    }
-    const int grid = (int)std::min<int64_t>((T + kWarps - 1) / kWarps, (int64_t)sms * 8);
-    mllt_rows_kernel<false><<<grid, kWarps * 32>>>(d_f.as<float>(), T, stride, model->D, model->DP, d_i.as<int32_t>(), dw,
-                                                   model->d_rows.as<float>(), model->d_gconsts.as<float>(),
-                                                   model->d_pdf_offsets.as<int32_t>(), P, d_o.as<int32_t>(), nullptr, nullptr,
-                                                   d_p.as<float>(), d_like.as<double>(), model->d_bad.as<unsigned long long>(),
-                                                   d_l.as<float>());
-    VB_CUDA(cudaGetLastError());
-    if (R > 0) VB_CUDA(cudaMemcpy(post, d_p.p, (size_t)R * 4, cudaMemcpyDeviceToHost));
-    if (loglikes) VB_CUDA(cudaMemcpy(loglikes, d_l.p, (size_t)T * 4, cudaMemcpyDeviceToHost));
-    unsigned long long bad = 0;
-    VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
-    if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
-    return 0;
-  };
-  rc = run();
-  for (vb::DevBuf *b : {&d_f, &d_i, &d_w, &d_o, &d_p, &d_l, &d_like}) b->release();
-  return rc;
+  VB_TRY(d_f.reserve((size_t)T * stride * 4));
+  VB_TRY(d_i.reserve((size_t)T * 4));
+  VB_TRY(d_o.reserve((size_t)(T + 1) * 4));
+  VB_TRY(d_p.reserve((size_t)std::max<int64_t>(R, 1) * 4));
+  VB_TRY(d_l.reserve((size_t)T * 4));
+  VB_TRY(d_like.reserve(8));
+  VB_CUDA(cudaMemcpy(d_f.p, feats, (size_t)T * stride * 4, cudaMemcpyHostToDevice));
+  VB_CUDA(cudaMemcpy(d_i.p, pdf_ids, (size_t)T * 4, cudaMemcpyHostToDevice));
+  VB_CUDA(cudaMemcpy(d_o.p, off.data(), (size_t)(T + 1) * 4, cudaMemcpyHostToDevice));
+  VB_CUDA(cudaMemset(d_p.p, 0, (size_t)std::max<int64_t>(R, 1) * 4));
+  VB_CUDA(cudaMemset(d_like.p, 0, 8));
+  VB_CUDA(cudaMemset(model->d_bad.p, 0, 8));
+  const float *dw = nullptr;
+  if (weights) {
+    VB_TRY(d_w.reserve((size_t)T * 4));
+    VB_CUDA(cudaMemcpy(d_w.p, weights, (size_t)T * 4, cudaMemcpyHostToDevice));
+    dw = d_w.as<float>();
+  }
+  const int grid = (int)std::min<int64_t>((T + kWarps - 1) / kWarps, (int64_t)sms * 8);
+  mllt_rows_kernel<false><<<grid, kWarps * 32>>>(d_f.as<float>(), T, stride, model->D, model->DP, d_i.as<int32_t>(), dw,
+                                                 model->d_rows.as<float>(), model->d_gconsts.as<float>(),
+                                                 model->d_pdf_offsets.as<int32_t>(), P, d_o.as<int32_t>(), nullptr, nullptr,
+                                                 d_p.as<float>(), d_like.as<double>(), model->d_bad.as<unsigned long long>(),
+                                                 d_l.as<float>());
+  VB_CUDA(cudaGetLastError());
+  if (R > 0) VB_CUDA(cudaMemcpy(post, d_p.p, (size_t)R * 4, cudaMemcpyDeviceToHost));
+  if (loglikes) VB_CUDA(cudaMemcpy(loglikes, d_l.p, (size_t)T * 4, cudaMemcpyDeviceToHost));
+  unsigned long long bad = 0;
+  VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
+  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  return 0;
 }
 
 }  // extern "C"

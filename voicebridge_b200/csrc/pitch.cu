@@ -565,8 +565,8 @@ __global__ void __launch_bounds__(128) pitch_process_kernel(vbgpu_process_pitch_
 struct vbgpu_pitch_s {
   vbgpu_pitch_opts o;
   int device = 0;
-  cudaStream_t stream = nullptr, copy_stream = nullptr;
-  cudaEvent_t ev_copied[4] = {nullptr, nullptr, nullptr, nullptr};
+  vb::Stream stream, copy_stream;
+  vb::Event ev_copied[4];
   int32_t in_hz = 0, out_hz = 0;
   int32_t last_lag = 0;
   PitchDev dev;
@@ -904,49 +904,22 @@ int vbgpu_pitch_create(const vbgpu_pitch_opts *opts, int device, vbgpu_pitch_t *
            o.resample_freq);
   VB_CHECK(o.min_f0 > 0 && o.max_f0 > o.min_f0 && o.delta_pitch > 0 && o.frame_shift_ms > 0 && o.frame_length_ms > 0,
            "bad pitch search options");
-  {
-    int n_dev = 0;
-    cudaError_t e = cudaGetDeviceCount(&n_dev);
-    if (e != cudaSuccess || n_dev <= 0)
-      return fail(VBGPU_ERR_CUDA, "no CUDA device available (%s); libvbgpu has no CPU fallback",
-                  e == cudaSuccess ? "count=0" : cudaGetErrorString(e));
-    VB_CHECK(device >= 0 && device < n_dev, "device %d out of range [0,%d)", device, n_dev);
-  }
+  VB_TRY(vb::check_device(device));
   DeviceGuard g(device);
-  vbgpu_pitch_s *h = new vbgpu_pitch_s();
+  std::unique_ptr<vbgpu_pitch_s, decltype(&vbgpu_pitch_destroy)> h(new vbgpu_pitch_s(), vbgpu_pitch_destroy);
   h->o = o;
   h->device = device;
-  cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-  if (e != cudaSuccess) {
-    delete h;
-    return fail(VBGPU_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
-  }
-  e = cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
-  for (int k = 0; k < 4 && e == cudaSuccess; k++) e = cudaEventCreateWithFlags(&h->ev_copied[k], cudaEventDisableTiming);
-  if (e != cudaSuccess) {
-    vbgpu_pitch_destroy(h);
-    return fail(VBGPU_ERR_CUDA, "copy stream / events: %s", cudaGetErrorString(e));
-  }
-  int rc = build_plan(h);
-  if (rc < 0) {
-    vbgpu_pitch_destroy(h);
-    return rc;
-  }
-  *out = h;
+  VB_TRY(h->stream.create());
+  VB_TRY(h->copy_stream.create());
+  for (vb::Event &ev : h->ev_copied) VB_TRY(ev.create());
+  VB_TRY(build_plan(h.get()));
+  *out = h.release();
   return 0;
 }
 
 void vbgpu_pitch_destroy(vbgpu_pitch_t h) {
   if (!h) return;
   DeviceGuard g(h->device);
-  for (DevBuf *b : {&h->d_lr_first, &h->d_lr_nw, &h->d_lr_w, &h->d_up_first, &h->d_up_n, &h->d_up_w, &h->d_soft_lag,
-                    &h->d_pitch_hz, &h->d_wave, &h->d_down, &h->d_stats, &h->d_utts, &h->d_nccf, &h->d_pov, &h->d_bp,
-                    &h->d_state, &h->d_raw, &h->d_aux, &h->d_out, &h->d_energy, &h->d_frame_offsets, &h->d_frame2utt})
-    b->release();
-  for (cudaEvent_t ev : h->ev_copied)
-    if (ev) cudaEventDestroy(ev);
-  if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-  if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
 }
 

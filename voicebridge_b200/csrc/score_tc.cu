@@ -1198,12 +1198,7 @@ void note_fallback(vbgpu_gmm_t h, const char *why) {
 namespace vb {
 
 void score_tc_release(vbgpu_gmm_t h) {
-  TcState *st = static_cast<TcState *>(h->tc);
-  if (!st) return;
-  for (DevBuf *b : {&st->d_bimg, &st->d_hdr, &st->d_grp, &st->d_centre, &st->d_s1, &st->d_s2, &st->d_col_of_pdf,
-                    &st->d_merge, &st->d_rowflag, &st->d_fixlist, &st->d_scratch})
-    b->release();
-  delete st;
+  delete static_cast<TcState *>(h->tc);
   h->tc = nullptr;
 }
 
@@ -1238,22 +1233,19 @@ int score_tc_prepare(vbgpu_gmm_t h, const float *gconsts, const float *miv, cons
   }
   const char *single = getenv("VBGPU_TC_SINGLE");
   const bool pair = !(single && atoi(single) != 0);
-  TcState *st = new TcState;
+  std::unique_ptr<TcState> st(new TcState);
   TcHostImage img;
-  const char *why = build_layout(h->D, h->N, h->P, h->h_pdf_offsets, gconsts, miv, iv, stride, pair, st, &img);
+  const char *why = build_layout(h->D, h->N, h->P, h->h_pdf_offsets, gconsts, miv, iv, stride, pair, st.get(), &img);
   if (why) {
-    delete st;
     note_fallback(h, why);
     return 0;
   }
-  int rc = 0;
-  auto up = [&](DevBuf &b, const void *src, size_t bytes) {
-    if (rc == 0) rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc == 0 && bytes && cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess)
-      rc = fail(VBGPU_ERR_CUDA, "upload of the tensor-core model image failed");
+  auto up = [](DevBuf &b, const void *src, size_t bytes) {  // every table gets at least 16 bytes
+    VB_TRY(b.reserve(std::max<size_t>(bytes, 16)));
+    return b.upload(src, bytes);
   };
-  up(st->d_bimg, st->h_bimg.data(), st->h_bimg.size());
-  up(st->d_hdr, img.hdr.data(), img.hdr.size() * sizeof(int4));
+  VB_TRY(up(st->d_bimg, st->h_bimg.data(), st->h_bimg.size()));
+  VB_TRY(up(st->d_hdr, img.hdr.data(), img.hdr.size() * sizeof(int4)));
   {  // dispatch entries per column class (warp >> 2): everything the epilogue would otherwise derive per group
     const size_t ng = img.grp.size();
     std::vector<int2> dev(4 * ng);
@@ -1263,17 +1255,16 @@ int score_tc_prepare(vbgpu_gmm_t h, const float *gconsts, const float *miv, cons
         const int key = (S - 1) + (W == 1 ? 0 : W == 2 ? kSmax : 2 * kSmax);
         dev[cls * ng + g] = make_int2(key | ((col0 + 4 * cls) << 16), img.grp[g].y + cls * (4 / W));
       }
-    up(st->d_grp, dev.data(), dev.size() * sizeof(int2));
+    VB_TRY(up(st->d_grp, dev.data(), dev.size() * sizeof(int2)));
     st->grp_stride = (int)ng;
   }
-  up(st->d_centre, img.centre.data(), h->D * 4);
-  up(st->d_s1, img.s1.data(), h->D * 4);
-  up(st->d_s2, img.s2.data(), h->D * 4);
-  up(st->d_col_of_pdf, st->col_of_pdf.data(), (size_t)h->P * 4);
-  up(st->d_merge, img.merge.data(), img.merge.size() * 4);
-  h->tc = st;
-  if (rc < 0) score_tc_release(h);
-  return rc;
+  VB_TRY(up(st->d_centre, img.centre.data(), h->D * 4));
+  VB_TRY(up(st->d_s1, img.s1.data(), h->D * 4));
+  VB_TRY(up(st->d_s2, img.s2.data(), h->D * 4));
+  VB_TRY(up(st->d_col_of_pdf, st->col_of_pdf.data(), (size_t)h->P * 4));
+  VB_TRY(up(st->d_merge, img.merge.data(), img.merge.size() * 4));
+  h->tc = st.release();
+  return 0;
 }
 
 // Host-only view of the layout (no device needed): what tests/test_tc_layout.py decodes and checks against the oracle.

@@ -137,7 +137,7 @@ struct vbgpu_resample_s {
   int device = 0;
   int32_t in_hz = 0, out_hz = 0, in_unit = 0, out_unit = 0, max_w = 0;
   vb::DevBuf d_first, d_nw, d_w, d_in, d_out;
-  cudaStream_t stream = nullptr;
+  vb::Stream stream;
 };
 
 namespace {
@@ -191,8 +191,10 @@ int vbgpu_downsample_create(float orig_freq, float new_freq, int32_t device, vbg
   VB_CHECK(out, "null argument");
   // the reference asserts new_freq < orig_freq (resample.cc:370); LinearResample takes the rates as int32
   VB_CHECK(new_freq < orig_freq && (int32_t)new_freq >= 1, "downsampling needs 1 <= new_freq (%g) < orig_freq (%g)", new_freq, orig_freq);
+  VB_TRY(vb::check_device(device));
   vb::DeviceGuard g(device);
-  vbgpu_resample_s *h = new (std::nothrow) vbgpu_resample_s;
+  std::unique_ptr<vbgpu_resample_s, decltype(&vbgpu_downsample_destroy)> h(new (std::nothrow) vbgpu_resample_s,
+                                                                             vbgpu_downsample_destroy);
   if (!h) return fail(VBGPU_ERR_NOMEM, "out of host memory");
   h->device = device;
   h->in_hz = (int32_t)orig_freq;
@@ -219,22 +221,11 @@ int vbgpu_downsample_create(float orig_freq, float new_freq, int32_t device, vbg
       w[(size_t)i * h->max_w + j] = filter_func((float)delta_t, cutoff, num_zeros) / h->in_hz;
     }
   }
-  int rc = 0;
-  auto up = [&](vb::DevBuf &b, const void *src, size_t bytes) {
-    if (rc == 0) rc = b.reserve(bytes);
-    if (rc == 0 && cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess)
-      rc = fail(VBGPU_ERR_CUDA, "upload of the resampling tables failed");
-  };
-  up(h->d_first, first.data(), first.size() * 4);
-  up(h->d_nw, nw.data(), nw.size() * 4);
-  up(h->d_w, w.data(), w.size() * 4);
-  if (rc == 0 && cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess)
-    rc = fail(VBGPU_ERR_CUDA, "cudaStreamCreate failed");
-  if (rc < 0) {
-    vbgpu_downsample_destroy(h);
-    return rc;
-  }
-  *out = h;
+  VB_TRY(h->d_first.upload(first.data(), first.size() * 4));
+  VB_TRY(h->d_nw.upload(nw.data(), nw.size() * 4));
+  VB_TRY(h->d_w.upload(w.data(), w.size() * 4));
+  VB_TRY(h->stream.create());
+  *out = h.release();
   return 0;
 }
 
@@ -242,8 +233,6 @@ void vbgpu_downsample_destroy(vbgpu_resample_t h) {
   if (!h) return;
   vb::DeviceGuard g(h->device);
   cudaDeviceSynchronize();
-  for (vb::DevBuf *b : {&h->d_first, &h->d_nw, &h->d_w, &h->d_in, &h->d_out}) b->release();
-  if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
 }
 
