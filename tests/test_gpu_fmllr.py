@@ -1,5 +1,6 @@
-"""fMLLR sufficient statistics on the device (SURVEY.md §8f n1) against the float64 restatement, the plain-C oracle and
-the reference's own FmllrDiagGmmAccs; the reference's solver must land on the same transform from either statistics."""
+"""fMLLR and MLLT sufficient statistics on the device (SURVEY.md §8f n1) against the float64 restatements and the plain-C
+oracle; where the reference is built (oracle/_ref), its solvers must also land on the same transform from the device's
+statistics as from its own."""
 import numpy as np
 import pytest
 
@@ -35,30 +36,97 @@ def test_fmllr_stats_single_speaker(orc, D, weighted, T):
     assert b0 == 0.0 and not K0.any() and not G0.any()
 
 
-def test_fmllr_stats_many_speakers_vs_reference(ref):
-    """A packed batch of ragged utterances from 5 speakers (one of them silent): every speaker's statistics equal the
-    reference's FmllrDiagGmmAccs run over that speaker's frames alone, and FmllrDiagGmmAccs::Update gives the same
-    transform from the device statistics as from its own."""
-    D, P = 39, 40
-    m = _model(ref, P, 300, D, 61)
-    rng = np.random.default_rng(62)
-    lens = [300, 1, 257, 0, 900, 512, 77, 640, 256, 1100]
-    u2s = np.array([0, 0, 1, 1, 2, 2, 4, 4, 4, 0], np.int32)  # speaker 3 has no data
+# A packed batch of (frames, speaker): speakers whose utterances are not adjacent, empty and one-frame utterances inside a
+# speaker's run, runs of 2600 (three 1024-frame work units), exactly 1024 and 1025 frames, and speakers without data.
+MANY_SPEAKERS = [
+    (300, 0),                                     # speaker 0 at the start ...
+    (257, 2), (0, 2), (1, 2), (130, 2),           # 0- and 1-frame utterances inside one run of speaker 2
+    (90, 1), (60, 4), (75, 1), (40, 5), (120, 1),  # speaker 1 interleaved with speakers 4 and 5
+    (1000, 6), (900, 6), (700, 6),                # one run of 2600 frames
+    (1024, 7),                                    # one run of exactly one work unit
+    (600, 8), (425, 8),                           # 1025 frames: a full unit and a one-frame unit
+    (0, 9),                                       # speaker 9: only an empty utterance
+    (100, 4), (0, 1), (50, 4),                    # an empty utterance of speaker 1 inside a run of speaker 4
+    (400, 0),                                     # ... and at the end
+]
+MANY_SPEAKERS_N = 11                              # speakers 3 and 10: no utterance at all
+
+
+@pytest.mark.parametrize("P,N,D,seed", [(5, 300, 13, 3), (40, 900, 39, 61), (12, 700, 40, 5)])
+def test_fmllr_stats_many_speakers(orc, monkeypatch, P, N, D, seed):
+    """Every speaker's statistics of one packed, weighted call equal the float64 restatement over that speaker's frames
+    alone, and the call's log-likelihood the oracle's.  The models hold pdfs of more than 64 Gaussians next to smaller
+    ones, so some frames take the bucketed posterior kernel and the rest fmllr_ab_kernel; VBGPU_ACC_FRAMEWISE sends every
+    frame through fmllr_ab_kernel; the device form reads strided features on a caller's stream.  All three agree with
+    the restatement.  Where the reference is built, FmllrDiagGmmAccs::Update also gives the same transform from the
+    device statistics as from the reference's own."""
+    import torch
+    from oracle import pyoracle as po
+    m = _model(orc, P, N, D, seed)
+    lens = np.array([n for n, _ in MANY_SPEAKERS])
+    u2s = np.array([s for _, s in MANY_SPEAKERS], np.int32)
     fo = np.zeros(len(lens) + 1, np.int64)
     fo[1:] = np.cumsum(lens)
-    T = int(fo[-1])
-    X = synth.make_feats(m, T, 63)
-    ali = synth.make_alignment(P, T, 64)
-    acc = host.FmllrDiagGmmAccsGpu(host.AmDiagGmmGpu.from_model(m), n_spk=5)
-    acc.AccumulateForUtterances(X, ali, frame_offsets=fo, utt2spk=u2s)
-    for s in range(5):
-        rows = np.concatenate([np.arange(fo[u], fo[u + 1]) for u in range(len(lens)) if u2s[u] == s] or [np.zeros(0, int)])
-        b, K, G = acc.stats(s)
-        if len(rows) == 0:
-            assert b == 0.0 and not K.any() and not G.any()
+    T, n_spk = int(fo[-1]), MANY_SPEAKERS_N
+    X = synth.make_feats(m, T, seed + 1)
+    ali = synth.make_alignment(P, T, seed + 2)
+    rng = np.random.default_rng(seed + 3)
+    w = rng.uniform(0.2, 1.0, T).astype(np.float32)
+    w[rng.random(T) < 0.1] = 0.0
+    sizes = np.diff(m.pdf_offsets)
+    big = sizes[ali] > 64  # frames of fmllr_ab_kernel; the rest take the bucketed kernel
+    assert (sizes > 64).any() and (sizes <= 64).any() and big.any() and (~big).any()
+    assert (big & (w == 0)).any() and (big & (w > 0)).any()
+    spk_rows = [np.concatenate([np.arange(fo[u], fo[u + 1]) for u in range(len(lens)) if u2s[u] == s] or [np.zeros(0, int)])
+                for s in range(n_spk)]
+    truth, want_like = {}, 0.0
+    for s, rows in enumerate(spk_rows):
+        if len(rows):
+            truth[s] = fmllr_truth(m, X[rows], ali[rows], w[rows])
+            rc, _, _, _, ol = orc.fmllr_acc(m, X[rows], ali[rows], w[rows])
+            assert rc == 0
+            want_like += ol
+    assert sorted(truth) == [0, 1, 2, 4, 5, 6, 7, 8]
+
+    def check(acc, what):
+        for s in range(n_spk):
+            b, K, G = acc.stats(s)
+            if s not in truth:
+                assert b == 0.0 and not K.any() and not G.any(), "%s: speaker %d has no data" % (what, s)
+            else:
+                assert_fmllr_close((b, K, G), truth[s], what="%s, speaker %d" % (what, s))
+
+    am = host.AmDiagGmmGpu.from_model(m)
+    acc = host.FmllrDiagGmmAccsGpu(am, n_spk=n_spk)
+    tl = acc.AccumulateForUtterances(X, ali, frame_offsets=fo, utt2spk=u2s, weights=w)
+    assert abs(tl - want_like) <= 1e-4 * abs(want_like)
+    check(acc, "GPU")
+    with monkeypatch.context() as mp:
+        mp.setenv("VBGPU_ACC_FRAMEWISE", "1")
+        fw = host.FmllrDiagGmmAccsGpu(am, n_spk=n_spk)
+        tl_fw = fw.AccumulateForUtterances(X, ali, frame_offsets=fo, utt2spk=u2s, weights=w)
+    assert abs(tl_fw - want_like) <= 1e-4 * abs(want_like)
+    check(fw, "GPU frame-wise")
+    # device form: rows D + 5 floats apart (the padding holds values no feature has), on a non-default stream
+    d_x = torch.full((T, D + 5), 1e3, dtype=torch.float32, device="cuda")
+    d_x[:, :D] = torch.from_numpy(X).cuda()
+    d_ids, d_w = torch.from_numpy(ali).cuda(), torch.from_numpy(w).cuda()
+    torch.cuda.synchronize()
+    stream = torch.cuda.Stream()
+    dev = host.FmllrDiagGmmAccsGpu(am, n_spk=n_spk)
+    dev.accumulate_dev(d_x, T, D + 5, d_ids, fo, u2s, d_w, stream=stream)
+    stream.synchronize()
+    check(dev, "GPU device form")
+    for s in truth:  # the same statistics as the host form (FP64 atomics: equal up to the order of the additions)
+        assert_fmllr_close(dev.stats(s), (*acc.stats(s), *truth[s][3:]), what="device form vs host form, speaker %d" % s)
+    if not po.have_ref():
+        return
+    ref = po.load("ref")
+    for s, rows in enumerate(spk_rows):
+        if s not in truth:
             continue
-        assert_fmllr_close((b, K, G), fmllr_truth(m, X[rows], ali[rows]), what="GPU, speaker %d" % s)
-        rc, rb, rK, rG, _ = ref.fmllr_acc(m, X[rows], ali[rows])
+        b, K, G = acc.stats(s)
+        rc, rb, rK, rG, _ = ref.fmllr_acc(m, X[rows], ali[rows], w[rows])
         assert rc == 0
         r1, x_gpu, i1, c1 = ref.fmllr_update(b, K, G)
         r2, x_ref, i2, c2 = ref.fmllr_update(rb, rK, rG)
@@ -123,14 +191,26 @@ def test_fmllr_stats_full_size_properties():
 
 
 # ------------------------------------------------------------------------------------------ MLLT statistics (gmm-acc-mllt)
-@pytest.mark.parametrize("D,weighted,T", [(40, False, 900), (13, True, 700), (39, True, 1)])
-def test_mllt_stats(orc, ref, D, weighted, T):
+@pytest.mark.parametrize("D,weighted,T,model", [
+    pytest.param(40, False, 900, (20, 150, 3), id="40-False-900"),
+    pytest.param(13, True, 700, (20, 150, 3), id="13-True-700"),
+    pytest.param(39, True, 1, (20, 150, 3), id="39-True-1"),
+    # pdfs of up to 123 Gaussians: several 32-Gaussian passes of mllt_rows_kernel, and more than 64 per pdf
+    pytest.param(39, True, 900, (12, 700, 5), id="39-True-900-large-pdfs"),
+    pytest.param(40, True, 900, (12, 700, 5), id="40-True-900-large-pdfs"),
+])
+def test_mllt_stats(orc, D, weighted, T, model):
     """MlltAccs on the device (the fMLLR G contraction over one pseudo-frame per (frame, Gaussian)) against the float64
-    restatement, the oracle, and through the reference's own MlltAccs::Update."""
+    restatement and the oracle; where the reference is built, also through its own MlltAccs::Update."""
+    from oracle import pyoracle as po
     from tests.common import mllt_truth
-    m = _model(orc, 20, 150, D, 3)
+    P, N, seed = model
+    m = _model(orc, P, N, D, seed)
+    if model[0] == 12:
+        sizes = np.diff(m.pdf_offsets)
+        assert (sizes > 64).any() and ((sizes > 32) & (sizes <= 64)).any() and (sizes <= 32).any()
     X = synth.make_feats(m, T, 4)
-    ali = synth.make_alignment(20, T, 5)
+    ali = synth.make_alignment(P, T, 5)
     w = np.random.default_rng(1).uniform(0.2, 1.0, T).astype(np.float32) if weighted else None
     acc = host.MlltAccsGpu(host.AmDiagGmmGpu.from_model(m))
     tl = acc.AccumulateForUtterance(X, ali, w)
@@ -139,7 +219,8 @@ def test_mllt_stats(orc, ref, D, weighted, T):
     tb, tG, SG = mllt_truth(m, X, ali, w)
     assert abs(acc.beta - tb) <= 1e-4 * max(tb, 1.0)
     assert (np.abs(acc.G - tG) / np.maximum(SG, 1e-30)).max() <= 1e-4
-    if T >= 700:
+    if T >= 700 and po.have_ref():
+        ref = po.load("ref")
         r1, M1, i1, c1 = ref.mllt_update(acc.beta, acc.G)
         r2, M2, i2, c2 = ref.mllt_update(ob, oG)
         assert r1 == 0 and r2 == 0 and np.abs(M1 - M2).max() <= 1e-3 and abs(i1 - i2) <= 1e-3 * max(abs(i2), 1.0)
@@ -147,14 +228,49 @@ def test_mllt_stats(orc, ref, D, weighted, T):
     assert abs(acc.beta - 2 * tb) <= 2e-4 * max(tb, 1.0)
 
 
+def _mllt_truth_by_pdf(model, X, ali, chunk=256):
+    """tests.common.mllt_truth (unweighted) with the frames of each pdf taken a chunk at a time: the same sums, fast
+    enough for tens of thousands of frames."""
+    X = np.asarray(X, np.float64)
+    D = X.shape[1]
+    gc, miv, iv = (np.asarray(v, np.float64) for v in (model.gconsts, model.miv, model.iv))
+    rr, cc = np.tril_indices(D)
+    G, SG = np.zeros((D, len(rr))), np.zeros((D, len(rr)))
+    beta = 0.0
+    for p in np.unique(ali):
+        g0, g1 = model.pdf_offsets[p], model.pdf_offsets[p + 1]
+        idx = np.flatnonzero(ali == p)
+        for c0 in range(0, len(idx), chunk):
+            x = X[idx[c0:c0 + chunk]]                                               # [n, D]
+            ll = gc[g0:g1] + x @ miv[g0:g1].T - 0.5 * ((x * x) @ iv[g0:g1].T)       # [n, M]
+            post = np.exp(ll - ll.max(axis=1, keepdims=True))
+            post /= post.sum(axis=1, keepdims=True)
+            off = (miv[g0:g1] / iv[g0:g1])[None] - x[:, None, :]                    # [n, M, D]
+            z = (off[:, :, rr] * off[:, :, cc]).reshape(-1, len(rr))               # [n M, pairs]
+            a = (iv[g0:g1][None] * post[:, :, None]).reshape(-1, D)               # [n M, D]
+            G += a.T @ z
+            SG += a.T @ np.abs(z)
+            beta += post.sum()
+    return beta, G, SG
+
+
 def test_mllt_stats_many_slabs_and_bad_ids(orc):
+    from tests.common import mllt_truth
     m = _model(orc, 30, 900, 39, 8)  # ~30 Gaussians per pdf: 60 000 frames make several row slabs
     T = 60000
     X = synth.make_feats(m, T, 9)
     ali = synth.make_alignment(30, T, 10)
+    assert np.diff(m.pdf_offsets)[ali].sum() > 1500000  # (frame, Gaussian) rows beyond one slab (kMaxRows)
     am = host.AmDiagGmmGpu.from_model(m)
     whole = host.MlltAccsGpu(am)
     whole.AccumulateForUtterance(X, ali)
+    # the grouped restatement is the per-frame one, and the device result of many slabs matches it
+    b1, G1, _ = _mllt_truth_by_pdf(m, X[:300], ali[:300])
+    b2, G2, S2 = mllt_truth(m, X[:300], ali[:300])
+    assert abs(b1 - b2) <= 1e-12 * b2 and (np.abs(G1 - G2) / np.maximum(S2, 1e-30)).max() <= 1e-12
+    tb, tG, SG = _mllt_truth_by_pdf(m, X, ali)
+    assert abs(whole.beta - tb) <= 1e-4 * tb
+    assert (np.abs(whole.G - tG) / np.maximum(SG, 1e-30)).max() <= 1e-4
     parts = host.MlltAccsGpu(am)
     for a, b in ((0, 7), (7, 25000), (25000, T)):
         parts.AccumulateForUtterance(X[a:b], ali[a:b])

@@ -518,19 +518,34 @@ def test_fbank_single_utterance(orc, kw, use_log, use_power):
     assert np.array_equal(got, fb.ComputeFeatures(w.astype(np.float32)))
 
 
-def test_fbank_batch_vtln_vs_reference(ref):
+# per-utterance VTLN warps of one ragged batch: 0.9 and 1.1 come back after other warps, 1.0 (no warp) sits between them
+BATCH_VTLN_LENS = [0, 399, 400, 4801, 16000, 7777, 3000, 5000, 2500]
+BATCH_VTLN_WARPS = [1.0, 0.9, 1.1, 1.0, 0.85, 1.2, 0.9, 1.1, 1.0]
+
+
+def _batch_vtln_wave():
+    so = np.zeros(len(BATCH_VTLN_LENS) + 1, np.int64)
+    so[1:] = np.cumsum(BATCH_VTLN_LENS)
+    return synth.make_wave(int(so[-1]), 3), so, np.array(BATCH_VTLN_WARPS, np.float32)
+
+
+@pytest.mark.parametrize("use_log,use_power", [(1, 1), (0, 1), (1, 0)])
+def test_fbank_batch_vtln(orc, use_log, use_power):
+    """A ragged batch with a VTLN warp per utterance (per-warp mel banks on the device): every utterance equals the oracle
+    run on it alone with its warp, and the reference's own code where it is built."""
     o = gopts(use_energy=1)
-    lens = [0, 399, 400, 4801, 16000, 7777]
-    so = np.zeros(len(lens) + 1, np.int64)
-    so[1:] = np.cumsum(lens)
-    pcm = synth.make_wave(int(so[-1]), 3)
-    vtln = np.array([1.0, 0.9, 1.1, 1.0, 0.85, 1.2], np.float32)
-    fb = host.Fbank(o)
+    pcm, so, vtln = _batch_vtln_wave()
+    fb = host.Fbank(o, use_log, use_power)
     got, fo = fb.compute_batch(pcm, so, vtln)
     oo = to_orc_opts(o)
-    for u in range(len(lens)):
-        want = ref.fbank(oo, pcm[so[u]:so[u + 1]].astype(np.float32), float(vtln[u]))
-        assert_feats_close(got[fo[u]:fo[u + 1]], want, what="fbank utt %d" % u)
+    ref = po.load("ref") if po.have_ref() else None
+    for u in range(len(so) - 1):
+        w = pcm[so[u]:so[u + 1]].astype(np.float32)
+        want = orc.fbank(oo, w, float(vtln[u]), use_log, use_power)
+        assert_feats_close(got[fo[u]:fo[u + 1]], want, what="fbank utt %d (warp %g)" % (u, vtln[u]))
+        if ref is not None:
+            assert_feats_close(got[fo[u]:fo[u + 1]], ref.fbank(oo, w, float(vtln[u]), use_log, use_power),
+                               what="fbank utt %d vs reference" % u)
 
 
 # ================================================================================== host threads (nj jobs of the recipes)
@@ -582,18 +597,19 @@ def test_plp_single_utterance(orc, kw):
         assert np.array_equal(got, plp.ComputeFeatures(w.astype(np.float32)))
 
 
-def test_plp_batch_vtln_vs_reference(ref):
+def test_plp_batch_vtln(orc):
+    """PLP of the same ragged VTLN batch (per-warp mel banks and equal-loudness tables): every utterance equals the oracle
+    with its warp, and the reference's own code where it is built."""
     o = gopts(use_energy=1)
-    lens = [0, 399, 400, 4801, 16000, 7777]
-    so = np.zeros(len(lens) + 1, np.int64)
-    so[1:] = np.cumsum(lens)
-    pcm = synth.make_wave(int(so[-1]), 3)
-    vtln = np.array([1.0, 0.9, 1.1, 1.0, 0.85, 1.2], np.float32)
+    pcm, so, vtln = _batch_vtln_wave()
     got, fo = host.Plp(o).compute_batch(pcm, so, vtln)
     oo = to_orc_opts(o)
-    for u in range(len(lens)):
-        want = ref.plp(oo, pcm[so[u]:so[u + 1]].astype(np.float32), float(vtln[u]))
-        assert_feats_close(got[fo[u]:fo[u + 1]], want, what="plp utt %d" % u)
+    ref = po.load("ref") if po.have_ref() else None
+    for u in range(len(so) - 1):
+        w = pcm[so[u]:so[u + 1]].astype(np.float32)
+        assert_feats_close(got[fo[u]:fo[u + 1]], orc.plp(oo, w, float(vtln[u])), what="plp utt %d (warp %g)" % (u, vtln[u]))
+        if ref is not None:
+            assert_feats_close(got[fo[u]:fo[u + 1]], ref.plp(oo, w, float(vtln[u])), what="plp utt %d vs reference" % u)
     with pytest.raises(capi.VbgpuError):  # num_ceps > lpc_order + 1 (feature-plp.cc:126)
         host.Plp(gopts(num_ceps=13), lpc_order=8)
 

@@ -1,5 +1,5 @@
 """Kaldi pitch on the device (SURVEY.md §8f n4: ComputeKaldiPitch, ProcessPitch, ComputeAndProcessKaldiPitch) against the
-plain-C oracle, the reference's own code (oracle/_ref, when it travelled) and the committed dumps of the compiled
+plain-C oracle, the reference's own code (oracle/_ref, where it is built) and the committed dumps of the compiled
 reference (tests/golden/pitch_golden.npz).  Tolerances: see tests.common.assert_pitch_close."""
 import os
 
@@ -61,10 +61,12 @@ def test_pitch_golden_dumps_of_the_reference():
     assert_process_pitch_close(p.Process(pv, g["raw16"]), g["proc16_variant"])
 
 
-def test_pitch_ragged_batch_vs_reference(ref):
-    """Empty, shorter-than-a-window, one-frame and long utterances in one packed batch: every utterance equals the
-    reference run on it alone (no leakage across utterance boundaries)."""
-    o = capi.default_pitch_opts()
+@pytest.mark.parametrize("kw", [PITCH_VARIANTS[0], PITCH_VARIANTS[1], PITCH_VARIANTS[6]],
+                         ids=lambda d: ",".join("%s=%s" % kv for kv in d.items()) or "default")
+def test_pitch_ragged_batch(orc, kw):
+    """Empty, shorter-than-a-window, one-frame and long utterances in one packed batch: every utterance equals the oracle
+    run on it alone (no leakage across utterance boundaries), and the reference's own code where it is built."""
+    o = capi.default_pitch_opts(**kw)
     lens = [0, 300, 399, 400, 560, 1700, 16000, 48000, 0, 131072, 7777]
     so = np.zeros(len(lens) + 1, np.int64)
     so[1:] = np.cumsum(lens)
@@ -72,12 +74,14 @@ def test_pitch_ragged_batch_vs_reference(ref):
     p = host.Pitch(o)
     got, ro = p.compute_batch(pcm, so)
     oo = orc_opts(o)
-    n_diff = 0
-    for u, n in enumerate(lens):
-        want = ref.pitch(oo, pcm[so[u]:so[u + 1]].astype(np.float32))
-        assert ro[u + 1] - ro[u] == len(want) == p.NumFrames(n)
-        n_diff += assert_pitch_close(got[ro[u]:ro[u + 1]], want, what="utt %d (%d samples)" % (u, n)) or 0
-    assert n_diff <= 0.03 * len(got)
+    checkers = [("oracle", orc)] + ([("reference", po.load("ref"))] if po.have_ref() else [])
+    for name, chk in checkers:
+        n_diff = 0
+        for u, n in enumerate(lens):
+            want = chk.pitch(oo, pcm[so[u]:so[u + 1]].astype(np.float32))
+            assert ro[u + 1] - ro[u] == len(want) == p.NumFrames(n)
+            n_diff += assert_pitch_close(got[ro[u]:ro[u + 1]], want, what="utt %d (%d samples) vs %s" % (u, n, name)) or 0
+        assert n_diff <= 0.03 * len(got), "%s: %d of %d frames on a different lag state" % (name, n_diff, len(got))
 
 
 def test_pitch_energy_correction(orc):

@@ -199,3 +199,179 @@ def test_wav_files_to_feature_archive_like_make_mfcc(ref):
         assert_feats_close(back, ref.mfcc(oo, waves[key].astype(np.float32)))
         seen += 1
     assert seen == len(waves)
+
+
+# ---------------------------------------------------------------------- matrix objects built here, without the reference
+# The bytes of FM / DM / CM / CM2 / CM3 objects as Matrix::Write and CompressedMatrix::Write lay them out
+# (kaldi-matrix.cc, compressed-matrix.cc:568-600), and CompressedMatrix::CopyToMat restated in NumPy with every float32 and
+# float64 step explicit.  The library must expand them to the same bits on the host and on the device.
+def _int32(v):
+    return b"\x04" + np.int32(v).tobytes()  # WriteBasicType: a size byte, then the value
+
+
+def _plain_obj(m, token):
+    with np.errstate(over="ignore"):
+        m = np.asarray(m, np.float32 if token == "FM" else np.float64)
+    return b"\0B" + token.encode() + b" " + _int32(m.shape[0]) + _int32(m.shape[1]) + m.tobytes()
+
+
+def _packed_obj(token, min_value, range_, rows, cols, payload):
+    head = np.array([min_value, range_], np.float32).tobytes() + np.array([rows, cols], np.int32).tobytes()
+    return b"\0B" + token.encode() + b" " + head + payload
+
+
+def _u16_to_float(mn, rg, q):  # min_value + range * 1.52590218966964e-05F * value, all in float
+    return (rg * np.float32(1.52590218966964e-05)) * np.asarray(q).astype(np.float32) + mn
+
+
+def _char_to_float(p0, p25, p75, p100, v):
+    """CharToFloat: p + (q - p) * k * (1/c.0), the float product (q - p) * k widened to double, scaled and added to p
+    there, then narrowed."""
+    v = np.asarray(v).astype(np.int32)
+    lo, mid = v <= 64, v <= 192
+    base = np.where(lo, p0, np.where(mid, p25, p75))
+    diff = np.where(lo, p25 - p0, np.where(mid, p75 - p25, p100 - p75))
+    k = np.where(lo, v, np.where(mid, v - 64, v - 192)).astype(np.float32)
+    scale = np.where(lo, 1 / 64.0, np.where(mid, 1 / 128.0, 1 / 63.0))
+    with np.errstate(over="ignore"):
+        prod = diff * k  # float32 [rows, cols]
+    return (base.astype(np.float64) + prod.astype(np.float64) * scale).astype(np.float32)
+
+
+def _copy_to_mat(token, min_value, range_, rows, cols, payload):
+    mn, rg = np.float32(min_value), np.float32(range_)
+    with np.errstate(over="ignore"):
+        if token == "CM":
+            hdr = np.frombuffer(payload, np.uint16, 4 * cols).reshape(cols, 4)
+            v = np.frombuffer(payload, np.uint8, rows * cols, 8 * cols).reshape(cols, rows).T
+            p = _u16_to_float(mn, rg, hdr)  # [cols, 4]
+            return _char_to_float(p[:, 0], p[:, 1], p[:, 2], p[:, 3], v)
+        dt, n = (np.uint16, 65535.0) if token == "CM2" else (np.uint8, 255.0)
+        inc = np.float32(np.float64(rg) * (1.0 / n))  # increment = range * (1.0 / 65535.0), narrowed to float
+        return np.frombuffer(payload, dt, rows * cols).reshape(rows, cols).astype(np.float32) * inc + mn
+
+
+# (p0, p25, p75, p100) quantiles of special columns: equal, descending, at the ends of the uint16 range
+_SPECIAL_HEADERS = [(0, 0, 0, 0), (65535, 65535, 65535, 65535), (30000, 30000, 30000, 30000), (65535, 40000, 1000, 0),
+                    (0, 0, 65535, 65535), (0, 65535, 0, 65535), (12345, 12346, 54321, 54322), (1, 32768, 32767, 65534),
+                    (11486, 53298, 60000, 65535), (0, 11486, 53298, 65535)]  # (the last two: see the boundary test)
+_RANGES = [(-3.5, 0.0), (0.0, 0.0), (-123.456, 250.75), (1.5, 1e-3), (-1e38, 2e38)]
+_SHAPES = [(1, 1), (3, 1), (31, 33), (256, 70), (300, 13)]
+
+
+def _cm_case(token, mn, rg, rows, cols, seed):
+    rng = np.random.default_rng(seed)
+    if token == "CM":
+        hdr = np.sort(rng.integers(0, 65536, (cols, 4)), axis=1).astype(np.uint16)
+        for j, h in enumerate(_SPECIAL_HEADERS[:cols]):
+            hdr[(j * 5) % cols] = h
+        # every byte value in every column (when rows >= 256), at a different row per column
+        v = ((np.arange(rows)[:, None] * 7 + np.arange(cols)[None, :] * 3) % 256).astype(np.uint8)
+        payload = hdr.tobytes() + np.ascontiguousarray(v.T).tobytes()
+    elif token == "CM2":
+        v = rng.integers(0, 65536, (rows, cols)).astype(np.uint16)
+        v.flat[:2] = (0, 65535)[:v.size]
+        payload = v.tobytes()
+    else:
+        v = ((np.arange(rows * cols) * 13 + seed) % 256).astype(np.uint8).reshape(rows, cols)
+        payload = v.tobytes()
+    return _packed_obj(token, mn, rg, rows, cols, payload), _copy_to_mat(token, mn, rg, rows, cols, payload)
+
+
+def _plain_case(token, rows, cols, seed):
+    m = np.random.default_rng(seed).standard_normal((rows, cols)) * 1e3
+    special = [np.nan, np.inf, -np.inf, -0.0, 1e39, -1e39, 1e-40, 1e-50, 1 + 2.0 ** -24, 1 + 3 * 2.0 ** -24,
+               -(1 + 2.0 ** -24), 3.4028235677973366e38]
+    m.flat[:len(special)] = special[:m.size]
+    with np.errstate(over="ignore"):  # Matrix<float>::Read of a DM object: element-wise (float) narrowing, to nearest
+        want = m.astype(np.float32)
+    return _plain_obj(m, token), want
+
+
+def _matrix_cases():
+    cases = []
+    for token in ("CM", "CM2", "CM3"):
+        for i, (mn, rg) in enumerate(_RANGES):
+            for j, (r, c) in enumerate(_SHAPES):
+                cases.append(("%s-min%g-range%g-%dx%d" % (token, mn, rg, r, c), token, r, c, 31 * i + j))
+    for token in ("FM", "DM"):
+        for j, (r, c) in enumerate(_SHAPES):
+            cases.append(("%s-%dx%d" % (token, r, c), token, r, c, j))
+    return cases
+
+
+def _build(token, rows, cols, seed):
+    if token in ("FM", "DM"):
+        return _plain_case(token, rows, cols, seed)
+    i = seed // 31
+    return _cm_case(token, *_RANGES[i], rows, cols, seed)
+
+
+MATRIX_CASES = _matrix_cases()
+
+
+def assert_same_bits(got, want, what=""):
+    """Bit for bit (the sign of zero included), with any NaN matching any NaN: a NaN's payload after narrowing is the
+    hardware's choice."""
+    got, want = np.asarray(got, np.float32), np.asarray(want, np.float32)
+    assert got.shape == want.shape, (what, got.shape, want.shape)
+    nan = np.isnan(want)
+    assert np.array_equal(np.isnan(got), nan), what + ": NaN pattern differs"
+    bad = np.flatnonzero(got.view(np.uint32)[~nan] != want.view(np.uint32)[~nan])
+    assert bad.size == 0, "%s: %d elements differ, first %r vs %r" % (what, bad.size, got[~nan][bad[0]], want[~nan][bad[0]])
+
+
+def test_copy_to_mat_restatement_sees_the_quantile_boundaries():
+    """The cases above must tell CharToFloat's three ranges apart at 64 | 65 and 192 | 193: for some column, the value
+    of byte 64 (first range) differs in its bits from p25 (where the second range starts), and likewise byte 192 from
+    p75.  Otherwise moving a boundary by one would go unseen."""
+    mn, rg = _RANGES[2]
+    cols = 70
+    b, want = _cm_case("CM", mn, rg, 256, cols, 7)
+    hdr = np.frombuffer(b[2 + 3 + 16:2 + 3 + 16 + 8 * cols], np.uint16).reshape(cols, 4)
+    p = _u16_to_float(np.float32(mn), np.float32(rg), hdr)
+    at = lambda v: _char_to_float(p[:, 0], p[:, 1], p[:, 2], p[:, 3], np.full(cols, v))
+    assert (at(64) != p[:, 1]).any() and (at(192) != p[:, 2]).any()
+    assert np.array_equal(at(0), p[:, 0]) and np.array_equal(at(65), _char_to_float(p[:, 0], p[:, 1], p[:, 2], p[:, 3],
+                                                                                       np.full(cols, 65)))
+
+
+@pytest.mark.parametrize("name,token,rows,cols,seed", MATRIX_CASES, ids=[c[0] for c in MATRIX_CASES])
+def test_read_matrix_matches_copy_to_mat(name, token, rows, cols, seed):
+    """Host expansion (vbgpu_io_read_matrix) of objects built here: bit-identical to the restatement, into a row
+    stride wider than cols with the padding untouched, and from inside an archive at an odd byte offset."""
+    b, want = _build(token, rows, cols, seed)
+    info = kio.object_info(b)
+    assert kio.KINDS[info.kind] == token and (info.rows, info.cols) == (rows, cols) and info.total_bytes == len(b)
+    assert_same_bits(kio.read_matrix(b), want, name)
+    stride = cols + 5
+    out = np.full((rows, stride), -7.0, np.float32)
+    a = np.frombuffer(b, np.uint8)
+    capi.check(capi.lib().vbgpu_io_read_matrix(a.ctypes.data, len(a), out.ctypes.data, stride))
+    assert_same_bits(out[:, :cols], want, name + " strided")
+    assert (out[:, cols:] == -7.0).all()
+    ark = kio.write_ark_entry("k1", kio.write_matrix(np.ones((2, 3), np.float32))) + kio.write_ark_entry("u7", b)
+    (_, _, o1), (k2, i2, o2) = list(kio.read_ark(ark))
+    assert k2 == "u7" and o2 % 2 == 1 and i2.total_bytes == len(b)
+    assert_same_bits(kio.read_matrix(ark, o2), want, name + " in an archive")
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name,token,rows,cols,seed", MATRIX_CASES, ids=[c[0] for c in MATRIX_CASES])
+def test_matrix_to_device_matches_copy_to_mat(name, token, rows, cols, seed):
+    """Device expansion (expand_cm_kernel / expand_linear_kernel / narrow_kernel / the strided copy) of the same objects:
+    bit-identical to the restatement, the stride padding untouched, also from an odd offset inside an archive."""
+    import torch
+    b, want = _build(token, rows, cols, seed)
+    ark = kio.write_ark_entry("k", b"") + kio.write_ark_entry("u7", b)
+    off = ark.index(b"\0B")
+    assert off % 2 == 1
+    for buf, at in ((b, 0), (ark, off)):
+        stride = cols + 3
+        d_out = torch.full((rows, stride), -7.0, dtype=torch.float32, device="cuda")
+        scratch = torch.empty(len(b) + 16, dtype=torch.uint8, device="cuda")
+        kio.matrix_to_device(buf, d_out, stride, scratch, offset=at)
+        torch.cuda.synchronize()
+        got = d_out.cpu().numpy()
+        assert_same_bits(got[:, :cols], want, "%s at offset %d" % (name, at))
+        assert (got[:, cols:] == -7.0).all()
