@@ -128,6 +128,9 @@ CASES = [
     ("one Gaussian per pdf", lambda: synth.make_model(50, 50, 39, 4)),
     ("large pdfs: 41, 100, 600 Gaussians", lambda: sized_model([3, 41, 100, 7, 600, 12, 20, 21, 40, 10, 11], 39, 5)),
     ("single pdf", lambda: sized_model([9], 20, 6)),
+    ("D=24 (KS=4)", lambda: sized_model([1, 1, 2, 5, 9, 10, 11, 14, 20, 21, 33, 40, 57, 3, 1, 7], 24, 7)),
+    ("D=31 (KS=4)", lambda: synth.make_model(90, 600, 31, 8)),
+    ("D=47 (KS=6)", lambda: sized_model([1, 4, 12, 25, 41, 2, 1, 18, 39, 6, 1, 1, 30], 47, 9)),
 ]
 
 
@@ -138,6 +141,7 @@ def test_layout_reproduces_oracle_loglikes(orc, name, make, pair):
     feats = synth.make_feats(model, 96, 11)
     lay, why = tc_layout(model, pair)
     assert lay is not None, why
+    assert lay["KS"] == (2 * model.dim + 2 + 15) // 16   # the K-step instantiation the device would launch
     P = model.num_pdfs
     col = lay["col_of_pdf"]
     assert len(set(col.tolist())) == P and col.min() >= 0 and col.max() < lay["n_cols"]
