@@ -277,7 +277,13 @@ int vbgpu_gmm_score_gather(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t
                            const int32_t *pdfs, int64_t n, float *out);
 int vbgpu_gmm_score_gather_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *frames,
                                const int32_t *pdfs, int64_t n, float *d_out, void *stream);
-/* Number of NaN/Inf values produced by _dev calls since the last query (synchronises the handle's work). */
+/* Errors counted by _dev calls on the model since the last query; resets the count (synchronises the device).  It adds up:
+ *   - NaN/Inf log-likelihoods of the _dev scoring calls, vbgpu_pipeline_score*_dev included;
+ *   - invalid pdf-ids and NaN/Inf likelihoods of vbgpu_acc_accumulate_dev, vbgpu_fmllr_accumulate_dev and
+ *     vbgpu_pipeline_accumulate_dev;
+ *   - out-of-range ids of vbgpu_acc_accumulate_transitions_dev.
+ * Host forms (synchronous calls on host buffers) report their own errors through their return code only and leave this
+ * count alone. */
 int vbgpu_gmm_bad_count(vbgpu_gmm_t h, int64_t *count);
 /* Frames of the handle's last scoring launch that the tensor-core path handed to the FP32 kernel: features outside the
  * fp16 scaling plan, or every score so low (below -27000 nats) that the padding columns of the layout would show through.

@@ -464,7 +464,7 @@ int bin_sort_launch(const int32_t *d_ids, int64_t T, int32_t P, const int32_t *d
 }
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
-               const int32_t *d_ids, const float *d_w, cudaStream_t s) {
+               const int32_t *d_ids, const float *d_w, unsigned long long *bad, cudaStream_t s) {
   if (T == 0) return 0;
   vbgpu_gmm_t g = h->model;
   if (g->D > kMaxD) return fail(VBGPU_ERR_INVALID, "feature dim %d > %d", g->D, kMaxD);
@@ -478,8 +478,7 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
   if (bucket) {
     // counting sort of the frames by pdf, then (pdf, chunk) work units
     BinSort bs;
-    VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), h->device, &h->d_work,
-                           g->d_bad.as<unsigned long long>(), s, &bs));
+    VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), h->device, &h->d_work, bad, s, &bs));
     if (!h->bucket_attr_set) {
       VB_CUDA(cudaFuncSetAttribute(acc_bucket_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       h->bucket_attr_set = true;
@@ -488,8 +487,8 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
     const int g2 = (int)std::min<int64_t>(max_units, (int64_t)sms * 3);
     acc_bucket_kernel<<<g2, kWarps * 32, smem, s>>>(d_feats, d_feats2, stride, g->D, g->DP, DY, d_w, g->d_rows.as<float>(),
                                                     g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, bs.start,
-                                                    bs.unit_off, bs.order, h->d_acc.as<double>(),
-                                                    g->d_bad.as<unsigned long long>(), nullptr, 0, nullptr, nullptr);
+                                                    bs.unit_off, bs.order, h->d_acc.as<double>(), bad, nullptr, 0, nullptr,
+                                                    nullptr);
     VB_CUDA(cudaGetLastError());
     if (g->max_pdf_size <= kMaxM) return 0;
   }
@@ -498,7 +497,7 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
   int grid = (int)(blocks < cap ? blocks : cap);
   acc_kernel<<<grid, kWarps * 32, 0, s>>>(d_feats, d_feats2, T, stride, g->D, g->DP, d_ids, d_w, g->d_rows.as<float>(),
                                           g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), g->P, g->N,
-                                          h->d_acc.as<double>(), g->d_bad.as<unsigned long long>(), bucket ? kMaxM : 0);
+                                          h->d_acc.as<double>(), bad, bucket ? kMaxM : 0);
   VB_CUDA(cudaGetLastError());
   return 0;
 }
@@ -507,11 +506,10 @@ int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64
 // for every frame whose pdf has at most kMaxM Gaussians; returns that bound so that the caller serves the rest.
 int acc_posterior_ab_launch(vbgpu_gmm_t g, DevBuf *work, const float *d_feats, int64_t T, int32_t stride,
                             const int32_t *d_ids, const float *d_w, float *d_ab, int32_t ab_pitch, float *d_cnt,
-                            double *d_like, int32_t *max_gauss_served, cudaStream_t s) {
+                            double *d_like, int32_t *max_gauss_served, unsigned long long *bad, cudaStream_t s) {
   const int P = g->P, sms = num_sms(g->device);
   BinSort bs;
-  VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), g->device, work, g->d_bad.as<unsigned long long>(),
-                         s, &bs));
+  VB_TRY(bin_sort_launch(d_ids, T, P, g->d_pdf_offsets.as<int32_t>(), g->device, work, bad, s, &bs));
   const int DY = (g->D + 3) / 4 * 4;
   const size_t smem = ((size_t)kChunk * DY + (size_t)2 * g->D * kMP + (size_t)kChunk * kMP) * 4;
   // (per device: set on every call — a process may drive several GPUs, and the call costs microseconds)
@@ -520,8 +518,7 @@ int acc_posterior_ab_launch(vbgpu_gmm_t g, DevBuf *work, const float *d_feats, i
   const int g2 = (int)std::min<int64_t>(max_units, (int64_t)sms * 3);
   acc_bucket_kernel<<<g2, kWarps * 32, smem, s>>>(d_feats, nullptr, stride, g->D, g->DP, DY, d_w, g->d_rows.as<float>(),
                                                   g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), P, g->N, bs.start,
-                                                  bs.unit_off, bs.order, nullptr, g->d_bad.as<unsigned long long>(), d_ab, ab_pitch,
-                                                  d_cnt, d_like);
+                                                  bs.unit_off, bs.order, nullptr, bad, d_ab, ab_pitch, d_cnt, d_like);
   VB_CUDA(cudaGetLastError());
   *max_gauss_served = kMaxM;
   return 0;

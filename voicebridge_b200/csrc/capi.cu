@@ -672,12 +672,15 @@ static bool uses_tc(vbgpu_gmm_t h) { return h->kernel == 2 || (h->kernel == 0 &&
 // Columns of the natively laid out score matrix (device column order): the tensor-core kernel's, or P (identity).
 static int32_t native_cols(vbgpu_gmm_t h) { return uses_tc(h) ? score_tc_num_cols(h) : h->P; }
 
+// Message of a host scoring form whose call produced NaN/Inf log-likelihoods.
+static const char kBadLoglikes[] = "%llu NaN/Inf log-likelihoods (overflow or invalid variances/features?)";
+
 // native: d_ll in device column order (see vbgpu_gmm_score_cols_dev), else in the model's pdf order.
 static int score_dispatch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, float *d_ll,
-                          int32_t ll_stride, bool native, cudaStream_t s) {
+                          int32_t ll_stride, bool native, unsigned long long *bad, cudaStream_t s) {
   VB_TRY(h->order.enter(s));  // the handle's scratch (row flags, gather scratch) may still be in use on another stream
-  VB_TRY(uses_tc(h) ? score_tc_launch(h, d_feats, T, stride, d_ll, ll_stride, native ? 1 : 0, s)
-                    : score_simt_launch(h, d_feats, T, stride, d_ll, ll_stride, s));
+  VB_TRY(uses_tc(h) ? score_tc_launch(h, d_feats, T, stride, d_ll, ll_stride, native ? 1 : 0, bad, s)
+                    : score_simt_launch(h, d_feats, T, stride, d_ll, ll_stride, bad, s));
   return h->order.leave(s);
 }
 
@@ -688,7 +691,8 @@ int vbgpu_gmm_score_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t 
   if (T == 0) return 0;
   VB_CHECK(d_feats && d_ll, "null buffer");
   DeviceGuard g(h->device);
-  return score_dispatch(h, d_feats, T, stride, d_ll, ll_stride, false, static_cast<cudaStream_t>(stream));
+  return score_dispatch(h, d_feats, T, stride, d_ll, ll_stride, false, h->d_bad.as<unsigned long long>(),
+                        static_cast<cudaStream_t>(stream));
 }
 
 int vbgpu_gmm_num_cols(vbgpu_gmm_t h) { return h ? native_cols(h) : fail(VBGPU_ERR_INVALID, "null handle"); }
@@ -720,7 +724,8 @@ int vbgpu_gmm_score_cols_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int
   if (T == 0) return 0;
   VB_CHECK(d_feats && d_ll, "null buffer");
   DeviceGuard g(h->device);
-  return score_dispatch(h, d_feats, T, stride, d_ll, ll_stride, true, static_cast<cudaStream_t>(stream));
+  return score_dispatch(h, d_feats, T, stride, d_ll, ll_stride, true, h->d_bad.as<unsigned long long>(),
+                        static_cast<cudaStream_t>(stream));
 }
 
 int vbgpu_gmm_bad_count(vbgpu_gmm_t h, int64_t *count) {
@@ -753,20 +758,17 @@ int vbgpu_gmm_score(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t stride
   slab = std::min(slab, T);
   VB_TRY(h->d_feats.reserve((size_t)slab * stride * 4));
   VB_TRY(h->d_ll.reserve((size_t)slab * ll_stride * 4));
-  VB_CUDA(cudaMemsetAsync(h->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   for (int64_t t0 = 0; t0 < T; t0 += slab) {
     const int64_t n = std::min(slab, T - t0);
     VB_TRY(h2d(h->d_feats.p, feats + t0 * stride, (size_t)n * stride * 4, s));
-    VB_TRY(score_dispatch(h, h->d_feats.as<float>(), n, stride, h->d_ll.as<float>(), ll_stride, false, s));
+    VB_TRY(score_dispatch(h, h->d_feats.as<float>(), n, stride, h->d_ll.as<float>(), ll_stride, false, bad, s));
     VB_TRY(d2h(loglikes + t0 * ll_stride, h->d_ll.p, (size_t)n * ll_stride * 4, s));
     VB_CUDA(cudaStreamSynchronize(s));
   }
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpy(&bad, h->d_bad.p, 8, cudaMemcpyDeviceToHost));
-  if (bad) {
-    cudaMemset(h->d_bad.p, 0, 8);
-    return fail(VBGPU_ERR_NUMERIC, "%llu NaN/Inf log-likelihoods (overflow or invalid variances/features?)", bad);
-  }
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
   return 0;
 }
 
@@ -790,7 +792,7 @@ struct SparseReq {
 // Dense scoring in slabs of frames (device column order) + extraction of what the request names.  The slab is sized for
 // a few waves of the tensor-core kernel and at most ~2 GiB, so the footprint does not depend on T.
 static int score_sparse_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, const SparseReq &rq,
-                            cudaStream_t s) {
+                            unsigned long long *bad, cudaStream_t s) {
   if (T == 0) return 0;
   const int32_t st = (native_cols(h) + 3) / 4 * 4;
   const int64_t wave = 256LL * std::max(1, num_sms(h->device) / 2);
@@ -823,7 +825,7 @@ static int score_sparse_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int3
   int64_t prev0 = 0, prev1 = 0;
   for (int64_t t0 = 0; t0 < T; t0 += slab, k++) {
     const int64_t n = std::min(slab, T - t0);
-    VB_TRY(score_dispatch(h, d_feats + t0 * stride, n, stride, h->d_sp_slab.as<float>(), st, true, s));
+    VB_TRY(score_dispatch(h, d_feats + t0 * stride, n, stride, h->d_sp_slab.as<float>(), st, true, bad, s));
     if (rq.mode == 0)
       VB_TRY(sparse_subset_launch(h->d_sp_slab.as<float>(), st, t0, t0 + n, rq.d_f2u, rq.d_fo, rq.d_so, rq.d_cols, rq.d_oo,
                                   rq.d_out, s));
@@ -912,16 +914,6 @@ static int sparse_prepare_gather(vbgpu_gmm_t h, int64_t T, const int32_t *frames
   return 0;
 }
 
-static int check_bad(vbgpu_gmm_t h) {
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpy(&bad, h->d_bad.p, 8, cudaMemcpyDeviceToHost));
-  if (bad) {
-    cudaMemset(h->d_bad.p, 0, 8);
-    return fail(VBGPU_ERR_NUMERIC, "%llu NaN/Inf log-likelihoods (overflow or invalid variances/features?)", bad);
-  }
-  return 0;
-}
-
 int vbgpu_gmm_score_subset_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, const int64_t *frame_offsets,
                                int32_t n_utts, const int64_t *subset_offsets, const int32_t *subset_pdfs, float *d_out,
                                int64_t *out_offsets, void *stream) {
@@ -934,7 +926,7 @@ int vbgpu_gmm_score_subset_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, i
   if (total == 0) return 0;
   VB_CHECK(d_feats && d_out, "null buffer");
   rq.d_out = d_out;
-  return score_sparse_dev(h, d_feats, T, stride, rq, s);
+  return score_sparse_dev(h, d_feats, T, stride, rq, h->d_bad.as<unsigned long long>(), s);
 }
 
 int vbgpu_gmm_score_subset(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t stride, const int64_t *frame_offsets,
@@ -950,13 +942,15 @@ int vbgpu_gmm_score_subset(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t
   VB_CHECK(feats && out, "null buffer");
   VB_TRY(h->d_feats.reserve((size_t)T * stride * 4));
   VB_TRY(h->d_sp_out.reserve((size_t)total * 4));
-  VB_CUDA(cudaMemsetAsync(h->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
   rq.d_out = h->d_sp_out.as<float>();
   rq.h_out = out;  // results leave slab by slab, behind the scoring of the next slab
-  VB_TRY(score_sparse_dev(h, h->d_feats.as<float>(), T, stride, rq, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  return check_bad(h);
+  VB_TRY(score_sparse_dev(h, h->d_feats.as<float>(), T, stride, rq, bad, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
 }
 
 int vbgpu_gmm_score_gather_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *frames,
@@ -969,7 +963,7 @@ int vbgpu_gmm_score_gather_dev(vbgpu_gmm_t h, const float *d_feats, int64_t T, i
   if (n == 0) return 0;
   VB_CHECK(d_feats && d_out, "null buffer");
   rq.d_out = d_out;
-  return score_sparse_dev(h, d_feats, T, stride, rq, s);
+  return score_sparse_dev(h, d_feats, T, stride, rq, h->d_bad.as<unsigned long long>(), s);
 }
 
 int vbgpu_gmm_score_gather(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t stride, const int32_t *frames,
@@ -983,13 +977,15 @@ int vbgpu_gmm_score_gather(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t
   VB_CHECK(feats && out, "null buffer");
   VB_TRY(h->d_feats.reserve((size_t)T * stride * 4));
   VB_TRY(h->d_sp_out.reserve((size_t)n * 4));
-  VB_CUDA(cudaMemsetAsync(h->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
   rq.d_out = h->d_sp_out.as<float>();
-  VB_TRY(score_sparse_dev(h, h->d_feats.as<float>(), T, stride, rq, s));
+  VB_TRY(score_sparse_dev(h, h->d_feats.as<float>(), T, stride, rq, bad, s));
   VB_TRY(d2h(out, h->d_sp_out.p, (size_t)n * 4, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  return check_bad(h);
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
 }
 
 // ================================================================================================================
@@ -1038,7 +1034,7 @@ int vbgpu_acc_accumulate_dev(vbgpu_acc_t h, const float *d_feats, const float *d
   DeviceGuard g(h->device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   VB_TRY(h->order.enter(s));  // the counting-sort work space of the bucketed accumulation
-  VB_TRY(acc_launch(h, d_feats, d_feats2, T, stride, d_pdf_ids, d_weights, s));
+  VB_TRY(acc_launch(h, d_feats, d_feats2, T, stride, d_pdf_ids, d_weights, h->model->d_bad.as<unsigned long long>(), s));
   return h->order.leave(s);
 }
 
@@ -1069,17 +1065,19 @@ int vbgpu_acc_accumulate(vbgpu_acc_t h, const float *feats, const float *feats2,
   }
   const size_t tail = (size_t)h->model->N * (2 * h->model->D + 1);
   double before = 0.0, after = 0.0;
+  unsigned long long *bad = nullptr, n_bad = 0;
   VB_CUDA(cudaMemcpyAsync(&before, h->d_acc.as<double>() + tail, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaMemsetAsync(h->model->d_bad.p, 0, 8, s));
-  VB_TRY(acc_launch(h, h->d_feats.as<float>(), d_f2, T, stride, h->d_ids.as<int32_t>(), d_w, s));
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(acc_launch(h, h->d_feats.as<float>(), d_f2, T, stride, h->d_ids.as<int32_t>(), d_w, bad, s));
   VB_CUDA(cudaMemcpyAsync(&after, h->d_acc.as<double>() + tail, 8, cudaMemcpyDeviceToHost, s));
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpyAsync(&bad, h->model->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaStreamSynchronize(s));
+  VB_TRY(h->count.end(s, &n_bad));
   if (tot_like) *tot_like = after - before;
-  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", n_bad);
   return 0;
 }
+
+// The transition accumulators behind tot_frames in the statistics buffer.
+static double *d_trans(vbgpu_acc_t h) { return h->d_acc.as<double>() + (size_t)h->model->N * (2 * h->model->D + 1) + 2; }
 
 int vbgpu_acc_accumulate_transitions_dev(vbgpu_acc_t h, const int32_t *d_tids, int64_t T, void *stream) {
   VB_CHECK(h && T >= 0, "bad argument");
@@ -1087,8 +1085,7 @@ int vbgpu_acc_accumulate_transitions_dev(vbgpu_acc_t h, const int32_t *d_tids, i
   if (T == 0) return 0;
   VB_CHECK(d_tids, "null buffer");
   DeviceGuard g(h->device);
-  double *trans = h->d_acc.as<double>() + (size_t)h->model->N * (2 * h->model->D + 1) + 2;
-  return acc_transitions_launch(trans, h->n_trans, d_tids, T, h->model->d_bad.as<unsigned long long>(),
+  return acc_transitions_launch(d_trans(h), h->n_trans, d_tids, T, h->model->d_bad.as<unsigned long long>(),
                                 static_cast<cudaStream_t>(stream));
 }
 
@@ -1100,13 +1097,12 @@ int vbgpu_acc_accumulate_transitions(vbgpu_acc_t h, const int32_t *tids, int64_t
   DeviceGuard g(h->device);
   cudaStream_t s = h->stream;
   VB_TRY(h->d_ids.reserve((size_t)T * 4));
-  VB_CUDA(cudaMemsetAsync(h->model->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   VB_TRY(h2d(h->d_ids.p, tids, (size_t)T * 4, s));
-  VB_TRY(vbgpu_acc_accumulate_transitions_dev(h, h->d_ids.as<int32_t>(), T, s));
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpyAsync(&bad, h->model->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  if (bad) return fail(VBGPU_ERR_INVALID, "%llu transition-ids outside [1, %d]", bad, h->n_trans - 1);
+  VB_TRY(acc_transitions_launch(d_trans(h), h->n_trans, h->d_ids.as<int32_t>(), T, bad, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_INVALID, "%llu transition-ids outside [1, %d]", n_bad, h->n_trans - 1);
   return 0;
 }
 
@@ -1115,8 +1111,7 @@ int vbgpu_acc_download_transitions(vbgpu_acc_t h, double *trans_accs) {
   VB_CHECK(h->n_trans > 0, "the accumulator was created without transition accumulators");
   DeviceGuard g(h->device);
   VB_CUDA(cudaDeviceSynchronize());
-  VB_CUDA(cudaMemcpy(trans_accs, h->d_acc.as<double>() + (size_t)h->model->N * (2 * h->model->D + 1) + 2,
-                     (size_t)h->n_trans * 8, cudaMemcpyDeviceToHost));
+  VB_CUDA(cudaMemcpy(trans_accs, d_trans(h), (size_t)h->n_trans * 8, cudaMemcpyDeviceToHost));
   return 0;
 }
 
@@ -1233,7 +1228,7 @@ int vbgpu_lda_accumulate_dev(vbgpu_lda_t h, const float *d_feats, int64_t T, int
   DeviceGuard g(h->device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   VB_TRY(h->order.enter(s));  // the counting-sort work space
-  VB_TRY(lda_launch(h, d_feats, T, stride, d_class_ids, d_weights, s));
+  VB_TRY(lda_launch(h, d_feats, T, stride, d_class_ids, d_weights, h->d_bad.as<unsigned long long>(), s));
   return h->order.leave(s);
 }
 
@@ -1255,16 +1250,12 @@ int vbgpu_lda_accumulate(vbgpu_lda_t h, const float *feats, int64_t T, int32_t s
     VB_TRY(h2d(h->d_w.p, weights, (size_t)T * 4, s));
     d_w = h->d_w.as<float>();
   }
-  // this call's invalid ids only: the count of earlier _dev calls is kept for vbgpu_lda_bad_count
-  unsigned long long before = 0, after = 0;
-  VB_CUDA(cudaMemcpyAsync(&before, h->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_TRY(lda_launch(h, h->d_feats.as<float>(), T, stride, h->d_ids.as<int32_t>(), d_w, s));
-  VB_CUDA(cudaMemcpyAsync(&after, h->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  VB_CUDA(cudaMemcpy(h->d_bad.p, &before, 8, cudaMemcpyHostToDevice));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(lda_launch(h, h->d_feats.as<float>(), T, stride, h->d_ids.as<int32_t>(), d_w, bad, s));
+  VB_TRY(h->count.end(s, &n_bad));
   VB_TRY(h->order.leave(s));
-  if (after != before)
-    return fail(VBGPU_ERR_NUMERIC, "%llu frames had a class id outside [0, %d)", after - before, h->C);
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had a class id outside [0, %d)", n_bad, h->C);
   return 0;
 }
 
@@ -1528,7 +1519,8 @@ static int pipeline_score_dev(vbgpu_pipeline_t h, const int16_t *d_pcm, const in
   const int64_t T = h->mfcc->layout.total_frames;
   if (T == 0) return 0;
   VB_CHECK(d_pcm && d_loglikes, "null buffer");
-  return score_dispatch(h->gmm, feats, T, fst, d_loglikes, ll_stride, native != 0, s);
+  return score_dispatch(h->gmm, feats, T, fst, d_loglikes, ll_stride, native != 0, h->gmm->d_bad.as<unsigned long long>(),
+                        s);
 }
 
 int vbgpu_pipeline_score_dev(vbgpu_pipeline_t h, const int16_t *d_pcm, const int64_t *sample_offsets, int32_t n_utts,
@@ -1564,7 +1556,8 @@ int vbgpu_pipeline_accumulate_dev(vbgpu_pipeline_t h, vbgpu_acc_t acc, const int
                         h->d_feats.as<float>(), fst, s));
   if (T == 0) return 0;
   VB_CHECK(d_pcm && d_pdf_ids, "null buffer");
-  VB_TRY(acc_launch(acc, h->d_feats.as<float>(), nullptr, T, fst, d_pdf_ids, nullptr, s));
+  VB_TRY(acc_launch(acc, h->d_feats.as<float>(), nullptr, T, fst, d_pdf_ids, nullptr,
+                    acc->model->d_bad.as<unsigned long long>(), s));
   VB_TRY(h->order.leave(s));  // (h->d_feats is read by the accumulation kernels)
   return acc->order.leave(s);
 }
@@ -1657,7 +1650,8 @@ int vbgpu_pipeline_score_i16(vbgpu_pipeline_t h, const int16_t *pcm, const int64
     VB_TRY(h->d_ll[i].reserve(slab_bytes));
     if (!direct) VB_TRY(h->pin_ll[i].reserve(slab_bytes));
   }
-  VB_CUDA(cudaMemsetAsync(h->gmm->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   bool inflight[2] = {false, false};
   int64_t pend_t0[2] = {0, 0}, pend_n[2] = {0, 0};
   int k = 0;
@@ -1669,7 +1663,8 @@ int vbgpu_pipeline_score_i16(vbgpu_pipeline_t h, const int16_t *pcm, const int64
         std::memcpy(loglikes + pend_t0[k] * ll_stride, h->pin_ll[k].p, (size_t)pend_n[k] * ll_stride * 4);
       inflight[k] = false;
     }
-    VB_TRY(score_dispatch(h->gmm, h->d_feats.as<float>() + t0 * fst, n, fst, h->d_ll[k].as<float>(), ll_stride, false, s));
+    VB_TRY(score_dispatch(h->gmm, h->d_feats.as<float>() + t0 * fst, n, fst, h->d_ll[k].as<float>(), ll_stride, false, bad,
+                          s));
     VB_CUDA(cudaEventRecord(h->ev_ll[k], s));
     VB_CUDA(cudaStreamWaitEvent(cs, h->ev_ll[k], 0));
     void *dst = direct ? static_cast<void *>(loglikes + t0 * ll_stride) : h->pin_ll[k].p;
@@ -1686,13 +1681,8 @@ int vbgpu_pipeline_score_i16(vbgpu_pipeline_t h, const int16_t *pcm, const int64
       if (!direct) std::memcpy(loglikes + pend_t0[j] * ll_stride, h->pin_ll[j].p, (size_t)pend_n[j] * ll_stride * 4);
     }
   }
-  VB_CUDA(cudaStreamSynchronize(s));
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpy(&bad, h->gmm->d_bad.p, 8, cudaMemcpyDeviceToHost));
-  if (bad) {
-    cudaMemset(h->gmm->d_bad.p, 0, 8);
-    return fail(VBGPU_ERR_NUMERIC, "%llu NaN/Inf log-likelihoods (overflow or invalid variances/features?)", bad);
-  }
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
   return 0;
 }
 
@@ -1715,12 +1705,14 @@ int vbgpu_pipeline_score_subset_i16(vbgpu_pipeline_t h, const int16_t *pcm, cons
   if (total == 0) return 0;
   VB_CHECK(out, "null output");
   VB_TRY(h->gmm->d_sp_out.reserve((size_t)total * 4));
-  VB_CUDA(cudaMemsetAsync(h->gmm->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   rq.d_out = h->gmm->d_sp_out.as<float>();
   rq.h_out = out;  // results leave slab by slab, behind the scoring of the next slab
-  VB_TRY(score_sparse_dev(h->gmm, h->d_feats.as<float>(), T, fst, rq, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  return check_bad(h->gmm);
+  VB_TRY(score_sparse_dev(h->gmm, h->d_feats.as<float>(), T, fst, rq, bad, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
 }
 
 // PCM (host) -> one log-likelihood per lattice arc: frames[] index the packed batch (lattice-functions.cc:1214-1360).
@@ -1739,12 +1731,14 @@ int vbgpu_pipeline_score_gather_i16(vbgpu_pipeline_t h, const int16_t *pcm, cons
   if (n == 0) return 0;
   VB_CHECK(out, "null output");
   VB_TRY(h->gmm->d_sp_out.reserve((size_t)n * 4));
-  VB_CUDA(cudaMemsetAsync(h->gmm->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   rq.d_out = h->gmm->d_sp_out.as<float>();
-  VB_TRY(score_sparse_dev(h->gmm, h->d_feats.as<float>(), T, fst, rq, s));
+  VB_TRY(score_sparse_dev(h->gmm, h->d_feats.as<float>(), T, fst, rq, bad, s));
   VB_TRY(d2h(out, h->gmm->d_sp_out.p, (size_t)n * 4, s));
-  VB_CUDA(cudaStreamSynchronize(s));
-  return check_bad(h->gmm);
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
 }
 
 }  // extern "C"

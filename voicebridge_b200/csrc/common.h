@@ -203,6 +203,25 @@ struct StreamOrder {
   }
 };
 
+// The error count of one host-form call, in a slot of its own: the call neither reads nor resets the running count that
+// the _dev calls add to (vbgpu_gmm_bad_count), and errors of other calls never show up in it.  begin() zeroes the slot on
+// s and hands out its device pointer; end() copies it back and synchronises s.  Host forms run on their handle's own
+// stream and synchronise before they return, so the slot needs no StreamOrder.
+struct CallCount {
+  DevBuf slot;
+  int begin(cudaStream_t s, unsigned long long **bad) {
+    VB_TRY(slot.reserve(8));
+    VB_CUDA(cudaMemsetAsync(slot.p, 0, 8, s));
+    *bad = slot.as<unsigned long long>();
+    return 0;
+  }
+  int end(cudaStream_t s, unsigned long long *n) {
+    VB_CUDA(cudaMemcpyAsync(n, slot.p, 8, cudaMemcpyDeviceToHost, s));
+    VB_CUDA(cudaStreamSynchronize(s));
+    return 0;
+  }
+};
+
 // ---- batch layout: the utterance structure of one packed batch, mirrored on the device ------------------------
 // Cached by content: bench / training loops re-use the same layout every step and pay nothing.
 struct BatchLayout {
@@ -223,10 +242,6 @@ void launch_fill_frame2utt(const int64_t *d_frame_offsets, int32_t n_utts, int64
 }  // namespace vb
 
 // ---- handle definitions -----------------------------------------------------------------------------------------
-struct MelTable {  // one per distinct VTLN warp factor
-  float warp;
-};
-
 struct vbgpu_mfcc_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_opts opts;
@@ -241,7 +256,6 @@ struct vbgpu_mfcc_s {
   std::vector<float> warps;  // distinct VTLN factors with a table on the device (warps[0] == 1.0)
   vb::DevBuf d_window, d_tw, d_mel_off, d_mel_len, d_mel_w, d_dct, d_lifter;
   vb::DevBuf d_pcm, d_out;
-  vb::PinBuf pin_in, pin_out;
   vb::BatchLayout layout;
   uint32_t dither_seed = 0x9E3779B9u;
 };
@@ -254,7 +268,6 @@ struct vbgpu_feat_s {
   int32_t in_dim = 0, mid_dim = 0, out_dim = 0, halo = 0;
   int32_t t_rows = 0, t_cols = 0;  // global transform (lda mode)
   std::vector<float> h_delta_scales;
-  std::vector<int32_t> h_delta_lens;
   vb::DevBuf d_transform, d_delta_scales, d_norm, d_stats, d_fmllr, d_in, d_out;
   vb::BatchLayout layout;
 };
@@ -268,7 +281,8 @@ struct vbgpu_gmm_s {
   int32_t max_pdf_size = 0;
   std::vector<int32_t> h_pdf_offsets;
   vb::DevBuf d_pdf_offsets, d_gconsts, d_rows;  // d_rows: [N][2*DP] = means_invvars | -0.5*inv_vars
-  vb::DevBuf d_bad;                             // int64 counter of NaN/Inf outputs
+  vb::DevBuf d_bad;                             // uint64 running count of the _dev calls' errors (vbgpu_gmm_bad_count)
+  vb::CallCount count;                          // the host forms' own errors
   vb::DevBuf d_feats, d_ll;
   vb::DevBuf d_sp_slab, d_sp_i64, d_sp_i32, d_sp_f2u, d_sp_out;  // sparse consumers (score_sparse.cu): slab + descriptors
   vb::Stream copy_stream;  // host-facing subset calls: results of slab k leave while slab k+1 is scored
@@ -287,6 +301,7 @@ struct vbgpu_acc_s {
   vb::DevBuf d_acc;  // [occ N | mean N*D | var N*D | tot_like | tot_frames | transition accs]
   vb::DevBuf d_feats, d_feats2, d_ids, d_w;
   vb::DevBuf d_work;  // counting-sort workspace of the bucketed accumulation (accum.cu)
+  vb::CallCount count;  // the host forms' own errors (the _dev forms count into the model's running count)
   bool bucket_attr_set = false;
 };
 
@@ -297,7 +312,8 @@ struct vbgpu_lda_s {
   int32_t C = 0, D = 0;
   int64_t n_doubles = 0;  // C + C*D + D(D+1)/2
   vb::DevBuf d_acc;       // [zero C | first C*D | second D(D+1)/2, SpMatrix packing]
-  vb::DevBuf d_bad;       // uint64 count of invalid class ids since the last query
+  vb::DevBuf d_bad;       // uint64 count of invalid class ids of the _dev calls since the last query
+  vb::CallCount count;    // the host entry point's own invalid class ids
   vb::DevBuf d_work;      // counting-sort workspace
   vb::DevBuf d_feats, d_ids, d_w;  // staging of the host entry point
 };
@@ -325,8 +341,9 @@ struct vbgpu_pipeline_s {
   int device = 0;
   vb::Stream stream, copy_stream;
   vb::DevBuf d_mfcc, d_feats, d_pcm, d_ll[2], d_fmllr, d_stats;
-  vb::PinBuf pin_pcm, pin_ll[2], pin_feats;
+  vb::PinBuf pin_pcm, pin_ll[2];
   vb::Event ev_ll[2], ev_copied[2];
+  vb::CallCount count;  // the host forms' own errors (the _dev forms count into the model's running count)
 };
 
 // ---- kernel launchers (defined in the .cu files) ----------------------------------------------------------------
@@ -341,16 +358,17 @@ int feat_launch_stats(vbgpu_feat_t h, const float *d_feats, int32_t stride, doub
 int feat_launch(vbgpu_feat_t h, const float *d_in, int32_t in_stride, const float *d_fmllr, int32_t fmllr_cols,
                 float *d_out, int32_t out_stride, cudaStream_t s);
 
+// The launchers that count errors (NaN/Inf results, invalid ids) add them to *bad: the caller decides which count that is.
 int score_simt_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, float *d_ll, int32_t ll_stride,
-                      cudaStream_t s);
+                      unsigned long long *bad, cudaStream_t s);
 int acc_posterior_ab_launch(vbgpu_gmm_t g, DevBuf *work, const float *d_feats, int64_t T, int32_t stride,
                             const int32_t *d_ids, const float *d_w, float *d_ab, int32_t ab_pitch, float *d_cnt,
-                            double *d_like, int32_t *max_gauss_served, cudaStream_t s);
+                            double *d_like, int32_t *max_gauss_served, unsigned long long *bad, cudaStream_t s);
 int score_tc_prepare(vbgpu_gmm_t h, const float *gconsts, const float *miv, const float *iv, int32_t stride);
 bool score_tc_available(vbgpu_gmm_t h);
 // native != 0: d_ll in device column order ([T x ll_stride], ll_stride >= score_tc_num_cols()); 0: the model's pdf order
 int score_tc_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, float *d_ll, int32_t ll_stride,
-                    int native, cudaStream_t s);
+                    int native, unsigned long long *bad, cudaStream_t s);
 int score_tc_rescored(vbgpu_gmm_t h, int64_t *n);        // frames of the last launch re-scored in FP32
 int32_t score_tc_num_cols(vbgpu_gmm_t h);                 // P when the model is not on the tensor-core plan
 const int32_t *score_tc_col_of_pdf(vbgpu_gmm_t h);        // host [P], null = identity
@@ -380,7 +398,7 @@ int bin_sort_launch(const int32_t *d_ids, int64_t T, int32_t P, const int32_t *d
                     unsigned long long *bad, cudaStream_t s, BinSort *out);
 
 int lda_launch(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_ids, const float *d_w,
-               cudaStream_t s);
+               unsigned long long *bad, cudaStream_t s);
 
 int tree_check(const vbgpu_tree_opts *o, const vbgpu_tid_tables *t, int32_t dim, int32_t max_keys);
 int tree_init(vbgpu_tree_t h, const vbgpu_tree_opts *o, const vbgpu_tid_tables *t);  // h->D, max_keys, stream set
@@ -393,7 +411,7 @@ int tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t 
              const double *sum_x, const double *sum_x2, int64_t *dropped);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
-               const int32_t *d_ids, const float *d_w, cudaStream_t s);
+               const int32_t *d_ids, const float *d_w, unsigned long long *bad, cudaStream_t s);
 int acc_axpy(double *d_dst, const double *d_src, double scale, int64_t n, cudaStream_t s);
 int acc_transitions_launch(double *d_trans, int32_t n_trans, const int32_t *d_tids, int64_t T, unsigned long long *bad,
                            cudaStream_t s);

@@ -34,6 +34,7 @@ struct vbgpu_fmllr_s {
   int64_t per_spk = 0;  // doubles per speaker: beta | K[D][D+1] | G[D][np]
   vb::DevBuf d_stats, d_ab, d_cnt, d_units, d_pairs, d_like, d_work;
   vb::DevBuf d_feats, d_ids, d_w;  // staging of the host entry point
+  vb::CallCount count;  // the host forms' own errors (the _dev form counts into the model's running count)
   std::vector<int32_t> h_units;
 };
 
@@ -401,7 +402,8 @@ int launch_gk(vbgpu_fmllr_t h, const float *d_rows, int32_t stride, int n_units,
 }
 
 int launch_all(vbgpu_fmllr_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_ids, const float *d_w,
-               const int64_t *frame_offsets, int32_t n_utts, const int32_t *utt2spk, cudaStream_t s) {
+               const int64_t *frame_offsets, int32_t n_utts, const int32_t *utt2spk, unsigned long long *bad,
+               cudaStream_t s) {
   vbgpu_gmm_t g = h->model;
   if (T >= (int64_t)1 << 31) return vb::fail(VBGPU_ERR_INVALID, "more than 2^31 frames in one call");
   // work units: (speaker, first frame, frames <= kFChunk); adjacent utterances of one speaker form one run of frames
@@ -445,13 +447,13 @@ int launch_all(vbgpu_fmllr_t h, const float *d_feats, int64_t T, int32_t stride,
   const bool framewise = getenv("VBGPU_ACC_FRAMEWISE") != nullptr;
   if (!framewise)
     VB_TRY(vb::acc_posterior_ab_launch(g, &h->d_work, d_feats, T, stride, d_ids, d_w, h->d_ab.as<float>(), kMaxD,
-                                       h->d_cnt.as<float>(), h->d_like.as<double>(), &served, s));
+                                       h->d_cnt.as<float>(), h->d_like.as<double>(), &served, bad, s));
   if (framewise || g->max_pdf_size > served) {
     const int grid = (int)std::min<int64_t>((T + kWarps - 1) / kWarps, (int64_t)sms * 8);
     fmllr_ab_kernel<<<grid, kWarps * 32, 0, s>>>(d_feats, T, stride, g->D, g->DP, d_ids, d_w, g->d_rows.as<float>(),
                                                  g->d_gconsts.as<float>(), g->d_pdf_offsets.as<int32_t>(), g->P,
-                                                 h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(),
-                                                 g->d_bad.as<unsigned long long>(), served);
+                                                 h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(), bad,
+                                                 served);
     VB_CUDA(cudaGetLastError());
   }
   VB_TRY(launch_gk(h, d_feats, stride, n_units, s));
@@ -519,7 +521,8 @@ int vbgpu_fmllr_accumulate_dev(vbgpu_fmllr_t h, const float *d_feats, int64_t T,
   DeviceGuard g(h->device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   VB_TRY(h->order.enter(s));
-  VB_TRY(launch_all(h, d_feats, T, stride, d_pdf_ids, d_weights, frame_offsets, n_utts, utt2spk, s));
+  VB_TRY(launch_all(h, d_feats, T, stride, d_pdf_ids, d_weights, frame_offsets, n_utts, utt2spk,
+                    h->model->d_bad.as<unsigned long long>(), s));
   return h->order.leave(s);
 }
 
@@ -545,15 +548,15 @@ int vbgpu_fmllr_accumulate(vbgpu_fmllr_t h, const float *feats, int64_t T, int32
     d_w = h->d_w.as<float>();
   }
   double before = 0.0, after = 0.0;
+  unsigned long long *bad = nullptr, n_bad = 0;
   VB_CUDA(cudaMemcpyAsync(&before, h->d_like.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaMemsetAsync(h->model->d_bad.p, 0, 8, s));
-  VB_TRY(launch_all(h, h->d_feats.as<float>(), T, stride, h->d_ids.as<int32_t>(), d_w, frame_offsets, n_utts, utt2spk, s));
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(launch_all(h, h->d_feats.as<float>(), T, stride, h->d_ids.as<int32_t>(), d_w, frame_offsets, n_utts, utt2spk, bad,
+                    s));
   VB_CUDA(cudaMemcpyAsync(&after, h->d_like.p, 8, cudaMemcpyDeviceToHost, s));
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpyAsync(&bad, h->model->d_bad.p, 8, cudaMemcpyDeviceToHost, s));
-  VB_CUDA(cudaStreamSynchronize(s));
+  VB_TRY(h->count.end(s, &n_bad));
   if (tot_like) *tot_like = after - before;
-  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", n_bad);
   return 0;
 }
 
@@ -584,7 +587,8 @@ int vbgpu_mllt_accumulate(vbgpu_gmm_t model, const float *feats, int64_t T, int3
   const std::vector<int32_t> &po = model->h_pdf_offsets;
   vb::DevBuf d_xi, d_off;
   std::vector<int32_t> off;
-  VB_CUDA(cudaMemsetAsync(model->d_bad.p, 0, 8, s));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
   const int64_t kMaxFrames = 262144, kMaxRows = 1500000;
   for (int64_t t0 = 0; t0 < T;) {
     // a slab of frames whose (frame, Gaussian) rows fit the row buffers
@@ -622,7 +626,7 @@ int vbgpu_mllt_accumulate(vbgpu_gmm_t model, const float *feats, int64_t T, int3
     mllt_rows_kernel<true><<<grid, kWarps * 32, 0, s>>>(
         h->d_feats.as<float>(), n, stride, D, model->DP, h->d_ids.as<int32_t>(), d_w, model->d_rows.as<float>(),
         model->d_gconsts.as<float>(), model->d_pdf_offsets.as<int32_t>(), P, d_off.as<int32_t>(), d_xi.as<float>(),
-        h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(), model->d_bad.as<unsigned long long>(), nullptr);
+        h->d_ab.as<float>(), h->d_cnt.as<float>(), h->d_like.as<double>(), bad, nullptr);
     VB_CUDA(cudaGetLastError());
     if (R > 0) {
       std::vector<int32_t> &u = h->h_units;
@@ -643,16 +647,15 @@ int vbgpu_mllt_accumulate(vbgpu_gmm_t model, const float *feats, int64_t T, int3
   const int np1 = (D + 1) * (D + 2) / 2, np = D * (D + 1) / 2;
   std::vector<double> st((size_t)h->per_spk);
   double like = 0.0;
-  unsigned long long bad = 0;
+  VB_TRY(h->count.end(s, &n_bad));
   VB_CUDA(cudaMemcpy(st.data(), h->d_stats.p, st.size() * 8, cudaMemcpyDeviceToHost));
   VB_CUDA(cudaMemcpy(&like, h->d_like.p, 8, cudaMemcpyDeviceToHost));
-  VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
   *beta += st[0];
   const double *g = st.data() + 1 + (size_t)D * (D + 1);
   for (int i = 0; i < D; i++)
     for (int k = 0; k < np; k++) G[(size_t)i * np + k] += g[(size_t)i * np1 + k];
   if (tot_like) *tot_like += like;
-  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", n_bad);
   return 0;
 }
 
@@ -676,6 +679,8 @@ int vbgpu_gmm_component_posteriors(vbgpu_gmm_t model, const float *feats, int64_
   }
   const int64_t R = off.back();
   vb::DevBuf d_f, d_i, d_w, d_o, d_p, d_l, d_like;
+  vb::CallCount count;  // on the legacy default stream, like every copy and the launch below
+  unsigned long long *bad = nullptr, n_bad = 0;
   VB_TRY(d_f.reserve((size_t)T * stride * 4));
   VB_TRY(d_i.reserve((size_t)T * 4));
   VB_TRY(d_o.reserve((size_t)(T + 1) * 4));
@@ -687,7 +692,7 @@ int vbgpu_gmm_component_posteriors(vbgpu_gmm_t model, const float *feats, int64_
   VB_CUDA(cudaMemcpy(d_o.p, off.data(), (size_t)(T + 1) * 4, cudaMemcpyHostToDevice));
   VB_CUDA(cudaMemset(d_p.p, 0, (size_t)std::max<int64_t>(R, 1) * 4));
   VB_CUDA(cudaMemset(d_like.p, 0, 8));
-  VB_CUDA(cudaMemset(model->d_bad.p, 0, 8));
+  VB_TRY(count.begin(0, &bad));
   const float *dw = nullptr;
   if (weights) {
     VB_TRY(d_w.reserve((size_t)T * 4));
@@ -698,14 +703,12 @@ int vbgpu_gmm_component_posteriors(vbgpu_gmm_t model, const float *feats, int64_
   mllt_rows_kernel<false><<<grid, kWarps * 32>>>(d_f.as<float>(), T, stride, model->D, model->DP, d_i.as<int32_t>(), dw,
                                                  model->d_rows.as<float>(), model->d_gconsts.as<float>(),
                                                  model->d_pdf_offsets.as<int32_t>(), P, d_o.as<int32_t>(), nullptr, nullptr,
-                                                 d_p.as<float>(), d_like.as<double>(), model->d_bad.as<unsigned long long>(),
-                                                 d_l.as<float>());
+                                                 d_p.as<float>(), d_like.as<double>(), bad, d_l.as<float>());
   VB_CUDA(cudaGetLastError());
   if (R > 0) VB_CUDA(cudaMemcpy(post, d_p.p, (size_t)R * 4, cudaMemcpyDeviceToHost));
   if (loglikes) VB_CUDA(cudaMemcpy(loglikes, d_l.p, (size_t)T * 4, cudaMemcpyDeviceToHost));
-  unsigned long long bad = 0;
-  VB_CUDA(cudaMemcpy(&bad, model->d_bad.p, 8, cudaMemcpyDeviceToHost));
-  if (bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", bad);
+  VB_TRY(count.end(0, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, "%llu frames had an invalid pdf-id or a NaN/Inf likelihood", n_bad);
   return 0;
 }
 

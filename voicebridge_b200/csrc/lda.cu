@@ -176,14 +176,14 @@ __global__ void __launch_bounds__(kTriThreads) lda_tri_kernel(const float *__res
 namespace vb {
 
 int lda_launch(vbgpu_lda_t h, const float *d_feats, int64_t T, int32_t stride, const int32_t *d_ids, const float *d_w,
-               cudaStream_t s) {
+               unsigned long long *bad, cudaStream_t s) {
   if (T == 0) return 0;
   if (T >= (int64_t)1 << 31) return fail(VBGPU_ERR_INVALID, "more than 2^31 frames in one call");
   const int C = h->C, D = h->D, sms = num_sms(h->device);
   double *zero = h->d_acc.as<double>(), *first = zero + C, *second = first + (size_t)C * D;
 
   BinSort bs;
-  VB_TRY(bin_sort_launch(d_ids, T, C, nullptr, h->device, &h->d_work, h->d_bad.as<unsigned long long>(), s, &bs));
+  VB_TRY(bin_sort_launch(d_ids, T, C, nullptr, h->device, &h->d_work, bad, s, &bs));
   const int64_t max_units = (int64_t)C + T / kSortChunk + 1;
   const int g1 = (int)std::min<int64_t>(max_units, (int64_t)sms * 16);
   lda_class_kernel<<<g1, kClassThreads, 0, s>>>(d_feats, stride, D, C, d_w, bs.start, bs.unit_off, bs.order, zero, first);

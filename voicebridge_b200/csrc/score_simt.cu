@@ -100,7 +100,7 @@ __global__ void __launch_bounds__(kWarps * 32) score_simt_kernel(const float *__
 namespace vb {
 
 int score_simt_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, float *d_ll, int32_t ll_stride,
-                      cudaStream_t s) {
+                      unsigned long long *bad, cudaStream_t s) {
   if (T == 0) return 0;
   const int64_t frame_ctas = (T + kWarps * 32 - 1) / (kWarps * 32);
   // split the pdfs over grid.y so that small batches still fill the GPU (>= 2 waves of 148 SMs x 2 CTAs)
@@ -113,7 +113,6 @@ int score_simt_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t st
   ysplit = (h->P + pdfs_per_cta - 1) / pdfs_per_cta;
   if (frame_ctas > 2147483647LL) return fail(VBGPU_ERR_INVALID, "too many frames in one call");
   dim3 grid((unsigned)frame_ctas, (unsigned)ysplit);
-  unsigned long long *bad = h->d_bad.as<unsigned long long>();
   const float4 *rows = h->d_rows.as<float4>();
   const float *gc = h->d_gconsts.as<float>();
   const int32_t *po = h->d_pdf_offsets.as<int32_t>();

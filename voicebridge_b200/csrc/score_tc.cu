@@ -1331,7 +1331,7 @@ int score_tc_update_gconsts(vbgpu_gmm_t h, const float *gconsts) {
 // native == 0: d_ll is [T x ll_stride] in the model's pdf order (the kernel writes a scratch matrix, a gather kernel
 // produces d_ll).
 int score_tc_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stride, float *d_ll, int32_t ll_stride,
-                    int native, cudaStream_t s) {
+                    int native, unsigned long long *bad, cudaStream_t s) {
   TcState *st = static_cast<TcState *>(h->tc);
   if (!st) return fail(VBGPU_ERR_INVALID, "tensor-core scorer unavailable for this model");
   if (T == 0) return 0;
@@ -1403,7 +1403,7 @@ int score_tc_launch(vbgpu_gmm_t h, const float *d_feats, int64_t T, int32_t stri
   const int padded = (h->D + 3) / 4 * 4;
   p.vec_ok = (((reinterpret_cast<uintptr_t>(out) & 15) == 0 && out_stride % 4 == 0) ? 1 : 0) |
              (((reinterpret_cast<uintptr_t>(d_feats) & 15) == 0 && stride % 4 == 0 && stride >= padded) ? 2 : 0);
-  p.bad = h->d_bad.as<unsigned long long>();
+  p.bad = bad;
   p.rowflag = st->d_rowflag.as<uint8_t>();
   const char *dbg_env = getenv("VBGPU_TC_DEBUG");
   p.dbg = dbg_env ? (uint32_t)atoi(dbg_env) : 0u;
