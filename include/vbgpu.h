@@ -30,6 +30,10 @@
  *   vbgpu_tree_*      replaces  AccumulateTreeStats (tree statistics of acc-tree-stats, with SplitToPhones / IsReordered)
  *                               hmm/tree-accu.cc, hmm/hmm-utils.cc, tree/clusterable-classes.cc (callers train_deltas,
  *                               train_lda_mllt, train_sat) and the summing of the per-job treeacc files (sum-tree-stats)
+ *   vbgpu_align_*     replaces  AlignUtteranceWrapper -> FasterDecoder::Decode / GetBestPath / GetLinearSymbolSequence
+ *                               decoder/decoder-wrappers.cc, decoder/faster-decoder.cc (caller VB/src/gmmbin/
+ *                               gmm-align-compiled.cpp, the realign iterations of train_mono / train_deltas /
+ *                               train_lda_mllt / train_sat) for a batch of utterances, with its subset scoring on the device
  *   vbgpu_io_*        reads / writes  Matrix / CompressedMatrix / Vector / int32-vector objects, archive entries, model
  *                               files (-> tid2pdf + flattened AmDiagGmm) and gmm-acc-stats-ali statistics files
  *                               matrix/kaldi-matrix.cc:1375-1460, matrix/compressed-matrix.cc:531-670, gmm/diag-gmm.cc:705-756
@@ -119,6 +123,7 @@ typedef struct vbgpu_pipeline_s *vbgpu_pipeline_t;
 typedef struct vbgpu_pitch_s *vbgpu_pitch_t;
 typedef struct vbgpu_lda_s *vbgpu_lda_t;
 typedef struct vbgpu_tree_s *vbgpu_tree_t;
+typedef struct vbgpu_align_s *vbgpu_align_t;
 
 /* ---- library ------------------------------------------------------------------------------------------------ */
 int vbgpu_version(void);
@@ -440,6 +445,57 @@ int vbgpu_tree_download(vbgpu_tree_t h, int32_t *pdf_class, int32_t *phones, dou
  * whose keys differ).  Returns VBGPU_ERR_NUMERIC when some entry found no room in the key table. */
 int vbgpu_tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t *phones, const double *count,
                    const double *sum_x, const double *sum_x2);
+
+/* ---- forced alignment (gmm-align-compiled) ------------------------------------------------------------------------------
+ * Replaces AlignUtteranceWrapper -> FasterDecoder::Decode / GetBestPath / GetLinearSymbolSequence as gmm-align-compiled
+ * drives them, for a packed batch of whole utterances.
+ *   Graph: utterance u has S_u states (local ids 0 ... S_u - 1; states of the handle are packed, u owning
+ *     [state_offsets[u], state_offsets[u+1])), a start state, a final cost per state (+inf = not final) and arcs
+ *     [arc_offsets[u], arc_offsets[u+1]) of (src, dst, ilabel, weight), src / dst local.  ilabel is a transition-id in
+ *     [1, num_tids] or 0 for an epsilon arc; weight is a tropical cost.  Output labels are not needed.
+ *   Transition costs: tid_cost[num_tids + 1] (host, nullable, entry 0 unused) is added to the weight of every arc carrying
+ *     that transition-id, in float as fst::Times does: how AddTransitionProbs of the current model is applied each
+ *     iteration without re-creating the handle.  Computing it from a model stays with the caller.
+ *   Costs are FP64, as FasterDecoder's tokens keep them.  Emitting step into frame t: cost = (prev + (double)w) +
+ *     (double)ac, ac = -(acoustic_scale * ll) formed in float (one rounding), ll = the log-likelihood of pdf
+ *     tid2pdf[ilabel] at frame t.  Epsilon step: cost = prev + (double)w.  Order: the epsilon closure of the start state
+ *     before frame 0, then per frame an emitting step followed by an epsilon closure.  Result: the best over states of
+ *     cost + final.  T_u = 0 is allowed (the closure of the start state, then the final costs).
+ *   Search: exact Viterbi, no beam.  The reference searches with beam 10 and retries at 40; the two results differ only
+ *     where its beam dropped the best path, and there this result has the lower cost.
+ *   Ties: of the predecessors of a state with the same cost, the arc first in the handle's arc order wins; an epsilon
+ *     relaxation replaces a cost only if it is strictly lower; of final states with the same cost + final, the lowest
+ *     state wins.  The reference breaks exact ties in hash-list order, so equal-cost paths may be chosen differently.
+ *   Output: ali[t] the transition-id of the best path's emitting arc at every frame (rows packed like the features);
+ *     pdf_ids[t] (nullable) tid2pdf of the same arc, what vbgpu_acc_accumulate_dev takes; tot_cost[u] the graph plus
+ *     acoustic cost of the best path (what AlignUtteranceWrapper turns into its log-likelihood).  An utterance with no
+ *     final state reachable gets tot_cost = +inf, ali rows 0 and pdf_ids rows -1 (the reference's "did not successfully
+ *     decode"; the caller counts it).
+ *   Non-finite log-likelihoods add to vbgpu_gmm_bad_count for _dev calls and give VBGPU_ERR_NUMERIC from the host form.
+ * Limits, checked at create before any device work: S_u <= 4096 (two FP64 costs per state in shared memory), at most 8192
+ * distinct pdfs per utterance, no epsilon cycle, src / dst inside the utterance, ilabel in [0, num_tids], tid2pdf[1 ...
+ * num_tids] >= 0, weights and final costs neither NaN nor -inf.  At call time: tid2pdf below the model's P, n_utts the
+ * handle's.  The log-likelihoods of a call come from the model's subset scorer (vbgpu_gmm_score_subset_dev: each
+ * utterance's pdf subset is the distinct tid2pdf of its emitting arcs); like it, a call waits for its stream while it
+ * uploads the subset descriptors.  Utterances are processed in groups whose workspace ((T_u + 1) S_u traceback entries of 2
+ * or 4 bytes + T_u x subset floats) stays under a cap (default 4 GiB; one utterance above it forms a group of its own);
+ * results do not depend on the grouping.  The handle holds the graphs, not the model: create it once per training stage
+ * and align with each iteration's model. */
+int vbgpu_align_create(int32_t n_utts, const int32_t *state_offsets, const int32_t *start, const float *final_cost,
+                       const int64_t *arc_offsets, const int32_t *arc_src, const int32_t *arc_dst, const int32_t *arc_ilabel,
+                       const float *arc_weight, const int32_t *tid2pdf, int32_t num_tids, int device, vbgpu_align_t *out);
+int vbgpu_align_destroy(vbgpu_align_t h);
+/* Workspace cap of the groups in bytes (<= 0: the default). */
+int vbgpu_align_set_workspace(vbgpu_align_t h, int64_t bytes);
+/* Device form: d_feats [T x stride] on the device, frame_offsets[n_utts + 1] and tid_cost on the host; d_ali[T],
+ * d_pdf_ids[T] (nullable) and d_tot_cost[n_utts] on the device. */
+int vbgpu_align_dev(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float acoustic_scale, const float *d_feats,
+                    int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali, int32_t *d_pdf_ids,
+                    double *d_tot_cost, void *stream);
+/* Host form, synchronous: the same on host buffers. */
+int vbgpu_align(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float acoustic_scale, const float *feats,
+                int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali, int32_t *pdf_ids,
+                double *tot_cost);
 
 /* ---- Kaldi wire / disk formats on memory buffers (SURVEY.md §8f n2) ----------------------------------------------------
  * Binary forms only (what the recipes' temp files and archives hold).  Every object may carry the "\0B" marker of

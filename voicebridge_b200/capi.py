@@ -188,6 +188,11 @@ _SIGS = {
     "vbgpu_tree_num_keys": (C.c_int, [_vp, C.POINTER(_i32)]),
     "vbgpu_tree_download": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "vbgpu_tree_add": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "vbgpu_align_create": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, C.c_int, C.POINTER(_vp)]),
+    "vbgpu_align_destroy": (C.c_int, [_vp]),
+    "vbgpu_align_set_workspace": (C.c_int, [_vp, _i64]),
+    "vbgpu_align_dev": (C.c_int, [_vp, _vp, _vp, _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "vbgpu_align": (C.c_int, [_vp, _vp, _vp, _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp]),
     "vbgpu_io_object_info": (C.c_int, [_vp, _i64, C.POINTER(IoInfo)]),
     "vbgpu_io_read_matrix": (C.c_int, [_vp, _i64, _vp, _i32]),
     "vbgpu_io_read_vector": (C.c_int, [_vp, _i64, _vp]),

@@ -989,6 +989,132 @@ int vbgpu_gmm_score_gather(vbgpu_gmm_t h, const float *feats, int64_t T, int32_t
 }
 
 // ================================================================================================================
+// Forced alignment (graph layout and kernels in align.cu): subset scoring, then Viterbi + traceback, group by group
+// ================================================================================================================
+int vbgpu_align_create(int32_t n_utts, const int32_t *state_offsets, const int32_t *start, const float *final_cost,
+                       const int64_t *arc_offsets, const int32_t *arc_src, const int32_t *arc_dst, const int32_t *arc_ilabel,
+                       const float *arc_weight, const int32_t *tid2pdf, int32_t num_tids, int device, vbgpu_align_t *out) {
+  return align_create(n_utts, state_offsets, start, final_cost, arc_offsets, arc_src, arc_dst, arc_ilabel, arc_weight,
+                      tid2pdf, num_tids, device, out);
+}
+
+int vbgpu_align_destroy(vbgpu_align_t h) {
+  if (!h) return 0;
+  DeviceGuard g(h->device);
+  if (h->stream) cudaStreamSynchronize(h->stream);
+  delete h;
+  return 0;
+}
+
+int vbgpu_align_set_workspace(vbgpu_align_t h, int64_t bytes) {
+  VB_CHECK(h, "null handle");
+  h->workspace_cap = bytes > 0 ? bytes : kAlignDefaultWorkspace;
+  return 0;
+}
+
+static int check_align_args(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, int32_t stride,
+                            const int64_t *frame_offsets, int32_t n_utts) {
+  VB_CHECK(h && model && frame_offsets, "null argument");
+  VB_CHECK(n_utts == h->n_utts, "frame_offsets describe %d utterances, the graphs %d", n_utts, h->n_utts);
+  VB_CHECK(model->device == h->device, "model on device %d, graphs on device %d", model->device, h->device);
+  VB_CHECK(h->max_pdf < model->P, "tid2pdf names pdf %d, the model has %d", h->max_pdf, model->P);
+  VB_CHECK(stride >= model->D, "stride %d < dim %d", stride, model->D);
+  VB_CHECK(frame_offsets[0] == 0, "frame_offsets[0] = %lld, not 0", (long long)frame_offsets[0]);
+  for (int32_t u = 0; u < n_utts; u++)
+    VB_CHECK(frame_offsets[u + 1] >= frame_offsets[u], "frame_offsets not monotone at utterance %d", u);
+  if (tid_cost)
+    for (int32_t i = 1; i <= h->num_tids; i++)
+      VB_CHECK(!std::isnan(tid_cost[i]) && tid_cost[i] != -INFINITY, "tid_cost[%d] is NaN or -inf", i);
+  return 0;
+}
+
+// Everything behind the argument checks, on device buffers; bad receives the count of non-finite log-likelihoods.
+static int align_run(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float scale, const float *d_feats,
+                     int32_t stride, const int64_t *fo, int32_t *d_ali, int32_t *d_pdf, double *d_tot,
+                     unsigned long long *bad, cudaStream_t s) {
+  const int32_t n = h->n_utts;
+  const int64_t tbb = h->tb_bytes;
+  std::vector<AlignCall> calls((size_t)n);
+  std::vector<int32_t> group_end;  // utterance after each group
+  int64_t tb_max = 0, ll_max = 0, tb_g = 0, ll_g = 0;
+  for (int32_t u = 0; u < n; u++) {
+    const int64_t T = fo[u + 1] - fo[u], tb = (T + 1) * h->h_S[u] * tbb, ll = T * h->h_nsub[u] * 4;
+    if (u > 0 && tb_g + ll_g + tb + ll > h->workspace_cap) group_end.push_back(u), tb_g = ll_g = 0;
+    calls[u] = AlignCall{fo[u], T, ll_g / 4, tb_g / tbb};
+    tb_g += tb, ll_g += ll;
+    tb_max = std::max(tb_max, tb_g), ll_max = std::max(ll_max, ll_g);
+  }
+  group_end.push_back(n);
+  VB_TRY(h->order.enter(s));
+  VB_TRY(h->d_tb.reserve((size_t)std::max<int64_t>(tb_max, 16)));
+  VB_TRY(h->d_ll.reserve((size_t)std::max<int64_t>(ll_max, 16)));
+  VB_TRY(h2d(h->d_calls.p, calls.data(), calls.size() * sizeof(AlignCall), s));
+  VB_TRY(align_set_weights(h, tid_cost, s));
+  std::vector<int64_t> g_fo, g_so;
+  int32_t u0 = 0;
+  for (int32_t u1 : group_end) {
+    const int32_t k = u1 - u0;
+    g_fo.assign((size_t)k + 1, 0);
+    g_so.assign((size_t)k + 1, 0);
+    int32_t max_S = 1, max_sub = 0;
+    for (int32_t i = 0; i < k; i++) {
+      g_fo[i + 1] = fo[u0 + i + 1] - fo[u0];
+      g_so[i + 1] = h->h_sub_off[u0 + i + 1] - h->h_sub_off[u0];
+      max_S = std::max(max_S, h->h_S[u0 + i]);
+      max_sub = std::max(max_sub, h->h_nsub[u0 + i]);
+    }
+    const int64_t Tg = g_fo[k];
+    SparseReq rq;
+    int64_t total = 0;
+    VB_TRY(sparse_prepare_subset(model, Tg, g_fo.data(), k, g_so.data(), h->h_sub_pdfs.data() + h->h_sub_off[u0], nullptr,
+                                 &total, &rq, s));
+    if (total > 0) {
+      rq.d_out = h->d_ll.as<float>();
+      VB_TRY(score_sparse_dev(model, d_feats + fo[u0] * stride, Tg, stride, rq, bad, s));
+    }
+    VB_TRY(align_group_launch(h, u0, k, max_S, max_sub, h->d_ll.as<float>(), scale, h->d_tb.p, d_ali, d_pdf, d_tot, s));
+    u0 = u1;
+  }
+  return h->order.leave(s);
+}
+
+int vbgpu_align_dev(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float acoustic_scale, const float *d_feats,
+                    int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali, int32_t *d_pdf_ids,
+                    double *d_tot_cost, void *stream) {
+  VB_TRY(check_align_args(h, model, tid_cost, stride, frame_offsets, n_utts));
+  VB_CHECK(d_tot_cost && (frame_offsets[n_utts] == 0 || (d_feats && d_ali)), "null buffer");
+  DeviceGuard g(h->device);
+  return align_run(h, model, tid_cost, acoustic_scale, d_feats, stride, frame_offsets, d_ali, d_pdf_ids, d_tot_cost,
+                   model->d_bad.as<unsigned long long>(), static_cast<cudaStream_t>(stream));
+}
+
+int vbgpu_align(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float acoustic_scale, const float *feats,
+                int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali, int32_t *pdf_ids,
+                double *tot_cost) {
+  VB_TRY(check_align_args(h, model, tid_cost, stride, frame_offsets, n_utts));
+  const int64_t T = frame_offsets[n_utts];
+  VB_CHECK(tot_cost && (T == 0 || (feats && ali)), "null buffer");
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->stream;
+  const size_t rows = (size_t)std::max<int64_t>(T, 1);
+  VB_TRY(h->d_feats.reserve(rows * stride * 4));
+  VB_TRY(h->d_ali.reserve(rows * 4));
+  VB_TRY(h->d_pdf.reserve(rows * 4));
+  VB_TRY(h->d_tot.reserve((size_t)n_utts * 8));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
+  VB_TRY(align_run(h, model, tid_cost, acoustic_scale, h->d_feats.as<float>(), stride, frame_offsets, h->d_ali.as<int32_t>(),
+                   pdf_ids ? h->d_pdf.as<int32_t>() : nullptr, h->d_tot.as<double>(), bad, s));
+  VB_TRY(d2h(ali, h->d_ali.p, (size_t)T * 4, s));
+  if (pdf_ids) VB_TRY(d2h(pdf_ids, h->d_pdf.p, (size_t)T * 4, s));
+  VB_TRY(d2h(tot_cost, h->d_tot.p, (size_t)n_utts * 8, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
+}
+
+// ================================================================================================================
 // Accumulators
 // ================================================================================================================
 int vbgpu_acc_create(vbgpu_gmm_t model, vbgpu_acc_t *out) { return vbgpu_acc_create_with_transitions(model, 0, out); }

@@ -333,6 +333,41 @@ struct vbgpu_tree_s {
   vb::BatchLayout layout;
 };
 
+namespace vb {
+// Forced alignment (align.cu).  Graph limits: the costs of a CTA's states and its staged rows live in shared memory.
+constexpr int32_t kAlignMaxStates = 4096, kAlignMaxSubset = 8192;
+constexpr int64_t kAlignDefaultWorkspace = 4ll << 30;  // traceback entries + subset log-likelihoods of one group
+struct AlignUtt {  // per utterance, fixed at create
+  int32_t S, start, n_sub, n_lvls;
+  int32_t state_base;  // first final cost
+  int32_t csr_base;    // first of the S + 1 offsets of its emitting / epsilon incoming-arc lists
+  int32_t lvl_base;    // first of its n_lvls + 1 level offsets
+  int32_t arc_base;    // first of its arcs in the original order
+};
+struct AlignCall {  // per utterance and call
+  int64_t f0, T;    // first row of the batch, frames
+  int64_t ll_off;   // its [T x n_sub] block in the group's subset log-likelihoods
+  int64_t tb_off;   // its [(T + 1) x S] traceback entries in the group's workspace
+};
+}  // namespace vb
+
+struct vbgpu_align_s {
+  vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
+  int device = 0;
+  vb::Stream stream;
+  int32_t n_utts = 0, num_tids = 0, max_pdf = -1;
+  int64_t n_arcs = 0;
+  int32_t tb_bytes = 2;  // traceback entry: int16 when every utterance has fewer than 32768 arcs, else int32
+  int64_t workspace_cap = vb::kAlignDefaultWorkspace;
+  std::vector<int32_t> h_S, h_nsub;   // states and subset size per utterance
+  std::vector<int64_t> h_sub_off;     // pdf subsets (what the subset scorer is asked for)
+  std::vector<int32_t> h_sub_pdfs;
+  vb::DevBuf d_utts, d_eoff, d_xoff, d_arcs, d_cw, d_clab, d_lvl_off, d_lvl_states, d_final, d_asrc, d_alab, d_tid2pdf;
+  vb::DevBuf d_tid_cost, d_calls, d_best, d_ll, d_tb;  // per-call scratch
+  vb::DevBuf d_feats, d_ali, d_pdf, d_tot;             // staging of the host form
+  vb::CallCount count;                                 // the host form's own errors
+};
+
 struct vbgpu_pipeline_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_t mfcc = nullptr;
@@ -409,6 +444,15 @@ int tree_counters(vbgpu_tree_t h, int64_t *bad_utts, int64_t *dropped, int64_t *
 int tree_download(vbgpu_tree_t h, int32_t *pdf_class, int32_t *phones, double *count, double *sum_x, double *sum_x2);
 int tree_add(vbgpu_tree_t h, int32_t n, const int32_t *pdf_class, const int32_t *phones, const double *count,
              const double *sum_x, const double *sum_x2, int64_t *dropped);
+
+int align_create(int32_t n_utts, const int32_t *state_offsets, const int32_t *start, const float *final_cost,
+                 const int64_t *arc_offsets, const int32_t *arc_src, const int32_t *arc_dst, const int32_t *arc_ilabel,
+                 const float *arc_weight, const int32_t *tid2pdf, int32_t num_tids, int device, vbgpu_align_t *out);
+int align_set_weights(vbgpu_align_t h, const float *tid_cost, cudaStream_t s);  // this call's arc weights
+// Utterances [u0, u0 + n) of a group: d_ll their subset blocks, d_tb their traceback workspace (AlignCall offsets).
+int align_group_launch(vbgpu_align_t h, int32_t u0, int32_t n, int32_t max_S, int32_t max_sub, const float *d_ll,
+                       float acoustic_scale, void *d_tb, int32_t *d_ali, int32_t *d_pdf_ids, double *d_tot_cost,
+                       cudaStream_t s);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
                const int32_t *d_ids, const float *d_w, unsigned long long *bad, cudaStream_t s);

@@ -10,6 +10,7 @@ Class / method names and argument meaning follow the Kaldi types VoiceBridge lin
   AccumAmDiagGmmGpu        AccumAmDiagGmm                            gmm/mle-am-diag-gmm.h:34-108
   LdaEstimateGpu           LdaEstimate (accumulation)                transform/lda-estimate.h
   TreeStatsGpu             AccumulateTreeStats (acc-tree-stats)      hmm/tree-accu.cc
+  GmmAlignCompiledGpu      AlignUtteranceWrapper + FasterDecoder (gmm-align-compiled)   decoder/decoder-wrappers.cc
   ScoringPipeline          the fused PCM -> loglikes job (compute-mfcc-feats ... gmm-latgen-faster's decodable)
 
 Errors surface as capi.VbgpuError (the reference throws std::runtime_error from KALDI_ERR).
@@ -784,6 +785,59 @@ class TreeStatsGpu(_Handle):
             cnt[k], sx[k], sx2[k] = other_stats[ev]
         check(capi.lib().vbgpu_tree_add(self.h, n, pc.ctypes.data, ph.ctypes.data, cnt.ctypes.data, sx.ctypes.data,
                                         sx2.ctypes.data))
+
+
+class GmmAlignCompiledGpu(_Handle):
+    """gmm-align-compiled on the device: exact Viterbi over each utterance's training graph (include/vbgpu.h,
+    vbgpu_align_*).  `graphs` is a dict of packed arrays (synth.make_training_graphs builds one): state_offsets, start,
+    final_cost, arc_offsets, arc_src, arc_dst, arc_ilabel, arc_weight.  The handle holds the graphs, not the model: create
+    it once per training stage and align with each iteration's model (and its transition costs, tid_cost)."""
+    _destroy = "vbgpu_align_destroy"
+    _KEYS = (("state_offsets", np.int32), ("start", np.int32), ("final_cost", np.float32), ("arc_offsets", np.int64),
+             ("arc_src", np.int32), ("arc_dst", np.int32), ("arc_ilabel", np.int32), ("arc_weight", np.float32))
+
+    def __init__(self, graphs, tid2pdf, device=0):
+        super().__init__()
+        self._g = {k: _np(graphs[k], t) for k, t in self._KEYS}
+        self.tid2pdf = _np(tid2pdf, np.int32)
+        self.n_utts = len(self._g["start"])
+        self.device = device
+        check(capi.lib().vbgpu_align_create(self.n_utts, *(_ptr(self._g[k]) for k, _ in self._KEYS), self.tid2pdf.ctypes.data,
+                                            len(self.tid2pdf) - 1, device, C.byref(self.h)))
+
+    def set_workspace(self, nbytes):
+        """Cap of the per-group workspace in bytes (<= 0: the default)."""
+        check(capi.lib().vbgpu_align_set_workspace(self.h, int(nbytes)))
+
+    def _tc(self, tid_cost):
+        if tid_cost is None:
+            return None
+        tc = _np(tid_cost, np.float32)
+        if len(tc) != len(self.tid2pdf):
+            raise ValueError("tid_cost has %d entries, expected num_tids + 1 = %d" % (len(tc), len(self.tid2pdf)))
+        return tc
+
+    def Align(self, am, feats, frame_offsets, tid_cost=None, acoustic_scale=0.1):
+        """Host form: returns (ali[T] transition-ids, pdf_ids[T], tot_cost[n_utts]); tot_cost = +inf (ali 0, pdf -1)
+        where no final state is reachable.  Raises VbgpuError (ERR_NUMERIC) on non-finite log-likelihoods."""
+        feats = _np(feats, np.float32)
+        fo = _np(frame_offsets, np.int64)
+        tc = self._tc(tid_cost)
+        T = int(fo[-1])
+        ali, pdf, tot = np.zeros(max(T, 1), np.int32), np.zeros(max(T, 1), np.int32), np.zeros(len(fo) - 1)
+        check(capi.lib().vbgpu_align(self.h, am.h, _ptr(tc), float(acoustic_scale), feats.ctypes.data,
+                                     feats.shape[1] if feats.ndim == 2 else 0, fo.ctypes.data, len(fo) - 1,
+                                     ali.ctypes.data, pdf.ctypes.data, tot.ctypes.data))
+        return ali[:T], pdf[:T], tot
+
+    def align_dev(self, am, d_feats, stride, frame_offsets, d_ali, d_pdf_ids, d_tot_cost, tid_cost=None,
+                  acoustic_scale=0.1, stream=None):
+        """Device form: d_ali / d_pdf_ids (nullable) [T] int32, d_tot_cost [n_utts] float64 device buffers."""
+        fo = _np(frame_offsets, np.int64)
+        tc = self._tc(tid_cost)
+        check(capi.lib().vbgpu_align_dev(self.h, am.h, _ptr(tc), float(acoustic_scale), _ptr(d_feats), stride,
+                                         fo.ctypes.data, len(fo) - 1, _ptr(d_ali), _ptr(d_pdf_ids), _ptr(d_tot_cost),
+                                         _stream_ptr(stream)))
 
 
 class ScoringPipeline(_Handle):

@@ -273,3 +273,86 @@ def make_phone_alignment(n_phones, frame_offsets, seed, reordered=False, zipf=1.
         seqs.append(phones)
         tids.append(phone_alignment(topo, phones, durs, reordered))
     return topo, (np.concatenate(tids) if tids else np.zeros(0, np.int32)).astype(np.int32), seqs
+
+
+def make_training_graphs(topo, phone_seqs, num_pdfs, seed, alt_prob=0.1, self_loop_scale=0.1, max_word_phones=3):
+    """Training graphs (what compile-train-graphs makes of a transcript) for the phone sequences of make_phone_alignment,
+    over `topo` (phone_topology), packed as vbgpu_align_create takes them.  Per utterance, the phones are cut into words of
+    1 ... max_word_phones phones; the graph is
+        start -eps-> J  word  J  word ... word  J -> pre -eps-> end
+    where every J is a junction with an optional 1-state silence (phone 1): J -eps-> next, J -eps-> sil, sil -> next.  Each
+    emitting HMM state gets a self-loop and a forward arc (transition-ids of topo["tid"], costs -s log 0.75 / -s log 0.25
+    with s = self_loop_scale); with probability alt_prob a phone gets an alternative pronunciation (another 3-state phone in
+    parallel, both joining the next state), so that such states have several incoming arcs.  `end` is final with cost 0,
+    `pre` with cost 0.5.  The generating alignment (phone_alignment of the same sequence) is a path through the graph.
+    tid2pdf maps every (phone, state) tuple to a distinct pdf of a num_pdfs-pdf model (at random).
+    Returns a dict: state_offsets, start, final_cost, arc_offsets, arc_src, arc_dst, arc_ilabel, arc_weight, tid2pdf,
+    num_tids."""
+    rng = np.random.default_rng(seed)
+    tid = topo["tid"]
+    n_tuples = len(topo["tuples"])
+    pdf_of_tuple = rng.permutation(num_pdfs)[:n_tuples] if n_tuples <= num_pdfs else rng.integers(0, num_pdfs, n_tuples)
+    ts = topo["trans_state"]
+    tid2pdf = np.zeros(len(ts), np.int32)
+    tid2pdf[1:] = pdf_of_tuple[ts[1:] - 1]
+    phones = sorted(topo["phone2entry"])
+    w_self = float(np.float32(-self_loop_scale * np.log(0.75)))
+    w_fwd = float(np.float32(-self_loop_scale * np.log(0.25)))
+    w_sil = float(np.float32(-np.log(0.5)))
+    w_alt, w_main = float(np.float32(-np.log(alt_prob or 1.0))), float(np.float32(-np.log(1.0 - alt_prob)))
+    so, ao, start, finals, src, dst, lab, wt = [0], [0], [], [], [], [], [], []
+    for seq in phone_seqs:
+        fin = []
+
+        def new(final=np.inf):
+            fin.append(final)
+            return len(fin) - 1
+
+        def arc(a, b, label, w):
+            src.append(a), dst.append(b), lab.append(label), wt.append(w)
+
+        def connect(pending, s):
+            for a, label, w in pending:
+                arc(a, s, label, w)
+
+        def phone(pending, p, extra=0.0):
+            pending = [(a, label, w + extra) for a, label, w in pending]
+            for i in range(len(topo["entries"][topo["phone2entry"][p]]) - 1):
+                s = new()
+                connect(pending, s)
+                arc(s, s, tid[(p, i, True)], w_self)
+                pending = [(s, tid[(p, i, False)], w_fwd)]
+            return pending
+
+        def junction(pending):
+            j, sil = new(), new()
+            connect(pending, j)
+            arc(j, sil, 0, w_sil)
+            arc(sil, sil, tid[(1, 0, True)], w_self)
+            return [(j, 0, w_sil), (sil, tid[(1, 0, False)], w_fwd)]
+
+        s0 = new()
+        start.append(s0)
+        pending = junction([(s0, 0, 0.0)])
+        k = 0
+        while k < len(seq):
+            n = int(rng.integers(1, max_word_phones + 1))
+            for p in seq[k:k + n]:
+                if p != 1 and alt_prob > 0 and rng.random() < alt_prob:
+                    q = int(rng.choice([x for x in phones if x not in (1, p)]))
+                    pending = phone(pending, p, w_main) + phone(pending, q, w_alt)
+                else:
+                    pending = phone(pending, p)
+            pending = junction(pending)
+            k += n
+        pre = new(0.5)
+        connect(pending, pre)
+        end = new(0.0)
+        arc(pre, end, 0, 0.0)
+        finals += fin
+        so.append(len(finals))
+        ao.append(len(src))
+    return dict(state_offsets=np.asarray(so, np.int32), start=np.asarray(start, np.int32),
+                final_cost=np.asarray(finals, np.float32), arc_offsets=np.asarray(ao, np.int64),
+                arc_src=np.asarray(src, np.int32), arc_dst=np.asarray(dst, np.int32), arc_ilabel=np.asarray(lab, np.int32),
+                arc_weight=np.asarray(wt, np.float32), tid2pdf=tid2pdf, num_tids=len(tid2pdf) - 1)
