@@ -34,6 +34,8 @@
  *                               decoder/decoder-wrappers.cc, decoder/faster-decoder.cc (caller VB/src/gmmbin/
  *                               gmm-align-compiled.cpp, the realign iterations of train_mono / train_deltas /
  *                               train_lda_mllt / train_sat) for a batch of utterances, with its subset scoring on the device
+ *   vbgpu_decoder_*   replaces  FasterDecoder::Decode / ReachedFinal / GetBestPath (decoder/faster-decoder.cc, caller
+ *                               gmm-decode-faster) for a batch of utterances over one shared graph, fed by the dense scorer
  *   vbgpu_io_*        reads / writes  Matrix / CompressedMatrix / Vector / int32-vector objects, archive entries, model
  *                               files (-> tid2pdf + flattened AmDiagGmm) and gmm-acc-stats-ali statistics files
  *                               matrix/kaldi-matrix.cc:1375-1460, matrix/compressed-matrix.cc:531-670, gmm/diag-gmm.cc:705-756
@@ -496,6 +498,89 @@ int vbgpu_align_dev(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, f
 int vbgpu_align(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float acoustic_scale, const float *feats,
                 int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali, int32_t *pdf_ids,
                 double *tot_cost);
+
+/* ---- decoding (gmm-decode-faster) ----------------------------------------------------------------------------------
+ * Replaces FasterDecoder::Decode / ReachedFinal / GetBestPath (decoder/faster-decoder.cc) as gmm-decode-faster drives
+ * them: one-best search over one decoding graph (HCLG) that every utterance of a packed batch shares.  Lattices
+ * (gmm-latgen-faster) stay with the host decoder.
+ *   Graph: num_states states, a start state, a final cost per state (+inf = not final) and num_arcs arcs of (src, dst,
+ *     ilabel, olabel, weight).  ilabel is a transition-id in [1, num_tids] or 0 for an epsilon arc; olabel is a word id
+ *     (0 = none); weight is a tropical cost, negative allowed (weight pushing).  The handle holds the graph, not the model.
+ *   Costs are FP64 with align's arithmetic: emitting step cost = (prev + (double)w) + (double)ac, ac = -(acoustic_scale *
+ *     ll) formed in float (one rounding), ll the log-likelihood of pdf tid2pdf[ilabel] at frame t, read at column
+ *     col_of_pdf[pdf] of the model's device column order (vbgpu_gmm_col_of_pdf); epsilon step cost = prev + (double)w.
+ *   Search, per utterance; the token set maps states to (cost, back-pointer):
+ *     1. Start: the start state at cost 0, then its epsilon closure with no cutoff.
+ *     2. Prune, before each frame t: with c1 <= c2 <= ... the costs of the set, the cutoff is c1 + beam (in double),
+ *        lowered to c_(max_active+1) when the set holds more than max_active tokens.  A token is expanded when its cost
+ *        is below the cutoff (strict <) or equals c1.
+ *     3. Emitting step: every emitting arc out of every expanded token is relaxed into frame t's set; of equal costs
+ *        into a state, the lowest arc index wins.
+ *     4. Epsilon closure, level by level (level = the longest epsilon path into a state, as align): epsilon arcs are
+ *        relaxed only out of tokens whose cost is below (the best cost after step 3) + beam.  A relaxation replaces a
+ *        cost only when strictly lower (so the emitting back-pointer keeps an equal cost); of equal epsilon candidates
+ *        into a state, the lowest arc index wins.
+ *     5. End, after the last frame (after step 1 when T_u = 0): status[u] =
+ *          0  some token has a finite final cost: the path of the best cost + final (lowest state on ties); tot_cost
+ *             = cost + final;
+ *          1  no token has a finite final cost (gmm-decode-faster's "did not reach end-state"): the path of the best
+ *             cost (lowest state on ties); tot_cost = cost;
+ *          2  a frame's set became empty: tot_cost = +inf, ali rows 0, pdf_ids rows -1, no words;
+ *          3  a frame's set outgrew max_tokens, or more than max_active tokens tied at c1 (their records would not fit):
+ *             as 2.  A set is never silently truncated.
+ *   Output: ali[t] the transition-id of the best path's emitting arc at frame t (rows packed like the features),
+ *     pdf_ids[t] (nullable) its pdf; words[u * max_words ...] the nonzero olabels along the path in order, of emitting
+ *     and epsilon arcs alike; num_words[u] the true count, of which the first max_words are written (nothing beyond).
+ *   Differences from FasterDecoder: no adaptive beam, no on-the-fly next_weight_cutoff, no min_active, no float cutoff
+ *     arithmetic, and ties broken by the rules above, not by hash order.  With beam = +inf and max_active = INT32_MAX
+ *     the search is exact Viterbi and, wherever a final state is reachable, equals vbgpu_align on the same graph.
+ *   Non-finite log-likelihoods add to vbgpu_gmm_bad_count for _dev calls (the feature form counts what its scorer
+ *     counts, the loglikes form those of the model's P columns) and give VBGPU_ERR_NUMERIC from the host form.
+ * Checks at create, before any device work: states, start, src / dst in range, ilabel in [0, num_tids], olabel >= 0,
+ * tid2pdf[1 ... num_tids] >= 0, weights and final costs neither NaN nor -inf, no epsilon cycle.  At call time: tid2pdf
+ * below the model's P, beam > 0 (+inf allowed), 1 <= max_active, 1 <= max_tokens, ll_stride >= vbgpu_gmm_num_cols,
+ * max_words >= 0.
+ * Memory: utterance u needs 12 S + 32 max_tokens + 12 R + 4 (2 + L) R T_u bytes (R = min(max_tokens, max_active),
+ * L = the graph's largest epsilon level: the dense state map and cost keys, the token set, the survivors and their
+ * records per frame), plus 4 T_u ll_stride for the feature form's log-likelihoods.  Utterances are processed in groups
+ * whose workspace stays under a cap (default 16 GiB; one utterance above it forms a group of its own); results do not
+ * depend on the grouping.  Like align, a call uploads its descriptors on its stream without waiting for it. */
+typedef struct vbgpu_decoder_s *vbgpu_decoder_t;
+typedef struct vbgpu_decoder_opts {
+  float beam;          /* 16 (FasterDecoderOptions); > 0, +inf allowed */
+  int32_t max_active;  /* INT32_MAX; >= 1 */
+  int32_t max_tokens;  /* 65536; per-utterance capacity of one frame's token set (after the emitting step and closure).
+                          The defaults do not bound the set: on a large graph, beam 16 with unlimited max_active
+                          outgrows 65536 tokens and every utterance ends in status 3 (a 20 000-word graph does).  Set a
+                          finite max_active (the decode scripts use 7000), or max_tokens >= the graph's state count,
+                          which rules out the capacity overflow at the memory cost stated above. */
+} vbgpu_decoder_opts;
+void vbgpu_decoder_opts_default(vbgpu_decoder_opts *o);
+int vbgpu_decoder_create(int32_t num_states, int32_t start, const float *final_cost, int64_t num_arcs,
+                         const int32_t *arc_src, const int32_t *arc_dst, const int32_t *arc_ilabel,
+                         const int32_t *arc_olabel, const float *arc_weight, const int32_t *tid2pdf, int32_t num_tids,
+                         int device, vbgpu_decoder_t *out);
+int vbgpu_decoder_destroy(vbgpu_decoder_t h);
+/* Workspace cap of the groups in bytes (<= 0: the default). */
+int vbgpu_decoder_set_workspace(vbgpu_decoder_t h, int64_t bytes);
+/* Feature form: d_feats [T x stride] on the device, scored densely (vbgpu_gmm_score_cols_dev) group by group, then
+ * searched.  frame_offsets[n_utts + 1] and o on the host; d_ali[T], d_pdf_ids[T] (nullable), d_words[n_utts x
+ * max_words] (nullable when max_words = 0), d_num_words, d_tot_cost and d_status [n_utts] on the device. */
+int vbgpu_decode_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                     const float *d_feats, int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali,
+                     int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words, int32_t *d_num_words, double *d_tot_cost,
+                     int32_t *d_status, void *stream);
+/* Log-likelihood form: d_loglikes [T x ll_stride] in the model's device column order (vbgpu_gmm_score_cols_dev or
+ * vbgpu_pipeline_score_cols_dev output). */
+int vbgpu_decode_loglikes_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                              const float *d_loglikes, int32_t ll_stride, const int64_t *frame_offsets, int32_t n_utts,
+                              int32_t *d_ali, int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words,
+                              int32_t *d_num_words, double *d_tot_cost, int32_t *d_status, void *stream);
+/* Host form of vbgpu_decode_dev, synchronous: the same on host buffers. */
+int vbgpu_decode(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                 const float *feats, int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali,
+                 int32_t *pdf_ids, int32_t *words, int32_t max_words, int32_t *num_words, double *tot_cost,
+                 int32_t *status);
 
 /* ---- Kaldi wire / disk formats on memory buffers (SURVEY.md §8f n2) ----------------------------------------------------
  * Binary forms only (what the recipes' temp files and archives hold).  Every object may carry the "\0B" marker of

@@ -80,6 +80,11 @@ class TidTables(C.Structure):
                 ("flags", _vp)]
 
 
+class DecoderOpts(C.Structure):
+    """vbgpu_decoder_opts (FasterDecoderOptions' beam and max_active, decoder/faster-decoder.h, plus the token capacity)."""
+    _fields_ = [("beam", C.c_float), ("max_active", C.c_int32), ("max_tokens", C.c_int32)]
+
+
 class TreeOpts(C.Structure):
     """vbgpu_tree_opts (acc-tree-stats --context-width / --central-position / --ci-phones)."""
     _fields_ = [("context_width", C.c_int32), ("central_position", C.c_int32), ("ci_phones", _vp),
@@ -193,6 +198,16 @@ _SIGS = {
     "vbgpu_align_set_workspace": (C.c_int, [_vp, _i64]),
     "vbgpu_align_dev": (C.c_int, [_vp, _vp, _vp, _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "vbgpu_align": (C.c_int, [_vp, _vp, _vp, _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp]),
+    "vbgpu_decoder_opts_default": (None, [C.POINTER(DecoderOpts)]),
+    "vbgpu_decoder_create": (C.c_int, [_i32, _i32, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, C.c_int, C.POINTER(_vp)]),
+    "vbgpu_decoder_destroy": (C.c_int, [_vp]),
+    "vbgpu_decoder_set_workspace": (C.c_int, [_vp, _i64]),
+    "vbgpu_decode_dev": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp,
+                                   _vp, _vp, _vp]),
+    "vbgpu_decode_loglikes_dev": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp,
+                                            _i32, _vp, _vp, _vp, _vp]),
+    "vbgpu_decode": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp,
+                               _vp]),
     "vbgpu_io_object_info": (C.c_int, [_vp, _i64, C.POINTER(IoInfo)]),
     "vbgpu_io_read_matrix": (C.c_int, [_vp, _i64, _vp, _i32]),
     "vbgpu_io_read_vector": (C.c_int, [_vp, _i64, _vp]),
@@ -270,6 +285,12 @@ def default_pitch_opts(**kw):
 def default_process_pitch_opts(**kw):
     o = ProcessPitchOpts()
     lib().vbgpu_process_pitch_opts_default(C.byref(o))
+    return _with(o, kw)
+
+
+def default_decoder_opts(**kw):
+    o = DecoderOpts()
+    lib().vbgpu_decoder_opts_default(C.byref(o))
     return _with(o, kw)
 
 

@@ -1115,6 +1115,177 @@ int vbgpu_align(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float
 }
 
 // ================================================================================================================
+// Decoding (graph layout and kernels in decode.cu): dense scoring (feature form), then search + traceback, group by group
+// ================================================================================================================
+void vbgpu_decoder_opts_default(vbgpu_decoder_opts *o) {
+  if (!o) return;
+  o->beam = 16.0f;
+  o->max_active = INT32_MAX;
+  o->max_tokens = 65536;
+}
+
+int vbgpu_decoder_create(int32_t num_states, int32_t start, const float *final_cost, int64_t num_arcs,
+                         const int32_t *arc_src, const int32_t *arc_dst, const int32_t *arc_ilabel,
+                         const int32_t *arc_olabel, const float *arc_weight, const int32_t *tid2pdf, int32_t num_tids,
+                         int device, vbgpu_decoder_t *out) {
+  return decoder_create(num_states, start, final_cost, num_arcs, arc_src, arc_dst, arc_ilabel, arc_olabel, arc_weight,
+                        tid2pdf, num_tids, device, out);
+}
+
+int vbgpu_decoder_destroy(vbgpu_decoder_t h) {
+  if (!h) return 0;
+  DeviceGuard g(h->device);
+  if (h->stream) cudaStreamSynchronize(h->stream);
+  delete h;
+  return 0;
+}
+
+int vbgpu_decoder_set_workspace(vbgpu_decoder_t h, int64_t bytes) {
+  VB_CHECK(h, "null handle");
+  h->workspace_cap = bytes > 0 ? bytes : kDecodeDefaultWorkspace;
+  return 0;
+}
+
+static int check_decode_args(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o,
+                             const int64_t *frame_offsets, int32_t n_utts, int32_t max_words) {
+  VB_CHECK(h && model && o && frame_offsets, "null argument");
+  VB_CHECK(n_utts >= 0, "n_utts %d is negative", n_utts);
+  VB_CHECK(model->device == h->device, "model on device %d, graph on device %d", model->device, h->device);
+  VB_CHECK(h->max_pdf < model->P, "tid2pdf names pdf %d, the model has %d", h->max_pdf, model->P);
+  VB_CHECK(o->beam > 0.0f, "beam %g must be > 0", (double)o->beam);
+  VB_CHECK(o->max_active >= 1, "max_active %d must be >= 1", o->max_active);
+  VB_CHECK(o->max_tokens >= 1, "max_tokens %d must be >= 1", o->max_tokens);
+  VB_CHECK(max_words >= 0, "max_words %d is negative", max_words);
+  VB_CHECK(frame_offsets[0] == 0, "frame_offsets[0] = %lld, not 0", (long long)frame_offsets[0]);
+  for (int32_t u = 0; u < n_utts; u++)
+    VB_CHECK(frame_offsets[u + 1] >= frame_offsets[u], "frame_offsets not monotone at utterance %d", u);
+  return 0;
+}
+
+// Everything behind the argument checks, on device buffers.  feats: d_in is [T x in_stride] features, scored group by
+// group into the handle's scratch (bad receives the scorer's count); else d_in is the [T x in_stride] log-likelihoods
+// in device column order (bad receives their non-finite entries).
+static int decode_run(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float scale, bool feats,
+                      const float *d_in, int32_t in_stride, const int64_t *fo, int32_t n, int32_t *d_ali, int32_t *d_pdf,
+                      int32_t *d_words, int32_t max_words, int32_t *d_nw, double *d_tot, int32_t *d_status,
+                      unsigned long long *bad, cudaStream_t s) {
+  if (n == 0) return 0;
+  const int32_t cap = std::min(o->max_tokens, h->S), cap2 = std::min(cap, o->max_active);
+  const float *d_feats = feats ? d_in : nullptr, *d_ll = feats ? nullptr : d_in;
+  const int32_t stride = in_stride, ll_stride = feats ? native_cols(model) : in_stride;
+  std::vector<DecodeCall> calls((size_t)n);
+  std::vector<int32_t> group_end;
+  int64_t ws_max = 0, ll_max = 0, ws_g = 0, ll_g = 0;
+  for (int32_t u = 0; u < n; u++) {
+    const int64_t T = fo[u + 1] - fo[u], ws = (decode_ws_bytes(h->S, cap, cap2, h->n_lvls, T) + 255) & ~int64_t(255);
+    const int64_t ll = feats ? T * ll_stride * 4 : 0;
+    if (u > 0 && ws_g + ll_g + ws + ll > h->workspace_cap) group_end.push_back(u), ws_g = ll_g = 0;
+    calls[u] = DecodeCall{fo[u], T, feats ? ll_g / ((int64_t)ll_stride * 4) : fo[u], ws_g};
+    ws_g += ws, ll_g += ll;
+    ws_max = std::max(ws_max, ws_g), ll_max = std::max(ll_max, ll_g);
+  }
+  group_end.push_back(n);
+  VB_TRY(h->order.enter(s));
+  VB_TRY(h->d_ws.reserve((size_t)ws_max));
+  if (feats) VB_TRY(h->d_ll.reserve((size_t)std::max<int64_t>(ll_max, 16)));
+  VB_TRY(h->d_best.reserve((size_t)n * 4));
+  VB_TRY(h->d_calls.reserve(calls.size() * sizeof(DecodeCall)));
+  VB_TRY(h2d(h->d_calls.p, calls.data(), calls.size() * sizeof(DecodeCall), s));
+  const int32_t *cop = uses_tc(model) ? score_tc_col_of_pdf_dev(model) : nullptr;
+  VB_TRY(decoder_set_cols(h, cop, s));
+  if (!feats) VB_TRY(decoder_count_bad(d_ll, ll_stride, fo[n], cop, model->P, bad, s));
+  DecodeArgs a{};
+  a.calls = h->d_calls.as<DecodeCall>();
+  a.ws = h->d_ws.as<unsigned char>();
+  a.e_off = h->d_e_off.as<int32_t>(), a.x_off = h->d_x_off.as<int32_t>(), a.lvl = h->d_lvl.as<int32_t>();
+  a.e_arcs = h->d_e_arcs.as<int4>(), a.x_arcs = h->d_x_arcs.as<int4>();
+  a.finals = h->d_final.as<float>();
+  a.ll = feats ? h->d_ll.as<float>() : d_ll;
+  a.ll_stride = ll_stride;
+  a.scale = scale, a.beam = o->beam;
+  a.max_active = o->max_active, a.S = h->S, a.start = h->start, a.n_lvls = h->n_lvls, a.cap = cap, a.cap2 = cap2;
+  a.max_words = max_words;
+  a.best = h->d_best.as<int32_t>(), a.status = d_status, a.ali = d_ali, a.pdf_ids = d_pdf, a.words = d_words;
+  a.num_words = d_nw, a.tot_cost = d_tot;
+  int32_t u0 = 0;
+  for (int32_t u1 : group_end) {
+    if (feats && fo[u1] > fo[u0])
+      VB_TRY(score_dispatch(model, d_feats + fo[u0] * stride, fo[u1] - fo[u0], stride, h->d_ll.as<float>(), ll_stride,
+                            true, bad, s));
+    VB_TRY(decoder_search_launch(a, u0, u1 - u0, s));
+    VB_TRY(decoder_traceback_launch(h, a, u0, u1 - u0, s));
+    u0 = u1;
+  }
+  return h->order.leave(s);
+}
+
+int vbgpu_decode_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                     const float *d_feats, int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali,
+                     int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words, int32_t *d_num_words, double *d_tot_cost,
+                     int32_t *d_status, void *stream) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_CHECK(stride >= model->D, "stride %d < dim %d", stride, model->D);
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (d_num_words && d_tot_cost && d_status && (T == 0 || (d_feats && d_ali)) &&
+                           (max_words == 0 || d_words)), "null buffer");
+  DeviceGuard g(h->device);
+  return decode_run(h, model, o, acoustic_scale, true, d_feats, stride, frame_offsets, n_utts, d_ali, d_pdf_ids, d_words, max_words, d_num_words, d_tot_cost,
+                    d_status, model->d_bad.as<unsigned long long>(), static_cast<cudaStream_t>(stream));
+}
+
+int vbgpu_decode_loglikes_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                              const float *d_loglikes, int32_t ll_stride, const int64_t *frame_offsets, int32_t n_utts,
+                              int32_t *d_ali, int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words,
+                              int32_t *d_num_words, double *d_tot_cost, int32_t *d_status, void *stream) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_CHECK(ll_stride >= native_cols(model), "ll_stride %d < the model's %d columns", ll_stride, native_cols(model));
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (d_num_words && d_tot_cost && d_status && (T == 0 || (d_loglikes && d_ali)) &&
+                           (max_words == 0 || d_words)), "null buffer");
+  DeviceGuard g(h->device);
+  return decode_run(h, model, o, acoustic_scale, false, d_loglikes, ll_stride, frame_offsets, n_utts, d_ali,
+                    d_pdf_ids, d_words, max_words, d_num_words, d_tot_cost, d_status,
+                    model->d_bad.as<unsigned long long>(), static_cast<cudaStream_t>(stream));
+}
+
+int vbgpu_decode(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float acoustic_scale,
+                 const float *feats, int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali,
+                 int32_t *pdf_ids, int32_t *words, int32_t max_words, int32_t *num_words, double *tot_cost,
+                 int32_t *status) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_CHECK(stride >= model->D, "stride %d < dim %d", stride, model->D);
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (num_words && tot_cost && status && (T == 0 || (feats && ali)) && (max_words == 0 || words)),
+           "null buffer");
+  if (n_utts == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->stream;
+  const size_t rows = (size_t)std::max<int64_t>(T, 1), nw = (size_t)n_utts * max_words;
+  VB_TRY(h->d_feats.reserve(rows * stride * 4));
+  VB_TRY(h->d_ali.reserve(rows * 4));
+  VB_TRY(h->d_pdf.reserve(rows * 4));
+  VB_TRY(h->d_words.reserve(std::max<size_t>(nw, 1) * 4));
+  VB_TRY(h->d_nw.reserve((size_t)n_utts * 4));
+  VB_TRY(h->d_tot.reserve((size_t)n_utts * 8));
+  VB_TRY(h->d_status.reserve((size_t)n_utts * 4));
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
+  VB_TRY(decode_run(h, model, o, acoustic_scale, true, h->d_feats.as<float>(), stride, frame_offsets, n_utts,
+                    h->d_ali.as<int32_t>(), pdf_ids ? h->d_pdf.as<int32_t>() : nullptr, h->d_words.as<int32_t>(),
+                    max_words, h->d_nw.as<int32_t>(), h->d_tot.as<double>(), h->d_status.as<int32_t>(), bad, s));
+  VB_TRY(d2h(ali, h->d_ali.p, (size_t)T * 4, s));
+  if (pdf_ids) VB_TRY(d2h(pdf_ids, h->d_pdf.p, (size_t)T * 4, s));
+  if (nw) VB_TRY(d2h(words, h->d_words.p, nw * 4, s));
+  VB_TRY(d2h(num_words, h->d_nw.p, (size_t)n_utts * 4, s));
+  VB_TRY(d2h(tot_cost, h->d_tot.p, (size_t)n_utts * 8, s));
+  VB_TRY(d2h(status, h->d_status.p, (size_t)n_utts * 4, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
+}
+
+// ================================================================================================================
 // Accumulators
 // ================================================================================================================
 int vbgpu_acc_create(vbgpu_gmm_t model, vbgpu_acc_t *out) { return vbgpu_acc_create_with_transitions(model, 0, out); }

@@ -368,6 +368,42 @@ struct vbgpu_align_s {
   vb::CallCount count;                                 // the host form's own errors
 };
 
+namespace vb {
+// Decoding (decode.cu).  The workspace of a group: per utterance vb::decode_ws_bytes, plus the log-likelihoods of the
+// feature form.
+constexpr int64_t kDecodeDefaultWorkspace = 16ll << 30;
+struct DecodeCall {  // per utterance and call
+  int64_t f0, T;     // first row of the batch, frames
+  int64_t ll_row0;   // its first row in the log-likelihood matrix the search reads
+  int64_t ws_off;    // its workspace, in bytes from the group's
+};
+struct DecodeArgs {  // everything the search and traceback kernels read, for one group
+  const DecodeCall *calls;
+  unsigned char *ws;
+  const int32_t *e_off, *x_off, *lvl;
+  const int4 *e_arcs, *x_arcs;  // {dst, column (emitting) / -1, weight bits, original arc index}
+  const float *finals, *ll;
+  int64_t ll_stride;
+  float scale, beam;
+  int32_t max_active, S, start, n_lvls, cap, cap2, max_words;
+  int32_t *best, *status, *ali, *pdf_ids, *words, *num_words;
+  double *tot_cost;
+};
+}  // namespace vb
+
+struct vbgpu_decoder_s {
+  vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
+  int device = 0;
+  vb::Stream stream;
+  int32_t S = 0, start = 0, num_tids = 0, max_pdf = -1, n_lvls = 0;
+  int64_t n_emit = 0;  // emitting arcs
+  int64_t workspace_cap = vb::kDecodeDefaultWorkspace;
+  vb::DevBuf d_e_off, d_x_off, d_e_arcs, d_x_arcs, d_e_pdf, d_lvl, d_final, d_tid2pdf, d_ilabel, d_olabel;
+  vb::DevBuf d_calls, d_best, d_ws, d_ll;              // per-call scratch
+  vb::DevBuf d_feats, d_ali, d_pdf, d_words, d_nw, d_tot, d_status;  // staging of the host form
+  vb::CallCount count;                                 // the host form's own errors
+};
+
 struct vbgpu_pipeline_s {
   vb::StreamOrder order;  // cross-stream ordering of the handle's scratch (see StreamOrder)
   vbgpu_mfcc_t mfcc = nullptr;
@@ -453,6 +489,17 @@ int align_set_weights(vbgpu_align_t h, const float *tid_cost, cudaStream_t s);  
 int align_group_launch(vbgpu_align_t h, int32_t u0, int32_t n, int32_t max_S, int32_t max_sub, const float *d_ll,
                        float acoustic_scale, void *d_tb, int32_t *d_ali, int32_t *d_pdf_ids, double *d_tot_cost,
                        cudaStream_t s);
+
+int decoder_create(int32_t num_states, int32_t start, const float *final_cost, int64_t num_arcs, const int32_t *arc_src,
+                   const int32_t *arc_dst, const int32_t *arc_ilabel, const int32_t *arc_olabel, const float *arc_weight,
+                   const int32_t *tid2pdf, int32_t num_tids, int device, vbgpu_decoder_t *out);
+// Workspace bytes of one utterance: T frames, cap tokens per set, cap2 survivor records per frame.
+int64_t decode_ws_bytes(int32_t S, int32_t cap, int32_t cap2, int32_t n_lvls, int64_t T);
+int decoder_set_cols(vbgpu_decoder_t h, const int32_t *d_col_of_pdf, cudaStream_t s);  // null map: identity
+int decoder_count_bad(const float *d_ll, int32_t ll_stride, int64_t T, const int32_t *d_col_of_pdf, int32_t P,
+                      unsigned long long *bad, cudaStream_t s);
+int decoder_search_launch(const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s);
+int decoder_traceback_launch(vbgpu_decoder_t h, const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,
                const int32_t *d_ids, const float *d_w, unsigned long long *bad, cudaStream_t s);

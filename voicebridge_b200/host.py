@@ -11,6 +11,7 @@ Class / method names and argument meaning follow the Kaldi types VoiceBridge lin
   LdaEstimateGpu           LdaEstimate (accumulation)                transform/lda-estimate.h
   TreeStatsGpu             AccumulateTreeStats (acc-tree-stats)      hmm/tree-accu.cc
   GmmAlignCompiledGpu      AlignUtteranceWrapper + FasterDecoder (gmm-align-compiled)   decoder/decoder-wrappers.cc
+  GmmDecodeFasterGpu       FasterDecoder Decode / ReachedFinal / GetBestPath (gmm-decode-faster)  decoder/faster-decoder.cc
   ScoringPipeline          the fused PCM -> loglikes job (compute-mfcc-feats ... gmm-latgen-faster's decodable)
 
 Errors surface as capi.VbgpuError (the reference throws std::runtime_error from KALDI_ERR).
@@ -838,6 +839,70 @@ class GmmAlignCompiledGpu(_Handle):
         check(capi.lib().vbgpu_align_dev(self.h, am.h, _ptr(tc), float(acoustic_scale), _ptr(d_feats), stride,
                                          fo.ctypes.data, len(fo) - 1, _ptr(d_ali), _ptr(d_pdf_ids), _ptr(d_tot_cost),
                                          _stream_ptr(stream)))
+
+
+class GmmDecodeFasterGpu(_Handle):
+    """gmm-decode-faster on the device: one-best beam search over one decoding graph (HCLG) shared by every utterance
+    (include/vbgpu.h, vbgpu_decoder_*).  `graph` is a dict (synth.make_decoding_graph builds one): num_states, start,
+    final_cost, arc_src, arc_dst, arc_ilabel, arc_olabel, arc_weight.  The handle holds the graph, not the model.
+    Options are FasterDecoderOptions' beam and max_active, plus max_tokens (a frame's token capacity).  On a large graph
+    the defaults (beam 16, unlimited max_active) outgrow max_tokens: pass a finite max_active (the decode scripts use
+    7000) or max_tokens >= the graph's state count."""
+    _destroy = "vbgpu_decoder_destroy"
+    _KEYS = (("arc_src", np.int32), ("arc_dst", np.int32), ("arc_ilabel", np.int32), ("arc_olabel", np.int32),
+             ("arc_weight", np.float32))
+
+    def __init__(self, graph, tid2pdf, beam=16.0, max_active=2**31 - 1, max_tokens=65536, device=0):
+        super().__init__()
+        self._g = {k: _np(graph[k], t) for k, t in self._KEYS}
+        self.final_cost = _np(graph["final_cost"], np.float32)
+        self.tid2pdf = _np(tid2pdf, np.int32)
+        self.device = device
+        self.opts = capi.default_decoder_opts(beam=beam, max_active=max_active, max_tokens=max_tokens)
+        check(capi.lib().vbgpu_decoder_create(int(graph["num_states"]), int(graph["start"]), self.final_cost.ctypes.data,
+                                              len(self._g["arc_src"]), *(self._g[k].ctypes.data for k, _ in self._KEYS),
+                                              self.tid2pdf.ctypes.data, len(self.tid2pdf) - 1, device, C.byref(self.h)))
+
+    def set_workspace(self, nbytes):
+        """Cap of the per-group workspace in bytes (<= 0: the default)."""
+        check(capi.lib().vbgpu_decoder_set_workspace(self.h, int(nbytes)))
+
+    def Decode(self, am, feats, frame_offsets, acoustic_scale=0.1, max_words=64):
+        """Host form (Decode + ReachedFinal + GetBestPath per utterance): returns (ali[T] transition-ids, pdf_ids[T],
+        words per utterance (lists, at most max_words each), num_words[n_utts], tot_cost[n_utts], status[n_utts]).
+        status: 0 reached a final state, 1 did not (partial best path), 2 no token left, 3 over max_tokens.  Raises
+        VbgpuError (ERR_NUMERIC) on non-finite log-likelihoods."""
+        feats = _np(feats, np.float32)
+        fo = _np(frame_offsets, np.int64)
+        n, T = len(fo) - 1, int(fo[-1])
+        ali, pdf = np.zeros(max(T, 1), np.int32), np.zeros(max(T, 1), np.int32)
+        words, nw = np.zeros(max(n * max_words, 1), np.int32), np.zeros(max(n, 1), np.int32)
+        tot, st = np.zeros(max(n, 1)), np.zeros(max(n, 1), np.int32)
+        check(capi.lib().vbgpu_decode(self.h, am.h, C.byref(self.opts), float(acoustic_scale), feats.ctypes.data,
+                                      feats.shape[1] if feats.ndim == 2 else 0, fo.ctypes.data, n, ali.ctypes.data,
+                                      pdf.ctypes.data, words.ctypes.data, max_words, nw.ctypes.data, tot.ctypes.data,
+                                      st.ctypes.data))
+        wl = [words[u * max_words:u * max_words + min(int(nw[u]), max_words)].tolist() for u in range(n)]
+        return ali[:T], pdf[:T], wl, nw[:n], tot[:n], st[:n]
+
+    def decode_dev(self, am, d_feats, stride, frame_offsets, d_ali, d_pdf_ids, d_words, max_words, d_num_words,
+                   d_tot_cost, d_status, acoustic_scale=0.1, stream=None):
+        """Feature form on device buffers: d_ali / d_pdf_ids (nullable) [T], d_words [n_utts * max_words],
+        d_num_words / d_status [n_utts] int32, d_tot_cost [n_utts] float64."""
+        fo = _np(frame_offsets, np.int64)
+        check(capi.lib().vbgpu_decode_dev(self.h, am.h, C.byref(self.opts), float(acoustic_scale), _ptr(d_feats), stride,
+                                          fo.ctypes.data, len(fo) - 1, _ptr(d_ali), _ptr(d_pdf_ids), _ptr(d_words),
+                                          max_words, _ptr(d_num_words), _ptr(d_tot_cost), _ptr(d_status),
+                                          _stream_ptr(stream)))
+
+    def decode_loglikes_dev(self, am, d_loglikes, ll_stride, frame_offsets, d_ali, d_pdf_ids, d_words, max_words,
+                            d_num_words, d_tot_cost, d_status, acoustic_scale=0.1, stream=None):
+        """Log-likelihood form: d_loglikes [T x ll_stride] in the model's device column order."""
+        fo = _np(frame_offsets, np.int64)
+        check(capi.lib().vbgpu_decode_loglikes_dev(self.h, am.h, C.byref(self.opts), float(acoustic_scale),
+                                                   _ptr(d_loglikes), ll_stride, fo.ctypes.data, len(fo) - 1, _ptr(d_ali),
+                                                   _ptr(d_pdf_ids), _ptr(d_words), max_words, _ptr(d_num_words),
+                                                   _ptr(d_tot_cost), _ptr(d_status), _stream_ptr(stream)))
 
 
 class ScoringPipeline(_Handle):

@@ -356,3 +356,102 @@ def make_training_graphs(topo, phone_seqs, num_pdfs, seed, alt_prob=0.1, self_lo
                 final_cost=np.asarray(finals, np.float32), arc_offsets=np.asarray(ao, np.int64),
                 arc_src=np.asarray(src, np.int32), arc_dst=np.asarray(dst, np.int32), arc_ilabel=np.asarray(lab, np.int32),
                 arc_weight=np.asarray(wt, np.float32), tid2pdf=tid2pdf, num_tids=len(tid2pdf) - 1)
+
+
+def make_decoding_graph(topo, n_words, num_pdfs, seed, phones_per_word=(1, 3), n_bigram=3, eps_olabel_frac=0.2,
+                        self_loop_scale=0.1):
+    """A decoding graph (HCLG-like, what mkgraph makes of a lexicon and a bigram grammar) over `topo` (phone_topology),
+    as vbgpu_decoder_create takes it.  Word ids 1 ... n_words each get a distinct pronunciation of phones_per_word 3-state
+    phones and one HMM chain E_w -> c_1 ... c_m (the arc into c_i emits the forward transition-id of its HMM state, a
+    self-loop at c_i its self-loop transition-id).  Grammar: the backoff state G (the start state) has an epsilon arc
+    to every E_w (unigram cost) and to an optional silence (phone 1) that returns to G; the end of word w goes by
+    epsilon to its history state H_w, which has epsilon arcs to n_bigram successors' E_v and an epsilon backoff arc to
+    G whose weight may be negative.  A fraction eps_olabel_frac of the words carries its olabel on the epsilon arcs into
+    E_w, the others on their first emitting arc.  G and every H_w are final (several final states); the epsilon levels
+    are c_m 0, H_w 1, G 2, E_w 3.  tid2pdf maps every (phone, state) tuple to a distinct pdf (at random) where the
+    model has enough.  Returns a dict: num_states, start, final_cost, arc_src, arc_dst, arc_ilabel, arc_olabel,
+    arc_weight, tid2pdf, num_tids, n_words, prons."""
+    rng = np.random.default_rng(seed)
+    tid = topo["tid"]
+    n_tuples = len(topo["tuples"])
+    pdf_of_tuple = rng.permutation(num_pdfs)[:n_tuples] if n_tuples <= num_pdfs else rng.integers(0, num_pdfs, n_tuples)
+    ts = topo["trans_state"]
+    tid2pdf = np.zeros(len(ts), np.int32)
+    tid2pdf[1:] = pdf_of_tuple[ts[1:] - 1]
+    phones = [p for p in sorted(topo["phone2entry"]) if p != 1]
+    w_self = float(np.float32(-self_loop_scale * np.log(0.75)))
+    w_fwd = float(np.float32(-self_loop_scale * np.log(0.25)))
+    src, dst, ilab, olab, wt, fin = [], [], [], [], [], []
+
+    def new(final=np.inf):
+        fin.append(final)
+        return len(fin) - 1
+
+    def arc(a, b, i, o, w):
+        src.append(a), dst.append(b), ilab.append(i), olab.append(o), wt.append(float(np.float32(w)))
+
+    G = new(float(np.float32(rng.uniform(1.0, 3.0))))
+    prons, seen = [], set()
+    while len(prons) < n_words:
+        pr = tuple(int(p) for p in rng.choice(phones, int(rng.integers(phones_per_word[0], phones_per_word[1] + 1))))
+        if pr not in seen:
+            seen.add(pr)
+            prons.append(pr)
+    uni = 1.0 / np.arange(1, n_words + 1)
+    uni = -np.log(uni[rng.permutation(n_words)] / uni.sum())
+    eps_ol = rng.random(n_words) < eps_olabel_frac
+    entry, hist = [], []
+    for k, pr in enumerate(prons):
+        w = k + 1
+        E = new()
+        entry.append(E)
+        prev, first = E, True
+        for p in pr:
+            for j in range(len(topo["entries"][topo["phone2entry"][p]]) - 1):
+                c = new()
+                arc(prev, c, tid[(p, j, False)], w if first and not eps_ol[k] else 0, w_fwd)
+                arc(c, c, tid[(p, j, True)], 0, w_self)
+                prev, first = c, False
+        H = new(float(np.float32(rng.uniform(0.5, 4.0))))
+        hist.append(H)
+        arc(prev, H, 0, 0, 0.0)
+    for k in range(n_words):
+        arc(G, entry[k], 0, k + 1 if eps_ol[k] else 0, uni[k])
+    for k in range(n_words):
+        for v in rng.choice(n_words, min(n_bigram, n_words), replace=False):
+            arc(hist[k], entry[v], 0, int(v) + 1 if eps_ol[v] else 0, rng.uniform(0.2, 2.0))
+        arc(hist[k], G, 0, 0, rng.uniform(-0.5, 1.0))
+    SE = new()
+    arc(G, SE, 0, 0, -np.log(0.3))
+    s1 = new()
+    arc(SE, s1, tid[(1, 0, False)], 0, w_fwd)
+    arc(s1, s1, tid[(1, 0, True)], 0, w_self)
+    arc(s1, G, 0, 0, 0.0)
+    return dict(num_states=len(fin), start=G, final_cost=np.asarray(fin, np.float32), arc_src=np.asarray(src, np.int32),
+                arc_dst=np.asarray(dst, np.int32), arc_ilabel=np.asarray(ilab, np.int32),
+                arc_olabel=np.asarray(olab, np.int32), arc_weight=np.asarray(wt, np.float32), tid2pdf=tid2pdf,
+                num_tids=len(tid2pdf) - 1, n_words=n_words, prons=prons)
+
+
+def sample_decoding_path(graph, seed, min_frames, self_loop_prob=0.5):
+    """A random path of a decoding graph from the start state to a final state with at least min_frames emitting arcs:
+    at each state a self-loop is taken with probability self_loop_prob (when there is one), else one of the other
+    outgoing arcs uniformly; the walk stops at the first final state once min_frames frames are emitted.  Returns
+    (words: the nonzero olabels along the path, tids[T]: its transition-ids, arcs: the arc indices of the path)."""
+    rng = np.random.default_rng(seed)
+    S = int(graph["num_states"])
+    src, dst = np.asarray(graph["arc_src"]), np.asarray(graph["arc_dst"])
+    lab, ol = np.asarray(graph["arc_ilabel"]), np.asarray(graph["arc_olabel"])
+    order = np.argsort(src, kind="stable")
+    off = np.searchsorted(src[order], np.arange(S + 1))
+    s, arcs, T = int(graph["start"]), [], 0
+    while not (T >= min_frames and graph["final_cost"][s] < np.inf):
+        out = order[off[s]:off[s + 1]]
+        loops = [a for a in out if dst[a] == s]
+        other = [a for a in out if dst[a] != s]
+        a = int(loops[0]) if loops and (not other or rng.random() < self_loop_prob) else int(rng.choice(other))
+        arcs.append(a)
+        T += lab[a] > 0
+        s = int(dst[a])
+    arcs = np.asarray(arcs, np.int64)
+    return ([int(o) for o in ol[arcs] if o], lab[arcs][lab[arcs] > 0].astype(np.int32), arcs)
