@@ -501,8 +501,9 @@ int vbgpu_align(vbgpu_align_t h, vbgpu_gmm_t model, const float *tid_cost, float
 
 /* ---- decoding (gmm-decode-faster) ----------------------------------------------------------------------------------
  * Replaces FasterDecoder::Decode / ReachedFinal / GetBestPath (decoder/faster-decoder.cc) as gmm-decode-faster drives
- * them: one-best search over one decoding graph (HCLG) that every utterance of a packed batch shares.  Lattices
- * (gmm-latgen-faster) stay with the host decoder.
+ * them: one-best search over one decoding graph (HCLG) that every utterance of a packed batch shares.  The same handle
+ * generates raw state-level lattices (gmm-latgen-faster; vbgpu_decode_lattice*, below); determinising them stays on the
+ * host.
  *   Graph: num_states states, a start state, a final cost per state (+inf = not final) and num_arcs arcs of (src, dst,
  *     ilabel, olabel, weight).  ilabel is a transition-id in [1, num_tids] or 0 for an epsilon arc; olabel is a word id
  *     (0 = none); weight is a tropical cost, negative allowed (weight pushing).  The handle holds the graph, not the model.
@@ -581,6 +582,84 @@ int vbgpu_decode(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts 
                  const float *feats, int32_t stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *ali,
                  int32_t *pdf_ids, int32_t *words, int32_t max_words, int32_t *num_words, double *tot_cost,
                  int32_t *status);
+
+/* ---- lattice generation (gmm-latgen-faster) ------------------------------------------------------------------------
+ * Replaces LatticeFasterDecoder::Decode / GetRawLattice (decoder/lattice-faster-decoder.cc) as gmm-latgen-faster drives
+ * them, up to the raw state-level lattice that DeterminizeLatticePhonePrunedWrapper takes; determinisation and
+ * everything after it stay on the host.  The handle, graph and options are vbgpu_decoder_*'s.
+ *   Search: exactly vbgpu_decode's (prune rule, cost arithmetic, epsilon levels, tie rules, statuses 0-3).  ali,
+ *     pdf_ids, words, num_words, tot_cost and status are bit-identical to vbgpu_decode_* on the same input and options.
+ *   Tokens: frame 0 is the start closure (step 1); frame f+1 is the set after the emitting step of frame f and its
+ *     closure (steps 3-4).  Token cost alpha is the search's FP64 cost.
+ *   Links: every emitting relaxation out of an expanded token with a finite candidate, won or not (graph cost the arc
+ *     weight, acoustic cost ac in float), and every epsilon relaxation out of a closure source (acoustic cost 0).
+ *   Exact final prune (PruneForwardLinksFinal / PruneForwardLinks in one pass, FP64, the search's operation order):
+ *     last-frame tokens start at extra = (alpha + final) - tot_cost under status 0 (+inf when not final), alpha -
+ *     tot_cost under status 1 (every end token final with cost 0, as LatticeFasterDecoder); an extra above
+ *     lattice_beam becomes +inf.  Then frames T ... 0, within a frame the epsilon levels from the highest down (epsilon
+ *     arcs go to higher levels, so one pass is exact): link_extra = dst.extra + (((src.alpha + w) + ac) - dst.alpha),
+ *     for an epsilon link dst.extra + ((src.alpha + w) - dst.alpha).  A link is kept iff link_extra is finite and <= lattice_beam; a
+ *     token's extra is the minimum of its own (last frame) and its kept links'; it is kept iff that is finite.  Every
+ *     link of the best path has link_extra exactly 0.
+ *   A token that the next frame's prune does not expand stays when it has an epsilon path to one that is expanded
+ *     (negative epsilon weights with a small max_active), as in LatticeFasterDecoder.
+ *   Output per utterance u, states at u * max_states, arcs at u * max_arcs: states in (frame, epsilon level, graph
+ *     state) order, the start token state 0 (a topological order); per state its frame, graph state and the graph part
+ *     of its final weight: the final cost (last frame, status 0), 0 (last frame, status 1), else +inf.  Arcs in (source
+ *     state, original arc index) order, each with src, dst, ilabel (a transition-id, 0 = epsilon), olabel, graph cost
+ *     and acoustic cost as float (LatticeWeight's two values).  num_states / num_arcs are the true counts.
+ *     Decoder status 2 or 3: an empty lattice.  lattice_status[u] =
+ *       0  written;
+ *       1  the lattice store overflowed (arena_tokens / arena_links): no lattice (counts 0);
+ *       2  the pruned lattice exceeds max_states or max_arcs: the true counts, contents unspecified; retry with them.
+ *     Under 1 and 2 the one-best outputs are still valid.
+ *   Differences from LatticeFasterDecoder: those of vbgpu_decode; no periodic pruning (prune_interval: it is
+ *     conservative and does not change the final lattice, so leaving it out costs store memory only); no
+ *     determinisation.  The output numbering ranks the kept tokens of each frame against each other: O(n_f^2) work for
+ *     n_f of them, cheap at the usual lattice beams.
+ * Checks at call time besides vbgpu_decode's: lattice_beam >= 0 (+inf allowed, not NaN), 1 <= arena_tokens, 1 <=
+ * arena_links, (T_u + 1) x arena_tokens and (T_u + 1) x arena_links below 2^31, max_states >= 0, max_arcs >= 0, output
+ * arrays non-null.  Memory: on top of vbgpu_decode's workspace, utterance u's lattice store takes 48 NT + 20 NL + 4 R'
+ * + 4 R + 8 (T_u + 2) bytes (NT = (T_u + 1) arena_tokens, NL = (T_u + 1) arena_links, R' = min(max_tokens, S), R as
+ * above), inside the same workspace cap; results do not depend on the grouping.  The store keeps, per frame, the
+ * tokens that survive the next prune (and their epsilon ancestors) and the links between them, plus the unpruned links
+ * of the frame being searched. */
+typedef struct vbgpu_lattice_opts {
+  float lattice_beam;    /* 10 (LatticeFasterDecoderConfig); >= 0, +inf allowed */
+  int32_t max_states;    /* 131072: per-utterance output capacity in states ... */
+  int32_t max_arcs;      /* 524288: ... and in arcs */
+  int32_t arena_tokens;  /* 8192: tokens the lattice store holds per frame of an utterance, on average */
+  int32_t arena_links;   /* 24576: links likewise */
+} vbgpu_lattice_opts;
+void vbgpu_lattice_opts_default(vbgpu_lattice_opts *o);
+/* Output arrays, on the device (host arrays for vbgpu_decode_lattice).  States [n_utts x max_states], arcs [n_utts x
+ * max_arcs], counts and status [n_utts]; arena_peak (nullable) [n_utts x 2]: tokens and links the store held at most. */
+typedef struct vbgpu_lattice_out {
+  int32_t *state_frame, *state_graph;
+  float *state_final;
+  int32_t *arc_src, *arc_dst, *arc_ilabel, *arc_olabel;
+  float *arc_graph_cost, *arc_ac_cost;
+  int32_t *num_states, *num_arcs, *lattice_status;
+  int32_t *arena_peak;
+} vbgpu_lattice_out;
+/* Feature form: as vbgpu_decode_dev, plus the lattice (out's arrays on the device). */
+int vbgpu_decode_lattice_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o,
+                             const vbgpu_lattice_opts *lo, float acoustic_scale, const float *d_feats, int32_t stride,
+                             const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali, int32_t *d_pdf_ids,
+                             int32_t *d_words, int32_t max_words, int32_t *d_num_words, double *d_tot_cost,
+                             int32_t *d_status, const vbgpu_lattice_out *out, void *stream);
+/* Log-likelihood form: as vbgpu_decode_loglikes_dev (PCM -> lattice stays on the device), plus the lattice. */
+int vbgpu_decode_lattice_loglikes_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o,
+                                      const vbgpu_lattice_opts *lo, float acoustic_scale, const float *d_loglikes,
+                                      int32_t ll_stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali,
+                                      int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words, int32_t *d_num_words,
+                                      double *d_tot_cost, int32_t *d_status, const vbgpu_lattice_out *out,
+                                      void *stream);
+/* Host form of vbgpu_decode_lattice_dev, synchronous: the same on host buffers (VBGPU_ERR_NUMERIC as vbgpu_decode). */
+int vbgpu_decode_lattice(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, const vbgpu_lattice_opts *lo,
+                         float acoustic_scale, const float *feats, int32_t stride, const int64_t *frame_offsets,
+                         int32_t n_utts, int32_t *ali, int32_t *pdf_ids, int32_t *words, int32_t max_words,
+                         int32_t *num_words, double *tot_cost, int32_t *status, const vbgpu_lattice_out *out);
 
 /* ---- Kaldi wire / disk formats on memory buffers (SURVEY.md §8f n2) ----------------------------------------------------
  * Binary forms only (what the recipes' temp files and archives hold).  Every object may carry the "\0B" marker of

@@ -85,6 +85,20 @@ class DecoderOpts(C.Structure):
     _fields_ = [("beam", C.c_float), ("max_active", C.c_int32), ("max_tokens", C.c_int32)]
 
 
+class LatticeOpts(C.Structure):
+    """vbgpu_lattice_opts (LatticeFasterDecoderConfig's lattice_beam, plus output capacities and the lattice store's
+    size per frame)."""
+    _fields_ = [("lattice_beam", C.c_float), ("max_states", C.c_int32), ("max_arcs", C.c_int32),
+                ("arena_tokens", C.c_int32), ("arena_links", C.c_int32)]
+
+
+class LatticeOut(C.Structure):
+    """vbgpu_lattice_out: the lattice arrays of a call (pointers)."""
+    _fields_ = [(k, _vp) for k in ("state_frame", "state_graph", "state_final", "arc_src", "arc_dst", "arc_ilabel",
+                                   "arc_olabel", "arc_graph_cost", "arc_ac_cost", "num_states", "num_arcs",
+                                   "lattice_status", "arena_peak")]
+
+
 class TreeOpts(C.Structure):
     """vbgpu_tree_opts (acc-tree-stats --context-width / --central-position / --ci-phones)."""
     _fields_ = [("context_width", C.c_int32), ("central_position", C.c_int32), ("ci_phones", _vp),
@@ -208,6 +222,14 @@ _SIGS = {
                                             _i32, _vp, _vp, _vp, _vp]),
     "vbgpu_decode": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), _f, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp,
                                _vp]),
+    "vbgpu_lattice_opts_default": (None, [C.POINTER(LatticeOpts)]),
+    "vbgpu_decode_lattice_dev": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), C.POINTER(LatticeOpts), _f, _vp, _i32, _vp,
+                                           _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(LatticeOut), _vp]),
+    "vbgpu_decode_lattice_loglikes_dev": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), C.POINTER(LatticeOpts), _f, _vp,
+                                                    _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp,
+                                                    C.POINTER(LatticeOut), _vp]),
+    "vbgpu_decode_lattice": (C.c_int, [_vp, _vp, C.POINTER(DecoderOpts), C.POINTER(LatticeOpts), _f, _vp, _i32, _vp,
+                                       _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(LatticeOut)]),
     "vbgpu_io_object_info": (C.c_int, [_vp, _i64, C.POINTER(IoInfo)]),
     "vbgpu_io_read_matrix": (C.c_int, [_vp, _i64, _vp, _i32]),
     "vbgpu_io_read_vector": (C.c_int, [_vp, _i64, _vp]),
@@ -291,6 +313,12 @@ def default_process_pitch_opts(**kw):
 def default_decoder_opts(**kw):
     o = DecoderOpts()
     lib().vbgpu_decoder_opts_default(C.byref(o))
+    return _with(o, kw)
+
+
+def default_lattice_opts(**kw):
+    o = LatticeOpts()
+    lib().vbgpu_lattice_opts_default(C.byref(o))
     return _with(o, kw)
 
 

@@ -1165,10 +1165,12 @@ static int check_decode_args(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_d
 // Everything behind the argument checks, on device buffers.  feats: d_in is [T x in_stride] features, scored group by
 // group into the handle's scratch (bad receives the scorer's count); else d_in is the [T x in_stride] log-likelihoods
 // in device column order (bad receives their non-finite entries).
+// lo / lat (both or neither): the lattice form, whose lattice store each utterance's workspace also holds.
 static int decode_run(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, float scale, bool feats,
                       const float *d_in, int32_t in_stride, const int64_t *fo, int32_t n, int32_t *d_ali, int32_t *d_pdf,
                       int32_t *d_words, int32_t max_words, int32_t *d_nw, double *d_tot, int32_t *d_status,
-                      unsigned long long *bad, cudaStream_t s) {
+                      unsigned long long *bad, cudaStream_t s, const vbgpu_lattice_opts *lo = nullptr,
+                      const vbgpu_lattice_out *lat = nullptr) {
   if (n == 0) return 0;
   const int32_t cap = std::min(o->max_tokens, h->S), cap2 = std::min(cap, o->max_active);
   const float *d_feats = feats ? d_in : nullptr, *d_ll = feats ? nullptr : d_in;
@@ -1177,10 +1179,12 @@ static int decode_run(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_
   std::vector<int32_t> group_end;
   int64_t ws_max = 0, ll_max = 0, ws_g = 0, ll_g = 0;
   for (int32_t u = 0; u < n; u++) {
-    const int64_t T = fo[u + 1] - fo[u], ws = (decode_ws_bytes(h->S, cap, cap2, h->n_lvls, T) + 255) & ~int64_t(255);
+    const int64_t T = fo[u + 1] - fo[u], ws1 = (decode_ws_bytes(h->S, cap, cap2, h->n_lvls, T) + 255) & ~int64_t(255);
+    const int32_t NT = lo ? (int32_t)((T + 1) * lo->arena_tokens) : 0, NL = lo ? (int32_t)((T + 1) * lo->arena_links) : 0;
+    const int64_t ws = ws1 + (lo ? (lattice_arena_bytes(NT, NL, cap, cap2, T) + 255) & ~int64_t(255) : 0);
     const int64_t ll = feats ? T * ll_stride * 4 : 0;
     if (u > 0 && ws_g + ll_g + ws + ll > h->workspace_cap) group_end.push_back(u), ws_g = ll_g = 0;
-    calls[u] = DecodeCall{fo[u], T, feats ? ll_g / ((int64_t)ll_stride * 4) : fo[u], ws_g};
+    calls[u] = DecodeCall{fo[u], T, feats ? ll_g / ((int64_t)ll_stride * 4) : fo[u], ws_g, ws_g + ws1, NT, NL};
     ws_g += ws, ll_g += ll;
     ws_max = std::max(ws_max, ws_g), ll_max = std::max(ll_max, ll_g);
   }
@@ -1207,13 +1211,19 @@ static int decode_run(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_
   a.max_words = max_words;
   a.best = h->d_best.as<int32_t>(), a.status = d_status, a.ali = d_ali, a.pdf_ids = d_pdf, a.words = d_words;
   a.num_words = d_nw, a.tot_cost = d_tot;
+  if (lo) {
+    a.lattice_beam = lo->lattice_beam, a.max_states = lo->max_states, a.max_arcs = lo->max_arcs;
+    a.ilabel = h->d_ilabel.as<int32_t>(), a.olabel = h->d_olabel.as<int32_t>(), a.weight = h->d_weight.as<float>();
+    a.lat = *lat;
+  }
   int32_t u0 = 0;
   for (int32_t u1 : group_end) {
     if (feats && fo[u1] > fo[u0])
       VB_TRY(score_dispatch(model, d_feats + fo[u0] * stride, fo[u1] - fo[u0], stride, h->d_ll.as<float>(), ll_stride,
                             true, bad, s));
-    VB_TRY(decoder_search_launch(a, u0, u1 - u0, s));
+    VB_TRY(decoder_search_launch(a, u0, u1 - u0, lo != nullptr, s));
     VB_TRY(decoder_traceback_launch(h, a, u0, u1 - u0, s));
+    if (lo) VB_TRY(decoder_lattice_launch(a, u0, u1 - u0, s));
     u0 = u1;
   }
   return h->order.leave(s);
@@ -1280,6 +1290,132 @@ int vbgpu_decode(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts 
   VB_TRY(d2h(num_words, h->d_nw.p, (size_t)n_utts * 4, s));
   VB_TRY(d2h(tot_cost, h->d_tot.p, (size_t)n_utts * 8, s));
   VB_TRY(d2h(status, h->d_status.p, (size_t)n_utts * 4, s));
+  VB_TRY(h->count.end(s, &n_bad));
+  if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
+  return 0;
+}
+
+// Lattice generation: decode_run's lattice form (store and kernels in decode.cu)
+void vbgpu_lattice_opts_default(vbgpu_lattice_opts *o) {
+  if (!o) return;
+  o->lattice_beam = 10.0f;
+  o->max_states = 131072;
+  o->max_arcs = 524288;
+  o->arena_tokens = 8192;
+  o->arena_links = 24576;
+}
+
+static int check_lattice_args(const vbgpu_lattice_opts *lo, const vbgpu_lattice_out *out, const int64_t *fo,
+                              int32_t n_utts) {
+  VB_CHECK(lo && out, "null argument");
+  VB_CHECK(lo->lattice_beam >= 0.0f, "lattice_beam %g must be >= 0", (double)lo->lattice_beam);
+  VB_CHECK(lo->max_states >= 0 && lo->max_arcs >= 0, "max_states %d / max_arcs %d is negative", lo->max_states,
+           lo->max_arcs);
+  VB_CHECK(lo->arena_tokens >= 1 && lo->arena_links >= 1, "arena_tokens %d / arena_links %d must be >= 1",
+           lo->arena_tokens, lo->arena_links);
+  for (int32_t u = 0; u < n_utts; u++) {
+    const int64_t T1 = fo[u + 1] - fo[u] + 1;
+    VB_CHECK(T1 * lo->arena_tokens < (1ll << 31) && T1 * lo->arena_links < (1ll << 31),
+             "utterance %d: (T + 1) x arena_tokens / arena_links reaches 2^31", u);
+  }
+  VB_CHECK(n_utts == 0 || (out->num_states && out->num_arcs && out->lattice_status), "null lattice buffer");
+  VB_CHECK(n_utts == 0 || lo->max_states == 0 || (out->state_frame && out->state_graph && out->state_final),
+           "null lattice state buffer");
+  VB_CHECK(n_utts == 0 || lo->max_arcs == 0 || (out->arc_src && out->arc_dst && out->arc_ilabel && out->arc_olabel &&
+                                                out->arc_graph_cost && out->arc_ac_cost),
+           "null lattice arc buffer");
+  return 0;
+}
+
+int vbgpu_decode_lattice_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o,
+                             const vbgpu_lattice_opts *lo, float acoustic_scale, const float *d_feats, int32_t stride,
+                             const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali, int32_t *d_pdf_ids,
+                             int32_t *d_words, int32_t max_words, int32_t *d_num_words, double *d_tot_cost,
+                             int32_t *d_status, const vbgpu_lattice_out *out, void *stream) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_TRY(check_lattice_args(lo, out, frame_offsets, n_utts));
+  VB_CHECK(stride >= model->D, "stride %d < dim %d", stride, model->D);
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (d_num_words && d_tot_cost && d_status && (T == 0 || (d_feats && d_ali)) &&
+                           (max_words == 0 || d_words)), "null buffer");
+  DeviceGuard g(h->device);
+  return decode_run(h, model, o, acoustic_scale, true, d_feats, stride, frame_offsets, n_utts, d_ali, d_pdf_ids,
+                    d_words, max_words, d_num_words, d_tot_cost, d_status, model->d_bad.as<unsigned long long>(),
+                    static_cast<cudaStream_t>(stream), lo, out);
+}
+
+int vbgpu_decode_lattice_loglikes_dev(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o,
+                                      const vbgpu_lattice_opts *lo, float acoustic_scale, const float *d_loglikes,
+                                      int32_t ll_stride, const int64_t *frame_offsets, int32_t n_utts, int32_t *d_ali,
+                                      int32_t *d_pdf_ids, int32_t *d_words, int32_t max_words, int32_t *d_num_words,
+                                      double *d_tot_cost, int32_t *d_status, const vbgpu_lattice_out *out,
+                                      void *stream) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_TRY(check_lattice_args(lo, out, frame_offsets, n_utts));
+  VB_CHECK(ll_stride >= native_cols(model), "ll_stride %d < the model's %d columns", ll_stride, native_cols(model));
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (d_num_words && d_tot_cost && d_status && (T == 0 || (d_loglikes && d_ali)) &&
+                           (max_words == 0 || d_words)), "null buffer");
+  DeviceGuard g(h->device);
+  return decode_run(h, model, o, acoustic_scale, false, d_loglikes, ll_stride, frame_offsets, n_utts, d_ali,
+                    d_pdf_ids, d_words, max_words, d_num_words, d_tot_cost, d_status,
+                    model->d_bad.as<unsigned long long>(), static_cast<cudaStream_t>(stream), lo, out);
+}
+
+int vbgpu_decode_lattice(vbgpu_decoder_t h, vbgpu_gmm_t model, const vbgpu_decoder_opts *o, const vbgpu_lattice_opts *lo,
+                         float acoustic_scale, const float *feats, int32_t stride, const int64_t *frame_offsets,
+                         int32_t n_utts, int32_t *ali, int32_t *pdf_ids, int32_t *words, int32_t max_words,
+                         int32_t *num_words, double *tot_cost, int32_t *status, const vbgpu_lattice_out *out) {
+  VB_TRY(check_decode_args(h, model, o, frame_offsets, n_utts, max_words));
+  VB_TRY(check_lattice_args(lo, out, frame_offsets, n_utts));
+  VB_CHECK(stride >= model->D, "stride %d < dim %d", stride, model->D);
+  const int64_t T = n_utts ? frame_offsets[n_utts] : 0;
+  VB_CHECK(n_utts == 0 || (num_words && tot_cost && status && (T == 0 || (feats && ali)) && (max_words == 0 || words)),
+           "null buffer");
+  if (n_utts == 0) return 0;
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->stream;
+  const size_t rows = (size_t)std::max<int64_t>(T, 1), nw = (size_t)n_utts * max_words;
+  const size_t nst = (size_t)n_utts * lo->max_states, nar = (size_t)n_utts * lo->max_arcs;
+  VB_TRY(h->d_feats.reserve(rows * stride * 4));
+  VB_TRY(h->d_ali.reserve(rows * 4));
+  VB_TRY(h->d_pdf.reserve(rows * 4));
+  VB_TRY(h->d_words.reserve(std::max<size_t>(nw, 1) * 4));
+  VB_TRY(h->d_nw.reserve((size_t)n_utts * 4));
+  VB_TRY(h->d_tot.reserve((size_t)n_utts * 8));
+  VB_TRY(h->d_status.reserve((size_t)n_utts * 4));
+  // staging: 3 state arrays, 6 arc arrays (all 4 bytes), then num_states, num_arcs, lattice_status, arena_peak x 2
+  for (int i = 0; i < 9; i++) VB_TRY(h->d_lat[i].reserve(std::max<size_t>(i < 3 ? nst : nar, 1) * 4));
+  VB_TRY(h->d_lat_n.reserve((size_t)n_utts * 5 * 4));
+  void *host_arr[9] = {out->state_frame, out->state_graph, out->state_final, out->arc_src, out->arc_dst,
+                       out->arc_ilabel, out->arc_olabel, out->arc_graph_cost, out->arc_ac_cost};
+  int32_t *dn = h->d_lat_n.as<int32_t>();
+  vbgpu_lattice_out d{};
+  d.state_frame = h->d_lat[0].as<int32_t>(), d.state_graph = h->d_lat[1].as<int32_t>();
+  d.state_final = h->d_lat[2].as<float>();
+  d.arc_src = h->d_lat[3].as<int32_t>(), d.arc_dst = h->d_lat[4].as<int32_t>();
+  d.arc_ilabel = h->d_lat[5].as<int32_t>(), d.arc_olabel = h->d_lat[6].as<int32_t>();
+  d.arc_graph_cost = h->d_lat[7].as<float>(), d.arc_ac_cost = h->d_lat[8].as<float>();
+  d.num_states = dn, d.num_arcs = dn + n_utts, d.lattice_status = dn + 2 * n_utts;
+  d.arena_peak = out->arena_peak ? dn + 3 * n_utts : nullptr;
+  unsigned long long *bad = nullptr, n_bad = 0;
+  VB_TRY(h->count.begin(s, &bad));
+  VB_TRY(h2d(h->d_feats.p, feats, (size_t)T * stride * 4, s));
+  VB_TRY(decode_run(h, model, o, acoustic_scale, true, h->d_feats.as<float>(), stride, frame_offsets, n_utts,
+                    h->d_ali.as<int32_t>(), pdf_ids ? h->d_pdf.as<int32_t>() : nullptr, h->d_words.as<int32_t>(),
+                    max_words, h->d_nw.as<int32_t>(), h->d_tot.as<double>(), h->d_status.as<int32_t>(), bad, s, lo, &d));
+  VB_TRY(d2h(ali, h->d_ali.p, (size_t)T * 4, s));
+  if (pdf_ids) VB_TRY(d2h(pdf_ids, h->d_pdf.p, (size_t)T * 4, s));
+  if (nw) VB_TRY(d2h(words, h->d_words.p, nw * 4, s));
+  VB_TRY(d2h(num_words, h->d_nw.p, (size_t)n_utts * 4, s));
+  VB_TRY(d2h(tot_cost, h->d_tot.p, (size_t)n_utts * 8, s));
+  VB_TRY(d2h(status, h->d_status.p, (size_t)n_utts * 4, s));
+  for (int i = 0; i < 9; i++)
+    if ((i < 3 ? nst : nar) > 0) VB_TRY(d2h(host_arr[i], h->d_lat[i].p, (i < 3 ? nst : nar) * 4, s));
+  VB_TRY(d2h(out->num_states, d.num_states, (size_t)n_utts * 4, s));
+  VB_TRY(d2h(out->num_arcs, d.num_arcs, (size_t)n_utts * 4, s));
+  VB_TRY(d2h(out->lattice_status, d.lattice_status, (size_t)n_utts * 4, s));
+  if (out->arena_peak) VB_TRY(d2h(out->arena_peak, d.arena_peak, (size_t)n_utts * 8, s));
   VB_TRY(h->count.end(s, &n_bad));
   if (n_bad) return fail(VBGPU_ERR_NUMERIC, kBadLoglikes, n_bad);
   return 0;

@@ -376,6 +376,8 @@ struct DecodeCall {  // per utterance and call
   int64_t f0, T;     // first row of the batch, frames
   int64_t ll_row0;   // its first row in the log-likelihood matrix the search reads
   int64_t ws_off;    // its workspace, in bytes from the group's
+  int64_t lat_off;   // lattice form: its lattice store (vb::lattice_arena_bytes), in bytes from the group's workspace
+  int32_t NT, NL;    //   tokens and links the store holds
 };
 struct DecodeArgs {  // everything the search and traceback kernels read, for one group
   const DecodeCall *calls;
@@ -388,6 +390,12 @@ struct DecodeArgs {  // everything the search and traceback kernels read, for on
   int32_t max_active, S, start, n_lvls, cap, cap2, max_words;
   int32_t *best, *status, *ali, *pdf_ids, *words, *num_words;
   double *tot_cost;
+  // lattice form
+  float lattice_beam;
+  int32_t max_states, max_arcs;
+  const int32_t *ilabel, *olabel;  // by original arc index
+  const float *weight;
+  vbgpu_lattice_out lat;
 };
 }  // namespace vb
 
@@ -398,9 +406,10 @@ struct vbgpu_decoder_s {
   int32_t S = 0, start = 0, num_tids = 0, max_pdf = -1, n_lvls = 0;
   int64_t n_emit = 0;  // emitting arcs
   int64_t workspace_cap = vb::kDecodeDefaultWorkspace;
-  vb::DevBuf d_e_off, d_x_off, d_e_arcs, d_x_arcs, d_e_pdf, d_lvl, d_final, d_tid2pdf, d_ilabel, d_olabel;
+  vb::DevBuf d_e_off, d_x_off, d_e_arcs, d_x_arcs, d_e_pdf, d_lvl, d_final, d_tid2pdf, d_ilabel, d_olabel, d_weight;
   vb::DevBuf d_calls, d_best, d_ws, d_ll;              // per-call scratch
-  vb::DevBuf d_feats, d_ali, d_pdf, d_words, d_nw, d_tot, d_status;  // staging of the host form
+  vb::DevBuf d_feats, d_ali, d_pdf, d_words, d_nw, d_tot, d_status;  // staging of the host forms
+  vb::DevBuf d_lat[9], d_lat_n;                                     //   (lattice arrays; counts and status)
   vb::CallCount count;                                 // the host form's own errors
 };
 
@@ -498,7 +507,10 @@ int64_t decode_ws_bytes(int32_t S, int32_t cap, int32_t cap2, int32_t n_lvls, in
 int decoder_set_cols(vbgpu_decoder_t h, const int32_t *d_col_of_pdf, cudaStream_t s);  // null map: identity
 int decoder_count_bad(const float *d_ll, int32_t ll_stride, int64_t T, const int32_t *d_col_of_pdf, int32_t P,
                       unsigned long long *bad, cudaStream_t s);
-int decoder_search_launch(const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s);
+// Lattice store bytes of one utterance: NT tokens, NL links, T frames.
+int64_t lattice_arena_bytes(int32_t NT, int32_t NL, int32_t cap, int32_t cap2, int64_t T);
+int decoder_search_launch(const DecodeArgs &a, int32_t u0, int32_t n, bool lattice, cudaStream_t s);
+int decoder_lattice_launch(const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s);
 int decoder_traceback_launch(vbgpu_decoder_t h, const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s);
 
 int acc_launch(vbgpu_acc_t h, const float *d_feats, const float *d_feats2, int64_t T, int32_t stride,

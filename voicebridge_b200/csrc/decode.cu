@@ -19,6 +19,10 @@
 //                            survivors of the prune are recorded: previous-frame record, emitting arc, epsilon chain.
 //   decode_traceback_kernel  a thread per utterance walks the best token's chain and the records back to the start
 //                            state and writes transition-ids, pdf-ids and words.
+// Lattice form (vbgpu_decode_lattice*): decode_search_kernel<true> also keeps every frame's tokens and links in the
+// utterance's lattice store (Lat), pruned at each frame to what can still reach the next frame, and
+//   decode_lattice_kernel    a CTA per utterance runs the exact final prune backwards over the store and writes the
+//                            numbered lattice.
 #include <algorithm>
 #include <cmath>
 #include <vector>
@@ -48,6 +52,7 @@ struct Smem {
   unsigned long long red;
   unsigned long long prefix;
   int kk, n, m, over;
+  int lover, lblock, ltop, ttop, lpeak;  // lattice: store full, links of the current frame, link / token tops, peak
 };
 
 __device__ unsigned long long block_min(unsigned long long v, Smem &sh) {
@@ -115,9 +120,11 @@ __device__ unsigned long long radix_select(const unsigned long long *keys, int n
   return sh.prefix;
 }
 
-// Calls work(source, arc) for every outgoing arc of sources [0, n_src): range(i, &a0, &deg) gives source i's arcs.
+// Calls work(source, arc, pos) for every outgoing arc of sources [0, n_src): range(i, &a0, &deg) gives source i's
+// arcs, pos numbers the arcs of all sources in source order from 0.  Returns the number of arcs.
 template <class Range, class Work>
-__device__ void for_each_arc(int n_src, Range range, Work work, Smem &sh) {
+__device__ int for_each_arc(int n_src, Range range, Work work, Smem &sh) {
+  int pos0 = 0;
   for (int base = 0; base < n_src; base += kThreads) {
     int a0 = 0, deg = 0;
     if (base + threadIdx.x < n_src) range(base + threadIdx.x, &a0, &deg);
@@ -134,10 +141,12 @@ __device__ void for_each_arc(int n_src, Range range, Work work, Smem &sh) {
         if (sh.off[mid] <= j) lo = mid;
         else hi = mid;
       }
-      work(base + lo, sh.a0[lo] + j - sh.off[lo]);
+      work(base + lo, sh.a0[lo] + j - sh.off[lo], pos0 + j);
     }
+    pos0 += total;
     __syncthreads();
   }
+  return pos0;
 }
 
 struct Utt {  // the workspace of one utterance (vb::decode_ws_bytes)
@@ -168,13 +177,50 @@ __device__ __forceinline__ void carve(Utt &w, unsigned char *p, int S, int cap, 
   w.rec = reinterpret_cast<int32_t *>(p);
 }
 
+// The lattice store of one utterance (vb::lattice_arena_bytes): the tokens and links of every frame, as each prune
+// keeps them.  A link is {source token, destination token, original arc index | kEpsLink, acoustic cost bits}.  Until
+// the prune of frame f, the links into frame f hold slots of the current set where they name frame f's tokens.
+constexpr int kEpsLink = (int)0x80000000;
+struct Lat {
+  double *alpha;                          // [NT] per token: cost
+  unsigned long long *extra, *key;        // [NT] lattice pass: extra cost key; (level, state) key
+  int32_t *state, *num, *e_first, *x_first, *abase, *ord;  // [NT] graph state; lattice pass: number, link runs ...
+  int4 *link;                             // [NL]
+  int32_t *keep;                          // [NL] lattice pass: kept by the final prune
+  int32_t *tid;                           // [cap] per slot: kept flag, then token index (-1: dropped)
+  int32_t *s_tok;                         // [cap2] per survivor: slot, then token index
+  int32_t *f_tok, *f_lnk;                 // [T + 2] frame f's tokens [f_tok[f], f_tok[f+1]), links into it likewise
+  int NT, NL;
+};
+
+__device__ __forceinline__ void carve_lat(Lat &L, unsigned char *p, int NT, int NL, int cap, int cap2, int64_t T) {
+  auto take = [&](size_t bytes) {
+    unsigned char *q = p;
+    p += (bytes + 15) & ~size_t(15);
+    return q;
+  };
+  L.NT = NT, L.NL = NL;
+  L.alpha = reinterpret_cast<double *>(take((size_t)NT * 8));
+  L.extra = reinterpret_cast<unsigned long long *>(take((size_t)NT * 8));
+  L.key = reinterpret_cast<unsigned long long *>(take((size_t)NT * 8));
+  L.link = reinterpret_cast<int4 *>(take((size_t)NL * 16));
+  int32_t **ints[] = {&L.state, &L.num, &L.e_first, &L.x_first, &L.abase, &L.ord};
+  for (int32_t **q : ints) *q = reinterpret_cast<int32_t *>(take((size_t)NT * 4));
+  L.keep = reinterpret_cast<int32_t *>(take((size_t)NL * 4));
+  L.tid = reinterpret_cast<int32_t *>(take((size_t)cap * 4));
+  L.s_tok = reinterpret_cast<int32_t *>(take((size_t)cap2 * 4));
+  L.f_tok = reinterpret_cast<int32_t *>(take((size_t)(T + 2) * 4));
+  L.f_lnk = reinterpret_cast<int32_t *>(take((size_t)(T + 2) * 4));
+}
+
 // One relaxation of the arcs out of n_src sources into the current set (emitting step or one epsilon level):
 // cost(i, a) is the candidate cost through arc position a of source i (NaN / +inf: no candidate), code(i, a) its
-// back-pointer code.  Returns false when the set outgrew its capacity.
-template <class Range, class Cost, class Code>
-__device__ bool relax(int n_src, Range range, Cost cost, Code code, const int4 *__restrict__ arcs, Utt &w, int cap,
-                      Smem &sh) {
-  for_each_arc(n_src, range, [&](int i, int a) {
+// back-pointer code.  Returns false when the set outgrew its capacity.  kLat: every arc is also recorded as a link,
+// link(i, a) giving its {source, acoustic cost bits}; a store without room for them ends the lattice (sh.lover).
+template <bool kLat, class Range, class Cost, class Code, class Link>
+__device__ bool relax(int n_src, Range range, Cost cost, Code code, Link link, int eps_bit,
+                      const int4 *__restrict__ arcs, Utt &w, Lat &L, int cap, Smem &sh) {
+  const int total = for_each_arc(n_src, range, [&](int i, int a, int) {
     const double v = cost(i, a);
     if (!(v < INFINITY)) return;
     const int d = __ldg(arcs + a).x;
@@ -190,12 +236,22 @@ __device__ bool relax(int n_src, Range range, Cost cost, Code code, const int4 *
     }
   }, sh);
   if (sh.over) return false;
-  for_each_arc(n_src, range, [&](int i, int a) {  // of the arcs that reach the minimum, the lowest code
+  const int lb = kLat ? sh.ltop : 0;
+  const bool rec = kLat && !sh.lover && (long long)lb + total <= L.NL;
+  for_each_arc(n_src, range, [&](int i, int a, int pos) {  // of the arcs that reach the minimum, the lowest code
     const double v = cost(i, a);
+    const int4 A = __ldg(arcs + a);
+    if (rec) {
+      const int2 sl = link(i, a);
+      L.link[lb + pos] = make_int4(sl.x, v < INFINITY ? w.map[A.x] : -1, A.w | eps_bit, sl.y);
+    }
     if (!(v < INFINITY)) return;
-    const int d = __ldg(arcs + a).x;
-    if (key_of(v) == w.key[d]) atomicMin(w.wn + w.map[d], code(i, a));
+    if (key_of(v) == w.key[A.x]) atomicMin(w.wn + w.map[A.x], code(i, a));
   }, sh);
+  if (kLat && threadIdx.x == 0) {
+    if (rec) sh.ltop = lb + total, sh.lpeak = max(sh.lpeak, lb + total);
+    else sh.lover = 1;
+  }
   const int n = sh.n;
   for (int k = threadIdx.x; k < n; k += kThreads) {  // commit: a lower cost takes the new back-pointer, an equal one
     const unsigned long long c = w.wn[k];           // keeps the lower code (emitting codes sort before epsilon ones)
@@ -210,7 +266,8 @@ __device__ bool relax(int n_src, Range range, Cost cost, Code code, const int4 *
 }
 
 // Epsilon closure of the current set, level after level, out of tokens whose cost is below cut.
-__device__ bool closure(const vb::DecodeArgs &g, Utt &w, double cut, Smem &sh) {
+template <bool kLat>
+__device__ bool closure(const vb::DecodeArgs &g, Utt &w, Lat &L, double cut, Smem &sh) {
   for (int l = 0; l < g.n_lvls; l++) {
     if (threadIdx.x == 0) sh.m = 0;
     __syncthreads();
@@ -223,7 +280,7 @@ __device__ bool closure(const vb::DecodeArgs &g, Utt &w, double cut, Smem &sh) {
     __syncthreads();
     const int m = sh.m;
     if (m == 0) continue;
-    const bool ok = relax(
+    const bool ok = relax<kLat>(
         m,
         [&](int i, int *a0, int *deg) {
           const int s = w.st[w.src[i]];
@@ -234,12 +291,66 @@ __device__ bool closure(const vb::DecodeArgs &g, Utt &w, double cut, Smem &sh) {
         [&](int i, int a) {
           return kEps | ((unsigned long long)__ldg(g.x_arcs + a).w << 32) | (unsigned)w.src[i];
         },
-        g.x_arcs, w, g.cap, sh);
+        [&](int i, int) { return make_int2(w.src[i], 0); }, kEpsLink, g.x_arcs, w, L, g.cap, sh);
     if (!ok) return false;
   }
   return true;
 }
 
+// Lattice, at the prune of frame t (n tokens in the current set, L.tid[k] = 1 for the tokens it expands, ns survivors
+// with L.s_tok[j] = their slot) or after the last frame (every token marked, ns = 0): also marks the tokens with an
+// epsilon path to a marked one (levels from the highest down: epsilon arcs go to higher levels), stores the marked
+// tokens as frame t's, and compacts the links into frame t in order, dropping those into unmarked tokens.
+__device__ void lat_keep(const vb::DecodeArgs &g, Utt &w, Lat &L, int n, int ns, int64_t t, Smem &sh) {
+  if (sh.lover) return;
+  const int lb = sh.lblock, le = sh.ltop;
+  for (int l = g.n_lvls - 1; l >= 0; l--) {
+    for (int i = lb + threadIdx.x; i < le; i += kThreads) {
+      const int4 k = L.link[i];
+      if (k.z < 0 && k.y >= 0 && L.tid[k.y] && __ldg(g.lvl + w.st[k.x]) == l) L.tid[k.x] = 1;
+    }
+    __syncthreads();
+  }
+  int top = sh.ttop;
+  for (int c = 0; c < n; c += kThreads) {
+    const int k = c + threadIdx.x, keep = k < n && L.tid[k];
+    int total;
+    const int j = top + block_scan(keep, sh, &total);
+    if (keep && j < L.NT) L.alpha[j] = cost_of(w.kb[k]), L.state[j] = w.st[k];
+    if (k < n) L.tid[k] = keep ? j : -1;
+    top += total;
+    __syncthreads();
+  }
+  if (top > L.NT) {
+    if (threadIdx.x == 0) sh.lover = 1;
+    __syncthreads();
+    return;
+  }
+  int lo = lb;
+  for (int c = lb; c < le; c += kThreads) {
+    const int i = c + threadIdx.x;
+    int4 k = i < le ? L.link[i] : make_int4(0, -1, 0, 0);
+    int d = k.y >= 0 ? L.tid[k.y] : -1;
+    if (d >= 0) {  // (the marking keeps the source of a link into a kept token; a dropped one drops the link)
+      k.y = d;
+      if (k.z < 0) k.x = L.tid[k.x], d = k.x >= 0 ? d : -1;
+    }
+    int total;
+    const int j = lo + block_scan(d >= 0, sh, &total);  // every thread has read its link
+    if (d >= 0) L.link[j] = k;
+    lo += total;
+    __syncthreads();
+  }
+  for (int j = threadIdx.x; j < ns; j += kThreads) L.s_tok[j] = L.tid[L.s_tok[j]];
+  if (threadIdx.x == 0) {
+    L.f_tok[t + 1] = top, L.f_lnk[t + 1] = lo;
+    sh.ttop = top, sh.ltop = lo, sh.lblock = lo;
+  }
+  __syncthreads();
+}
+
+// kLat: the lattice form, which also records tokens and links in the utterance's lattice store (Lat).
+template <bool kLat>
 __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeArgs g, int32_t u0) {
   __shared__ Smem sh;
   const int u = u0 + blockIdx.x;
@@ -247,15 +358,19 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
   const int S = g.S, cap = g.cap, cap2 = g.cap2, RW = 2 + g.n_lvls;
   Utt w;
   carve(w, g.ws + C.ws_off, S, cap, cap2);
+  Lat L{};
+  if (kLat) carve_lat(L, g.ws + C.lat_off, C.NT, C.NL, cap, cap2, C.T);
   for (int s = threadIdx.x; s < S; s += kThreads) w.key[s] = kKeyInf, w.map[s] = -1;
   __syncthreads();
   if (threadIdx.x == 0) {
     sh.n = 1, sh.over = 0;
+    sh.lover = 0, sh.lblock = 0, sh.ltop = 0, sh.ttop = 0, sh.lpeak = 0;
+    if (kLat) L.f_tok[0] = 0, L.f_lnk[0] = 0;
     w.st[0] = g.start, w.kb[0] = key_of(0.0), w.win[0] = kNone, w.wn[0] = kNone;
     w.key[g.start] = key_of(0.0), w.map[g.start] = 0;
   }
   __syncthreads();
-  int status = closure(g, w, INFINITY, sh) ? 0 : 3;
+  int status = closure<kLat>(g, w, L, INFINITY, sh) ? 0 : 3;
   for (int64_t t = 0; t < C.T && status == 0; t++) {
     // prune: cutoff c1 + beam, lowered to c_(max_active + 1) when the set is larger; the best token always survives
     const int n = sh.n;
@@ -269,6 +384,8 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
       cut = ck < cut ? ck : cut;
     }
     if (threadIdx.x == 0) sh.m = 0;
+    if (kLat)
+      for (int k = threadIdx.x; k < n; k += kThreads) L.tid[k] = 0;
     __syncthreads();
     int32_t *row = w.rec + t * cap2 * RW;
     for (int k = threadIdx.x; k < n; k += kThreads) {
@@ -276,6 +393,7 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
       if (!(c < cut || w.kb[k] == kmin)) continue;
       const int j = atomicAdd(&sh.m, 1);
       if (j >= cap2) continue;
+      if (kLat) L.tid[k] = 1, L.s_tok[j] = k;
       w.s_st[j] = w.st[k], w.s_cost[j] = c;
       int32_t *r = row + (int64_t)j * RW;  // the survivor's epsilon chain, newest arc first, then its emitting arc
       int x = k, e = 0;
@@ -295,13 +413,14 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
       status = 3;
       break;
     }
+    if (kLat) lat_keep(g, w, L, n, ns, t, sh);
     for (int k = threadIdx.x; k < n; k += kThreads) w.key[w.st[k]] = kKeyInf, w.map[w.st[k]] = -1;
     __syncthreads();
     if (threadIdx.x == 0) sh.n = 0;
     __syncthreads();
     // emitting step of frame t
     const float *llr = g.ll + (C.ll_row0 + t) * g.ll_stride;
-    const bool ok = relax(
+    const bool ok = relax<kLat>(
         ns,
         [&](int i, int *a0, int *deg) {
           const int s = w.s_st[i];
@@ -313,8 +432,11 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
           const float ac = -__fmul_rn(g.scale, __ldg(llr + A.y));
           return (w.s_cost[i] + (double)__int_as_float(A.z)) + (double)ac;
         },
-        [&](int i, int a) { return ((unsigned long long)__ldg(g.e_arcs + a).w << 32) | (unsigned)i; }, g.e_arcs, w,
-        cap, sh);
+        [&](int i, int a) { return ((unsigned long long)__ldg(g.e_arcs + a).w << 32) | (unsigned)i; },
+        [&](int i, int a) {
+          return make_int2(L.s_tok[i], __float_as_int(-__fmul_rn(g.scale, __ldg(llr + __ldg(g.e_arcs + a).y))));
+        },
+        0, g.e_arcs, w, L, cap, sh);
     if (!ok) {
       status = 3;
       break;
@@ -327,7 +449,18 @@ __global__ void __launch_bounds__(kThreads, 4) decode_search_kernel(vb::DecodeAr
     unsigned long long bmin = kNone;
     for (int k = threadIdx.x; k < n1; k += kThreads) bmin = min(bmin, w.kb[k]);
     bmin = block_min(bmin, sh);
-    if (!closure(g, w, cost_of(bmin) + (double)g.beam, sh)) status = 3;
+    if (!closure<kLat>(g, w, L, cost_of(bmin) + (double)g.beam, sh)) status = 3;
+  }
+  if (kLat) {
+    if (status == 0) {  // the last frame's tokens are all kept until the final prune
+      for (int k = threadIdx.x; k < sh.n; k += kThreads) L.tid[k] = 1;
+      __syncthreads();
+      lat_keep(g, w, L, sh.n, 0, C.T, sh);
+    }
+    if (threadIdx.x == 0) {
+      g.lat.lattice_status[u] = sh.lover;
+      if (g.lat.arena_peak) g.lat.arena_peak[2 * u] = sh.ttop, g.lat.arena_peak[2 * u + 1] = sh.lpeak;
+    }
   }
   // end: the best cost + final (status 0), else the best cost (status 1); equal values go to the lower state
   const int n = sh.n;
@@ -421,6 +554,151 @@ __global__ void __launch_bounds__(64) decode_traceback_kernel(vb::DecodeArgs g, 
   g.num_words[u] = nw;
 }
 
+// A CTA per utterance, after the search: the exact final prune of the lattice store, then the numbered output.
+__global__ void __launch_bounds__(kThreads) decode_lattice_kernel(vb::DecodeArgs g, int32_t u0) {
+  __shared__ Smem sh;
+  __shared__ unsigned long long tile[kThreads];
+  const int u = u0 + blockIdx.x;
+  const vb::DecodeCall C = g.calls[u];
+  const vbgpu_lattice_out &o = g.lat;
+  const int status = g.status[u];
+  if (status >= 2 || o.lattice_status[u] != 0) {  // an empty lattice / a store that overflowed
+    if (threadIdx.x == 0) {
+      o.num_states[u] = 0, o.num_arcs[u] = 0;
+      if (status >= 2) o.lattice_status[u] = 0;
+    }
+    return;
+  }
+  Lat L;
+  carve_lat(L, g.ws + C.lat_off, C.NT, C.NL, g.cap, g.cap2, C.T);
+  const int T = (int)C.T, nt = L.f_tok[T + 1], nl = L.f_lnk[T + 1];
+  const double tot = g.tot_cost[u], beam = (double)g.lattice_beam;
+  for (int i = threadIdx.x; i < nt; i += kThreads) L.extra[i] = kKeyInf, L.e_first[i] = -1, L.x_first[i] = -1;
+  __syncthreads();
+  for (int i = L.f_tok[T] + threadIdx.x; i < nt; i += kThreads) {  // the last frame: extra cost of ending there
+    const float f = __ldg(g.finals + L.state[i]);
+    const double e = status == 0 ? (f < INFINITY ? (L.alpha[i] + (double)f) - tot : INFINITY) : L.alpha[i] - tot;
+    if (e <= beam) L.extra[i] = key_of(e);
+  }
+  __syncthreads();
+  auto visit = [&](int i, const int4 k) {
+    const double dx = cost_of(L.extra[k.y]);
+    int keep = 0;
+    if (dx < INFINITY) {
+      double c = L.alpha[k.x] + (double)__ldg(g.weight + (k.z & 0x7fffffff));
+      if (k.z >= 0) c += (double)__int_as_float(k.w);
+      const double e = dx + (c - L.alpha[k.y]);
+      if (e <= beam) keep = 1, atomicMin(L.extra + k.x, key_of(e));
+    }
+    L.keep[i] = keep;
+  };
+  for (int f = T; f >= 0; f--) {  // frames from the last, each frame's epsilon levels from the highest
+    if (f < T) {
+      for (int i = L.f_lnk[f + 1] + threadIdx.x; i < L.f_lnk[f + 2]; i += kThreads) {
+        const int4 k = L.link[i];
+        if (k.z >= 0) visit(i, k);
+      }
+      __syncthreads();
+    }
+    for (int l = g.n_lvls - 1; l >= 0; l--) {
+      for (int i = L.f_lnk[f] + threadIdx.x; i < L.f_lnk[f + 1]; i += kThreads) {
+        const int4 k = L.link[i];
+        if (k.z < 0 && __ldg(g.lvl + L.state[k.x]) == l) visit(i, k);
+      }
+      __syncthreads();
+    }
+  }
+  // runs: the links out of one token are two runs in arc order, its emitting and its epsilon arcs
+  for (int i = threadIdx.x; i < nl; i += kThreads) {
+    const int4 k = L.link[i];
+    if (i == 0 || L.link[i - 1].x != k.x || ((L.link[i - 1].z ^ k.z) < 0)) (k.z < 0 ? L.x_first : L.e_first)[k.x] = i;
+  }
+  // state numbers: per frame, the rank of (level, state) among the kept tokens
+  int ns = 0;
+  for (int f = 0; f <= T; f++) {
+    const int a = L.f_tok[f], b = L.f_tok[f + 1];
+    int nk = 0;
+    for (int c = a; c < b; c += kThreads) {
+      const int i = c + threadIdx.x, keep = i < b && L.extra[i] != kKeyInf;
+      int total;
+      const int p = a + nk + block_scan(keep, sh, &total);
+      if (keep) L.key[p] = ((unsigned long long)__ldg(g.lvl + L.state[i]) << 32) | (unsigned)L.state[i], L.num[i] = p;
+      nk += total;
+      __syncthreads();
+    }
+    for (int c = 0; c < nk; c += kThreads) {
+      const bool mine = c + threadIdx.x < nk;
+      const unsigned long long kp = mine ? L.key[a + c + threadIdx.x] : 0;
+      int r = 0;
+      for (int q = 0; q < nk; q += kThreads) {
+        tile[threadIdx.x] = q + threadIdx.x < nk ? L.key[a + q + threadIdx.x] : ~0ull;
+        __syncthreads();
+        const int m = min(kThreads, nk - q);
+        for (int j = 0; j < m; j++) r += tile[j] < kp;
+        __syncthreads();
+      }
+      if (mine) L.abase[a + c + threadIdx.x] = ns + r;
+    }
+    __syncthreads();
+    for (int i = a + threadIdx.x; i < b; i += kThreads) {
+      const int n = L.extra[i] != kKeyInf ? L.abase[L.num[i]] : -1;
+      if (n >= 0) {
+        L.ord[n] = i;
+        if (n < g.max_states) {
+          const int st = L.state[i];
+          o.state_frame[(int64_t)u * g.max_states + n] = f;
+          o.state_graph[(int64_t)u * g.max_states + n] = st;
+          o.state_final[(int64_t)u * g.max_states + n] =
+              f < T ? INFINITY : status == 0 ? __ldg(g.finals + st) : 0.0f;
+        }
+      }
+      L.num[i] = n;  // each thread rewrites only its own tokens, whose abase entries it read
+    }
+    ns += nk;
+    __syncthreads();
+  }
+  // arcs: out-degrees, their prefix sum in state order, then each token's kept links merged by arc index
+  auto walk = [&](int i, bool out) {
+    int e = L.e_first[i], x = L.x_first[i], pos = 0;
+    const int base = out ? L.abase[i] : 0;
+    for (;;) {
+      const bool ve = e >= 0 && e < nl && L.link[e].x == i && L.link[e].z >= 0;
+      const bool vx = x >= 0 && x < nl && L.link[x].x == i && L.link[x].z < 0;
+      if (!ve && !vx) break;
+      const int j = ve && (!vx || L.link[e].z < (L.link[x].z & 0x7fffffff)) ? e++ : x++;
+      if (!L.keep[j]) continue;
+      if (out && base + pos < g.max_arcs) {
+        const int4 k = L.link[j];
+        const int arc = k.z & 0x7fffffff;
+        const int64_t q = (int64_t)u * g.max_arcs + base + pos;
+        o.arc_src[q] = L.num[i], o.arc_dst[q] = L.num[k.y];
+        o.arc_ilabel[q] = __ldg(g.ilabel + arc), o.arc_olabel[q] = __ldg(g.olabel + arc);
+        o.arc_graph_cost[q] = __ldg(g.weight + arc), o.arc_ac_cost[q] = k.z < 0 ? 0.0f : __int_as_float(k.w);
+      }
+      pos++;
+    }
+    return pos;
+  };
+  for (int i = threadIdx.x; i < nt; i += kThreads)
+    if (L.num[i] >= 0) L.abase[i] = walk(i, false);
+  __syncthreads();
+  int na = 0;
+  for (int c = 0; c < ns; c += kThreads) {
+    const int n = c + threadIdx.x, i = n < ns ? L.ord[n] : 0;
+    int total;
+    const int p = na + block_scan(n < ns ? L.abase[i] : 0, sh, &total);
+    if (n < ns) L.abase[i] = p;
+    na += total;
+    __syncthreads();
+  }
+  for (int i = threadIdx.x; i < nt; i += kThreads)
+    if (L.num[i] >= 0) walk(i, true);
+  if (threadIdx.x == 0) {
+    o.num_states[u] = ns, o.num_arcs[u] = na;
+    o.lattice_status[u] = ns > g.max_states || na > g.max_arcs ? 2 : 0;
+  }
+}
+
 // The model's column of every emitting arc (outgoing order) for this call: col_of_pdf[pdf], or pdf itself.
 __global__ void decode_cols_kernel(const int32_t *__restrict__ arc_pdf, const int32_t *__restrict__ col_of_pdf,
                                    int4 *__restrict__ arcs, int64_t n) {
@@ -456,6 +734,12 @@ int64_t decode_ws_bytes(int32_t S, int32_t cap, int32_t cap2, int32_t n_lvls, in
   return (int64_t)(align16((size_t)S * 8) + 3 * align16((size_t)cap * 8) + align16((size_t)cap2 * 8) +
                    align16((size_t)S * 4) + 2 * align16((size_t)cap * 4) + align16((size_t)cap2 * 4)) +
          align16((size_t)(T * cap2 * (2 + n_lvls) * 4));
+}
+
+int64_t lattice_arena_bytes(int32_t NT, int32_t NL, int32_t cap, int32_t cap2, int64_t T) {
+  return (int64_t)(3 * align16((size_t)NT * 8) + align16((size_t)NL * 16) + 6 * align16((size_t)NT * 4) +
+                   align16((size_t)NL * 4) + align16((size_t)cap * 4) + align16((size_t)cap2 * 4) +
+                   2 * align16((size_t)(T + 2) * 4));
 }
 
 int decoder_create(int32_t num_states, int32_t start, const float *final_cost, int64_t num_arcs, const int32_t *arc_src,
@@ -543,6 +827,7 @@ int decoder_create(int32_t num_states, int32_t start, const float *final_cost, i
   const int32_t zero = 0;
   VB_TRY(h->d_ilabel.upload(num_arcs ? arc_ilabel : &zero, (size_t)std::max<int64_t>(num_arcs, 1) * 4));
   VB_TRY(h->d_olabel.upload(num_arcs ? arc_olabel : &zero, (size_t)std::max<int64_t>(num_arcs, 1) * 4));
+  VB_TRY(h->d_weight.upload(num_arcs ? (const void *)arc_weight : &zero, (size_t)std::max<int64_t>(num_arcs, 1) * 4));
   *out = h.release();
   return 0;
 }
@@ -565,9 +850,17 @@ int decoder_count_bad(const float *d_ll, int32_t ll_stride, int64_t T, const int
   return 0;
 }
 
-int decoder_search_launch(const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s) {
+int decoder_search_launch(const DecodeArgs &a, int32_t u0, int32_t n, bool lattice, cudaStream_t s) {
   if (n == 0) return 0;
-  decode_search_kernel<<<n, kThreads, 0, s>>>(a, u0);
+  if (lattice) decode_search_kernel<true><<<n, kThreads, 0, s>>>(a, u0);
+  else decode_search_kernel<false><<<n, kThreads, 0, s>>>(a, u0);
+  VB_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int decoder_lattice_launch(const DecodeArgs &a, int32_t u0, int32_t n, cudaStream_t s) {
+  if (n == 0) return 0;
+  decode_lattice_kernel<<<n, kThreads, 0, s>>>(a, u0);
   VB_CUDA(cudaGetLastError());
   return 0;
 }

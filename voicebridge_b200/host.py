@@ -905,6 +905,91 @@ class GmmDecodeFasterGpu(_Handle):
                                                    _ptr(d_tot_cost), _ptr(d_status), _stream_ptr(stream)))
 
 
+    # lattice arrays of vbgpu_lattice_out: (name, dtype, per state (True) or per arc)
+    LATTICE_ARRAYS = (("state_frame", np.int32, True), ("state_graph", np.int32, True), ("state_final", np.float32, True),
+                      ("arc_src", np.int32, False), ("arc_dst", np.int32, False), ("arc_ilabel", np.int32, False),
+                      ("arc_olabel", np.int32, False), ("arc_graph_cost", np.float32, False),
+                      ("arc_ac_cost", np.float32, False))
+
+    @staticmethod
+    def lattice_out(arrays):
+        """vbgpu_lattice_out over a dict of arrays (numpy or torch): the LATTICE_ARRAYS names plus num_states,
+        num_arcs, lattice_status and optionally arena_peak."""
+        return capi.LatticeOut(**{k: _ptr(arrays.get(k)) for k, _ in capi.LatticeOut._fields_})
+
+    def DecodeLattice(self, am, feats, frame_offsets, acoustic_scale=0.1, max_words=64, lattice_beam=10.0,
+                      max_states=131072, max_arcs=524288, arena_tokens=8192, arena_links=24576):
+        """Host form of lattice generation (LatticeFasterDecoder up to GetRawLattice): returns Decode's tuple plus a
+        list with one dict per utterance: state_frame, state_graph, state_final (per state), arc_src, arc_dst,
+        arc_ilabel, arc_olabel, arc_graph_cost, arc_ac_cost (per arc), num_states, num_arcs, lattice_status (0 written,
+        1 lattice store overflow, 2 over max_states / max_arcs: counts only) and arena_peak (tokens, links)."""
+        feats = _np(feats, np.float32)
+        fo = _np(frame_offsets, np.int64)
+        n, T = len(fo) - 1, int(fo[-1])
+        lo = capi.default_lattice_opts(lattice_beam=lattice_beam, max_states=max_states, max_arcs=max_arcs,
+                                       arena_tokens=arena_tokens, arena_links=arena_links)
+        ali, pdf = np.zeros(max(T, 1), np.int32), np.zeros(max(T, 1), np.int32)
+        words, nw = np.zeros(max(n * max_words, 1), np.int32), np.zeros(max(n, 1), np.int32)
+        tot, st = np.zeros(max(n, 1)), np.zeros(max(n, 1), np.int32)
+        arr = {k: np.zeros(max(n * (max_states if per_state else max_arcs), 1), t)
+               for k, t, per_state in self.LATTICE_ARRAYS}
+        for k in ("num_states", "num_arcs", "lattice_status"):
+            arr[k] = np.zeros(max(n, 1), np.int32)
+        arr["arena_peak"] = np.zeros(max(2 * n, 2), np.int32)
+        out = self.lattice_out(arr)
+        check(capi.lib().vbgpu_decode_lattice(self.h, am.h, C.byref(self.opts), C.byref(lo), float(acoustic_scale),
+                                              feats.ctypes.data, feats.shape[1] if feats.ndim == 2 else 0,
+                                              fo.ctypes.data, n, ali.ctypes.data, pdf.ctypes.data, words.ctypes.data,
+                                              max_words, nw.ctypes.data, tot.ctypes.data, st.ctypes.data, C.byref(out)))
+        wl = [words[u * max_words:u * max_words + min(int(nw[u]), max_words)].tolist() for u in range(n)]
+        return ali[:T], pdf[:T], wl, nw[:n], tot[:n], st[:n], self.split_lattices(arr, n, max_states, max_arcs)
+
+    @classmethod
+    def split_lattices(cls, arr, n, max_states, max_arcs):
+        """Per-utterance dicts from the flat arrays of a call (numpy)."""
+        lats = []
+        for u in range(n):
+            ns, na, ls = int(arr["num_states"][u]), int(arr["num_arcs"][u]), int(arr["lattice_status"][u])
+            d = {"num_states": ns, "num_arcs": na, "lattice_status": ls}
+            if "arena_peak" in arr and arr["arena_peak"] is not None:
+                d["arena_peak"] = (int(arr["arena_peak"][2 * u]), int(arr["arena_peak"][2 * u + 1]))
+            for k, _, per_state in cls.LATTICE_ARRAYS:
+                cap, cnt = (max_states, ns) if per_state else (max_arcs, na)
+                d[k] = np.asarray(arr[k][u * cap:u * cap + (cnt if ls == 0 else 0)]).copy()
+            lats.append(d)
+        return lats
+
+    def _lattice_opts(self, lattice_opts):
+        return lattice_opts if lattice_opts is not None else capi.default_lattice_opts()
+
+    def decode_lattice_dev(self, am, d_feats, stride, frame_offsets, d_ali, d_pdf_ids, d_words, max_words,
+                           d_num_words, d_tot_cost, d_status, lattice, lattice_opts=None, acoustic_scale=0.1,
+                           stream=None):
+        """Feature form of lattice generation on device buffers: the decode_dev arguments plus `lattice`, a dict of
+        device arrays (lattice_out) sized by lattice_opts (capi.default_lattice_opts)."""
+        fo = _np(frame_offsets, np.int64)
+        out = self.lattice_out(lattice)
+        check(capi.lib().vbgpu_decode_lattice_dev(self.h, am.h, C.byref(self.opts),
+                                                  C.byref(self._lattice_opts(lattice_opts)), float(acoustic_scale),
+                                                  _ptr(d_feats), stride, fo.ctypes.data, len(fo) - 1, _ptr(d_ali),
+                                                  _ptr(d_pdf_ids), _ptr(d_words), max_words, _ptr(d_num_words),
+                                                  _ptr(d_tot_cost), _ptr(d_status), C.byref(out), _stream_ptr(stream)))
+
+    def decode_lattice_loglikes_dev(self, am, d_loglikes, ll_stride, frame_offsets, d_ali, d_pdf_ids, d_words,
+                                    max_words, d_num_words, d_tot_cost, d_status, lattice, lattice_opts=None,
+                                    acoustic_scale=0.1, stream=None):
+        """Log-likelihood form of lattice generation: d_loglikes [T x ll_stride] in the model's device column order."""
+        fo = _np(frame_offsets, np.int64)
+        out = self.lattice_out(lattice)
+        check(capi.lib().vbgpu_decode_lattice_loglikes_dev(self.h, am.h, C.byref(self.opts),
+                                                           C.byref(self._lattice_opts(lattice_opts)),
+                                                           float(acoustic_scale), _ptr(d_loglikes), ll_stride,
+                                                           fo.ctypes.data, len(fo) - 1, _ptr(d_ali), _ptr(d_pdf_ids),
+                                                           _ptr(d_words), max_words, _ptr(d_num_words),
+                                                           _ptr(d_tot_cost), _ptr(d_status), C.byref(out),
+                                                           _stream_ptr(stream)))
+
+
 class ScoringPipeline(_Handle):
     """PCM -> per-frame per-pdf log-likelihoods in one call (MFCC -> CMVN -> deltas|LDA -> fMLLR -> GMM scoring)."""
     _destroy = "vbgpu_pipeline_destroy"
