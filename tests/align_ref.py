@@ -43,13 +43,14 @@ def _padded(arcs, dests, rows):
     return m
 
 
-def viterbi_align_ref(graphs, u, ll, pdfs, tid2pdf, tid_cost=None, acoustic_scale=0.1):
+def viterbi_align_ref(graphs, u, ll, pdfs, tid2pdf, tid_cost=None, acoustic_scale=0.1, path=None):
     """float64 restatement of vbgpu_align for utterance u (include/vbgpu.h): ll [T_u, len(pdfs)] holds the log-likelihoods
     of the pdfs `pdfs` (align_subsets order).  Same operation order as the device: arc weights plus tid_cost in float32,
     ac = -(acoustic_scale * ll) in float32, emitting cost (prev + w) + ac and epsilon cost prev + w in float64; the
     epsilon closure level by level (longest epsilon path into a state), first-in-arc-order wins ties, an epsilon
     relaxation only when strictly lower, the lowest state among equal final costs.
-    Returns (tot_cost, ali[T_u] transition-ids, pdf_ids[T_u]); (+inf, zeros, -1s) when no final state is reachable."""
+    Returns (tot_cost, ali[T_u] transition-ids, pdf_ids[T_u]); (+inf, zeros, -1s) when no final state is reachable.
+    path (a list) receives the arcs of the best path, epsilon arcs included, in order, as arc indices of utterance u."""
     so, ao = graphs["state_offsets"], graphs["arc_offsets"]
     S, a0, a1 = int(so[u + 1] - so[u]), int(ao[u]), int(ao[u + 1])
     src, dst = np.asarray(graphs["arc_src"][a0:a1], np.int64), np.asarray(graphs["arc_dst"][a0:a1], np.int64)
@@ -103,12 +104,15 @@ def viterbi_align_ref(graphs, u, ll, pdfs, tid2pdf, tid_cost=None, acoustic_scal
     s = int(np.argmin(tot))
     if not tot[s] < inf:
         return inf, np.zeros(T, np.int32), np.full(T, -1, np.int32)
-    ali, r = np.zeros(T, np.int32), T
+    ali, r, arcs = np.zeros(T, np.int32), T, []
     while tb[r, s] >= 0:
         a = int(tb[r, s])
+        arcs.append(a)
         if lab[a]:
             r -= 1
             ali[r] = lab[a]
         s = int(src[a])
     assert r == 0
+    if path is not None:
+        path.extend(arcs[::-1])
     return float(tot[int(np.argmin(tot))]), ali, tid2pdf[ali].astype(np.int32)
